@@ -3,6 +3,8 @@
 
     python bench.py --gpus N --steps K --warmup W            # B200 arm (this repository's CUDA path)
     python bench.py --impl reference --gpus N --steps K ...  # reference arm: the reference's algorithm on host cores
+    python bench.py --steps K --dump-outputs bench_outputs/A # also write the last timed step's outputs (two builds
+                                                             # given the same arguments see the same inputs)
 
 A step = one forward pass of the encoder over one synthetic batch.  Workload at every N: BASELINE.json configs[1],
 Conformer-CTC Large encoder (d_model 512, 17 layers, 8 heads, ff x4, striding x4), batch 32 x 20 s (T = 2000 mel
@@ -397,9 +399,10 @@ def build_batches(args, kw, rank, world, name=None):
 
 
 def measure_workload(enc, args, host_batches, audio_sec_job, device, barrier, max_over_ranks, sampler=None,
-                     eager=True):
+                     eager=True, keep_outputs=False):
     """Times one workload on this rank's sub-batches: device-resident steps launched eagerly, then through CUDA-graph
-    replay (the headline), then end to end with host buffers.  Returns a dict; every time is the max over ranks."""
+    replay (the headline), then end to end with host buffers.  Returns a dict; every time is the max over ranks.
+    keep_outputs: the dict also holds `outputs`, the [(encoded, encoded_len), ...] of the last timed step on the host."""
     use_host_lens = args.packed != "off"
     enc.packed = True if args.packed == "on" else "auto"
     dev_batches = [(x.to(device), ln.to(device), ln.tolist() if use_host_lens else None) for x, ln in host_batches]
@@ -407,12 +410,10 @@ def measure_workload(enc, args, host_batches, audio_sec_job, device, barrier, ma
     concurrent = [False]  # set once graphs with private workspaces are on: sub-batches overlap on side streams
 
     def step():
+        """One forward of every sub-batch: [(encoded, encoded_len), ...]."""
         if concurrent[0]:
-            return enc.forward_many(dev_batches, args.streams)[-1]
-        out = None
-        for xd, ld, hl in dev_batches:
-            out = enc(audio_signal=xd, length=ld, length_host=hl)
-        return out
+            return enc.forward_many(dev_batches, args.streams)
+        return [enc(audio_signal=xd, length=ld, length_host=hl) for xd, ld, hl in dev_batches]
 
     enc.enable_cuda_graphs(False)
     launches_per_step = 0
@@ -455,11 +456,23 @@ def measure_workload(enc, args, host_batches, audio_sec_job, device, barrier, ma
         sampler.mark()
     e0.record()
     for _ in range(args.steps):
-        y, ylen = step()
+        outs = step()
     e1.record()
     barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if sampler is not None else None
+    outputs = None
+    if keep_outputs:
+        # graph replays return views of the graph's static buffers, which the end-to-end pass below overwrites.  One after
+        # the other, sub-batches of one shape also replay one graph, so the last step kept only the last one's result:
+        # then one more (untimed) step copies every result out before the next forward; the forward is deterministic.
+        if len(dev_batches) > 1 and not concurrent[0]:
+            outputs = []
+            for xd, ld, hl in dev_batches:
+                y, ylen = enc(audio_signal=xd, length=ld, length_host=hl)
+                outputs.append((y.cpu(), ylen.cpu()))
+        else:
+            outputs = [(y.cpu(), ylen.cpu()) for y, ylen in outs]
     ms_step = ms_total / args.steps
     value = audio_sec_job / (ms_step / 1e3)
 
@@ -469,7 +482,7 @@ def measure_workload(enc, args, host_batches, audio_sec_job, device, barrier, ma
     # D2H are inside the timed region; the closing event waits for the last D2H.
     n_buf = 2
     shapes = [(x.shape[0], enc.output_frames(x.shape[2])) for x, _ in host_batches]
-    d_out = y.shape[1]
+    d_out = outs[-1][0].shape[1]
     max_b = max(sh[0] for sh in shapes)
     max_bt = max(sh[0] * sh[1] for sh in shapes)
     max_in = max(x.numel() for x, _ in host_batches)
@@ -570,7 +583,42 @@ def measure_workload(enc, args, host_batches, audio_sec_job, device, barrier, ma
            "h2d_bytes_per_step": sum(x.numel() * 4 + ln.numel() * 8 for x, ln in host_batches),
            "d2h_bytes_per_step": sum(bb * tt * d_out * 4 + bb * 4 for bb, tt in shapes)}
     return {"value": value, "ms_per_step": ms_step, "eager_ms_per_step": eager_ms, "e2e": e2e, "clocks": clocks,
-            "launches_per_step": launches_per_step, "step": step, "sub_batches_in_flight": args.streams if concurrent[0] else 1}
+            "launches_per_step": launches_per_step, "step": step, "sub_batches_in_flight": args.streams if concurrent[0] else 1,
+            "outputs": outputs}
+
+
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much
+DUMP_WHOLE_BYTES = 1 << 20  # arrays up to this size are always written whole
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes the [(encoded, encoded_len), ...] of one step as out_dir/encoded.npy and out_dir/encoded_len.npy (with a
+    _<i> suffix per sub-batch when there are several): floating arrays as float32, integer ones as float64 (exact).
+    When the arrays exceed DUMP_BYTES, each one larger than DUMP_WHOLE_BYTES is replaced by the same seeded sample of
+    its flattened (C-order) elements, written as <name>.npy beside the float64 flat indices in <name>_index.npy."""
+    import numpy as np
+
+    named = {}
+    for i, (y, ylen) in enumerate(outputs):
+        sfx = f"_{i}" if len(outputs) > 1 else ""
+        named["encoded" + sfx] = y.float().contiguous().numpy()
+        named["encoded_len" + sfx] = ylen.double().numpy()
+    total = sum(a.nbytes for a in named.values())
+    if total > DUMP_BYTES:
+        big = [k for k, a in named.items() if a.nbytes > DUMP_WHOLE_BYTES]
+        headers = 1024 * (len(named) + len(big))  # a .npy header is 128 bytes
+        budget = DUMP_BYTES - headers - sum(a.nbytes for k, a in named.items() if k not in big)
+        frac = budget / sum(named[k].size * (named[k].itemsize + 8) for k in big)  # a sampled value + its index
+        for k in big:
+            a = named.pop(k).reshape(-1)
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randperm(a.size, generator=g)[: int(a.size * frac)].sort().values.numpy()
+            named[k] = a[idx]
+            named[k + "_index"] = idx.astype("float64")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in named.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    return sorted(named)
 
 
 def packing_stats(enc, host_batches):
@@ -625,7 +673,10 @@ def run_b200(args):
     if rank == 0:
         sampler.start()
     head = measure_workload(enc, args, host_batches, audio_sec_job, device, barrier, max_over_ranks,
-                            sampler if rank == 0 else None)
+                            sampler if rank == 0 else None, keep_outputs=bool(args.dump_outputs) and rank == 0)
+    outputs = head.pop("outputs", None)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     step = head["step"]
     if args.ncu:
         # profiling helper: 3 warm-up steps above, ONE eager step here, nothing else (no graphs, no e2e, no JSON):
@@ -768,12 +819,12 @@ def run_b200(args):
                 worst, per_rank = 0.0, []
                 for r in range(w):
                     rb, _, _, _ = build_batches(args, kw, r, w, name="cfg3")
-                    saved = (args.steps, args.settle)
-                    args.steps, args.settle = min(args.steps, 10), 0.0
+                    saved = args.settle
+                    args.settle = 0.0
                     try:
                         m = measure_workload(enc, args, rb, s_audio, device, barrier, max_over_ranks, None, eager=False)
                     finally:
-                        args.steps, args.settle = saved
+                        args.settle = saved
                     per_rank.append(round(m["ms_per_step"], 4))
                     worst = max(worst, m["ms_per_step"])
                 sim[str(w)] = {"ms_per_step_slowest_rank": worst, "value": s_audio / (worst / 1e3),
@@ -789,7 +840,7 @@ def run_b200(args):
     pipelines = None
     if rank == 0 and world == 1 and args.pipelines and args.workload == "cfg2":
         try:
-            pipelines = measure_pipelines(enc, device)
+            pipelines = measure_pipelines(enc, device, steps=args.steps)
         except Exception as e:  # noqa: BLE001 -- an extra record must never cost the headline
             pipelines = {"unavailable": f"{type(e).__name__}: {e}"}
 
@@ -932,7 +983,8 @@ def main():
     os.dup2(2, 1)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the throughput measurements (headline, eager, e2e, strong, pipelines); the per-kernel and "
+                         "per-stage breakdowns and cpu_baseline keep their own counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS))
@@ -955,7 +1007,13 @@ def main():
     ap.add_argument("--settle", type=float, default=1.0, help="seconds of extra warm-up load before timing")
     ap.add_argument("--ncu", action="store_true", help="3 warm-up steps + 1 eager step only (for ncu -s/-c)")
     ap.add_argument("--no-graphs", action="store_true", help="launch every step eagerly (no CUDA graph replay)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the encoder outputs of the last timed step of the headline as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.ncu):
+        ap.error("--dump-outputs needs the timed steps of the b200 arm")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -12,6 +12,10 @@ import conformer_nemo_b200 as cn
 from oracle import reference_loader as rl
 
 needs_ref = pytest.mark.skipif(not rl.reference_available(), reason="reference tree not mounted")
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "collation.json")  # tests/golden/make_golden_collation.py
+MANIFEST_KWARGS = [dict(), dict(min_duration=0.1, max_duration=16.7), dict(max_number=7, min_duration=1.0),
+                   dict(do_sort_by_duration=True, max_duration=20.0)]
+NO_AUDIO = [(None, None, torch.tensor([1, 2, 3]), torch.tensor(3)), (None, None, torch.tensor([4]), torch.tensor(1))]
 
 
 def _batch(gen, n, with_ids, max_len=50, max_tok=7, dtype=torch.float32):
@@ -42,8 +46,7 @@ def test_collate_equals_reference(with_ids):
 @needs_ref
 def test_collate_edge_cases_equal_reference():
     a2t, _ = rl.load_reference_collation()
-    no_audio = [(None, None, torch.tensor([1, 2, 3]), torch.tensor(3)), (None, None, torch.tensor([4]), torch.tensor(1))]
-    want, got = a2t._speech_collate_fn(no_audio, pad_id=0), cn.speech_collate(no_audio, pad_id=0)
+    want, got = a2t._speech_collate_fn(NO_AUDIO, pad_id=0), cn.speech_collate(NO_AUDIO, pad_id=0)
     assert got[0] is None and got[1] is None and want[0] is None
     assert torch.equal(got[2], want[2]) and torch.equal(got[3], want[3])
     for bad in ([(torch.zeros(3), torch.tensor(3), torch.tensor([1]))], ):
@@ -77,18 +80,20 @@ def _write_manifest(path, rng, n):
             f.write(json.dumps(item) + "\n")
 
 
+def _manifest_parser(text):
+    return None if text == "skip me" else [ord(c) - 96 for c in text if c != " "]
+
+
 @needs_ref
-@pytest.mark.parametrize("kw", [dict(), dict(min_duration=0.1, max_duration=16.7), dict(max_number=7, min_duration=1.0),
-                                dict(do_sort_by_duration=True, max_duration=20.0)])
+@pytest.mark.parametrize("kw", MANIFEST_KWARGS)
 def test_manifest_equals_reference(tmp_path, kw):
     _, coll = rl.load_reference_collation()
     rng = random.Random(5)
     paths = [str(tmp_path / "a.json"), str(tmp_path / "b.json")]
     _write_manifest(paths[0], rng, 23)
     _write_manifest(paths[1], rng, 9)
-    parser = lambda text: None if text == "skip me" else [ord(c) - 96 for c in text if c != " "]
-    want = coll.ASRAudioText(manifests_files=paths, parser=parser, **kw)
-    got = cn.read_manifest(",".join(paths), parser=parser, **kw)
+    want = coll.ASRAudioText(manifests_files=paths, parser=_manifest_parser, **kw)
+    got = cn.read_manifest(",".join(paths), parser=_manifest_parser, **kw)
     assert len(got) == len(want) > 0
     for g, w in zip(got, want):
         assert (g.id, g.audio_file, g.duration, g.text_tokens, g.offset, g.text_raw) == \
@@ -117,6 +122,65 @@ def test_bucketing_iterator_equals_reference():
     for n, k in ((10, 4), (8, 4), (3, 5), (0, 2)):
         assert list(cn.BucketingIterator(iter(range(n)), k)) == list(a2t.BucketingIterator(iter(range(n)), k))
     assert list(cn.BucketingIterator(range(5), 2)) == [[0, 1], [2, 3], [4]]
+
+
+def _golden():
+    with open(GOLDEN) as f:
+        return json.load(f)
+
+
+def _tensor(j):
+    return None if j is None else torch.tensor(j["data"], dtype=getattr(torch, j["dtype"])).reshape(j["shape"])
+
+
+@pytest.mark.parametrize("with_ids", [False, True])
+def test_collate_equals_golden(with_ids):
+    """The same seeded batches as test_collate_equals_reference, against the stored collate outputs."""
+    cases = _golden()["collate"][str(with_ids)]
+    gen = torch.Generator().manual_seed(3)
+    for n, want in zip((1, 2, 7), cases):
+        batch = _batch(gen, n, with_ids)
+        got = cn.speech_collate(batch, pad_id=28)
+        assert len(got) == len(want)
+        for g, w in zip(got, want):
+            w = _tensor(w)
+            assert g.dtype == w.dtype and torch.equal(g, w)
+        staged = cn.speech_collate(batch, pad_id=28, audio_out=torch.full((9, 64), 7.0))
+        assert torch.equal(staged[0], _tensor(want[0]))
+    assert len(cases) == 3
+
+
+def test_collate_edge_cases_equal_golden():
+    z = _golden()
+    got = cn.speech_collate(NO_AUDIO, pad_id=0)
+    assert got[0] is None and got[1] is None and z["no_audio"][0] is None and z["no_audio"][1] is None
+    assert torch.equal(got[2], _tensor(z["no_audio"][2])) and torch.equal(got[3], _tensor(z["no_audio"][3]))
+    assert z["errors"] == {"three_tuple": "ValueError", "length_exceeds_signal": "RuntimeError"}
+    with pytest.raises(ValueError):
+        cn.speech_collate([(torch.zeros(3), torch.tensor(3), torch.tensor([1]))], pad_id=0)
+    with pytest.raises(RuntimeError):
+        cn.speech_collate([(torch.zeros(5), torch.tensor(4), torch.tensor([1]), torch.tensor(1)),
+                           (torch.zeros(6), torch.tensor(6), torch.tensor([1]), torch.tensor(1))], pad_id=0)
+
+
+@pytest.mark.parametrize("kw", MANIFEST_KWARGS)
+def test_manifest_equals_golden(tmp_path, kw):
+    """The same two manifests and filter settings as test_manifest_equals_reference, against the stored entries."""
+    (want,) = [m["entries"] for m in _golden()["manifest"] if m["kwargs"] == kw]
+    rng = random.Random(5)
+    paths = [str(tmp_path / "a.json"), str(tmp_path / "b.json")]
+    _write_manifest(paths[0], rng, 23)
+    _write_manifest(paths[1], rng, 9)
+    got = cn.read_manifest(",".join(paths), parser=_manifest_parser, **kw)
+    assert len(want) > 0
+    assert [[e.id, e.audio_file, e.duration, e.text_tokens, e.offset, e.text_raw] for e in got] == want
+
+
+def test_bucketing_iterator_equals_golden():
+    cases = _golden()["bucketing"]
+    assert len(cases) == 4
+    for c in cases:
+        assert [list(b) for b in cn.BucketingIterator(iter(range(c["n"])), c["k"])] == c["chunks"]
 
 
 def _service(n_ranks, rank, device=None, n=41, seed=2):

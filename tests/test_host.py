@@ -196,11 +196,24 @@ model:
     assert isinstance(enc, cn.ConformerEncoder) and len(enc.layers) == 2
     cfg["_target_"] = "conformer_nemo_b200.ConformerEncoder"
     assert isinstance(cn.instantiate_encoder(cfg), cn.ConformerEncoder)
-    ref_recipes = "/root/reference/configs"
-    if os.path.isdir(ref_recipes):  # every shipped recipe resolves and is accepted by the constructor
-        for name in sorted(os.listdir(ref_recipes)):
-            c = cn.load_encoder_config(os.path.join(ref_recipes, name), overrides=dict(n_layers=1))
-            assert isinstance(cn.instantiate_encoder(c), cn.ConformerEncoder), name
+    from oracle import reference_loader as rl
+
+    # every recipe resolves and is accepted by the constructor: the stored encoder blocks (tests/golden/recipes), plus the
+    # shipped recipes themselves when the reference tree is reachable
+    stored = os.path.join(ROOT, "tests", "golden", "recipes")
+    want = {"conformer_ctc_bpe.yaml": (512, 18, 8), "conformer_transducer_bpe.yaml": (512, 17, 8),
+            "conformer_ctc_char.yaml": (256, 16, 8)}
+    assert sorted(os.listdir(stored)) == sorted(want)
+    for name, (d, layers, heads) in want.items():
+        c = cn.load_encoder_config(os.path.join(stored, name))
+        assert (c["feat_in"], c["d_model"], c["n_layers"], c["n_heads"]) == (80, d, layers, heads), name
+    ref_recipes = os.path.join(rl.REFERENCE_ROOT, "configs")
+    paths = [os.path.join(stored, n) for n in sorted(want)]
+    if os.path.isdir(ref_recipes):
+        paths += [os.path.join(ref_recipes, n) for n in sorted(os.listdir(ref_recipes))]
+    for path in paths:
+        c = cn.load_encoder_config(path, overrides=dict(n_layers=1))
+        assert isinstance(cn.instantiate_encoder(c), cn.ConformerEncoder), path
 
 
 def test_plan_shards_properties():

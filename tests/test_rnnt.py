@@ -109,6 +109,20 @@ def test_sample_level_greedy_of_the_reference_gives_the_batched_hypotheses():
         assert (h.dec_state is None) == (n == 0)
 
 
+@pytest.mark.parametrize("name", CASES)
+def test_one_utterance_at_a_time_gives_the_reference_batched_golden(name):
+    """The premise of test_sample_level_greedy_of_the_reference_gives_the_batched_hypotheses without the reference tree:
+    decoding each utterance alone (decoding.strategy = greedy) reproduces the reference's stored greedy_batch
+    hypotheses -- tokens and timesteps exactly, scores to fp32 rounding."""
+    g = load(name)
+    for b in range(g["x"].shape[0]):
+        (r,) = ro.rnnt_greedy_decode(g["x"][b:b + 1], g["lens"][b:b + 1], g["dec_sd"], g["joint_sd"], g["max_symbols"],
+                                     g["activation"], True)
+        n = int(g["n"][b])
+        assert r.tokens == g["tokens"][b, :n].tolist() and r.timesteps == g["timesteps"][b, :n].tolist(), b
+        assert abs(r.score - float(g["scores"][b])) <= 1e-4 * max(1.0, abs(float(g["scores"][b]))), b
+
+
 def test_oracle_per_utterance_independence():
     g = load("rnnt_bpe128")
     full = ro.rnnt_greedy_decode(g["x"], g["lens"], g["dec_sd"], g["joint_sd"], g["max_symbols"], g["activation"], False)

@@ -9,4 +9,5 @@ from .sharding import plan_shards, forward_sharded  # noqa: F401
 from .ctc_head import ConvASRDecoder, ctc_collapse_device, ctc_greedy_decode  # noqa: F401
 from .preprocessor import AudioToMelSpectrogramPreprocessor  # noqa: F401
 from .rnnt import RNNTDecoder, RNNTJoint, GreedyBatchedRNNTInfer, GreedyRNNTInfer, Hypothesis  # noqa: F401
+from .rnnt import BeamRNNTInfer, NBestHypotheses  # noqa: F401
 from .collation import (BucketingIterator, CollationService, ManifestEntry, read_manifest, speech_collate)  # noqa: F401

@@ -25,7 +25,7 @@ SYMBOLS = [
     "cfb_workspace_bytes", "cfb_forward", "cfb_packed_workspace_bytes", "cfb_forward_packed", "cfb_debug_buffer", "cfb_set_profiling", "cfb_profile_report",
     "cfb_last_launch_count", "cfb_op_gemm", "cfb_op_ctc_head", "cfb_ctc_head_scratch_bytes", "cfb_op_ctc_collapse",
     "cfb_op_layernorm", "cfb_op_depthwise", "cfb_op_dw_pw2", "cfb_op_logmel", "cfb_op_rel_attention", "cfb_op_lengths",
-    "cfb_rnnt_greedy_scratch_bytes", "cfb_op_rnnt_greedy",
+    "cfb_rnnt_greedy_scratch_bytes", "cfb_op_rnnt_greedy", "cfb_rnnt_beam_scratch_bytes", "cfb_op_rnnt_beam",
 ]
 
 
@@ -47,6 +47,11 @@ class CfbRnntWeights(ctypes.Structure):
         ("embed", _fp), ("w_ih", _fp), ("w_hh", _fp), ("b_ih", _fp), ("b_hh", _fp), ("w_pred", _fp), ("b_pred", _fp),
         ("w_enc", _fp), ("b_enc", _fp), ("w_out", _fp), ("b_out", _fp),
     ]
+
+
+class CfbRnntBeamCaps(ctypes.Structure):
+    _fields_ = [("max_expansions", ctypes.c_int32), ("max_hyps", ctypes.c_int32), ("max_nodes", ctypes.c_int32),
+                ("max_states", ctypes.c_int32), ("max_len", ctypes.c_int32), ("reserved", ctypes.c_int32 * 3)]
 
 
 _lock = threading.Lock()
@@ -96,9 +101,13 @@ def load_library() -> ctypes.CDLL:
         lib.cfb_rnnt_greedy_scratch_bytes.argtypes = [i32, i32, i32, i32, i32]
         lib.cfb_op_rnnt_greedy.argtypes = [ctypes.POINTER(CfbRnntWeights), vp, i32, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp,
                                            vp, vp, vp, sz, vp]
+        caps = ctypes.POINTER(CfbRnntBeamCaps)
+        lib.cfb_rnnt_beam_scratch_bytes.argtypes = [i32, i32, i32, i32, i32, i32, caps]
+        lib.cfb_op_rnnt_beam.argtypes = [ctypes.POINTER(CfbRnntWeights), vp, i32, vp, i32, i32, i32, i32, ctypes.c_float, caps,
+                                         vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
         for name in SYMBOLS:
             fn = getattr(lib, name)
-            if name in ("cfb_ctc_head_scratch_bytes", "cfb_rnnt_greedy_scratch_bytes"):
+            if name in ("cfb_ctc_head_scratch_bytes", "cfb_rnnt_greedy_scratch_bytes", "cfb_rnnt_beam_scratch_bytes"):
                 fn.restype = ctypes.c_size_t
             elif name not in ("cfb_destroy", "cfb_last_error"):
                 fn.restype = ctypes.c_int

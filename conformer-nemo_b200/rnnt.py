@@ -8,8 +8,9 @@ Same constructor arguments, same ``state_dict`` keys (``prediction.embed.weight`
 ``greedy(encoder_output=(B, D, T), encoded_lengths=(B,)) -> (List[Hypothesis],)`` with ``y_sequence`` / ``timestep`` /
 ``score`` / ``dec_state`` / ``length`` filled like the reference does.  The whole decode -- joint.enc over every frame,
 then the symbol loop with the LSTM and the joint -- runs in libcfb.so (``cfb_op_rnnt_greedy``, csrc/rnnt_greedy.cu)
-with ONE device-to-host read at the end; the reference synchronises once per symbol step.  No CPU fallback; training
-(``forward`` over label sequences, the transducer loss) stays with the reference modules.
+with ONE device-to-host read at the end; the reference synchronises once per symbol step.  ``decoding.strategy = beam``
+(parts/submodules/rnnt_beam_decoding.py, ``BeamRNNTInfer``) runs in ``cfb_op_rnnt_beam`` (csrc/rnnt_beam.cu).  No CPU
+fallback; training (``forward`` over label sequences, the transducer loss) stays with the reference modules.
 """
 from __future__ import annotations
 
@@ -23,6 +24,7 @@ from torch import nn
 from . import _lib
 
 _ACTIVATIONS = {"relu": 0, "sigmoid": 1, "tanh": 2}
+_MAX_HYPS = 2048  # entries of a hypothesis list of cfb_op_rnnt_beam (shared memory)
 
 
 @dataclass
@@ -272,6 +274,180 @@ class GreedyBatchedRNNTInfer:
             hyps.append(Hypothesis(score=float(scores[i]), y_sequence=tokens[i, :k].clone(), timestep=steps[i, :k].tolist(),
                                    dec_state=state, length=lens_cpu[i]))
         return (hyps,)
+
+
+@dataclass
+class NBestHypotheses:
+    """parts/utils/rnnt_utils.py: the sorted n-best list of one utterance (``return_best_hypothesis=False``)."""
+    n_best_hypotheses: Optional[List[Hypothesis]]
+
+
+class BeamRNNTInfer:
+    """``decoding.strategy = beam`` (parts/submodules/rnnt_beam_decoding.py, ``BeamRNNTInfer``): ``search_type='default'``
+    (default_beam_search) and, for ``beam_size == 1``, the class's own sample-level greedy_search.  The search for every
+    utterance of the batch runs in one persistent kernel (``cfb_op_rnnt_beam``, csrc/rnnt_beam.cu) with one device-to-host
+    read at the end; the reference decodes one utterance at a time and synchronises once per hypothesis expansion.
+
+    Hypotheses are filled like the reference's pack_hypotheses: ``y_sequence`` a LongTensor with its leading blank,
+    ``timestep`` with its leading -1 (greedy_search: neither), ``score`` the double sum of log-probabilities,
+    ``dec_state`` the LSTM state ``(h, c)`` as (1, 1, H) CPU tensors (None for greedy_search before its first label),
+    ``length`` the utterance's encoded length.  TSD / ALSD / MAES, language models, alignments and partial hypotheses raise
+    NotImplementedError."""
+
+    def __init__(self, decoder_model: RNNTDecoder, joint_model: RNNTJoint, beam_size: int, search_type: str = "default",
+                 score_norm: bool = True, return_best_hypothesis: bool = True, tsd_max_sym_exp_per_step: Optional[int] = 50,
+                 alsd_max_target_len: Union[int, float] = 1.0, nsc_max_timesteps_expansion: int = 1,
+                 nsc_prefix_alpha: int = 1, maes_num_steps: int = 2, maes_prefix_alpha: int = 1,
+                 maes_expansion_gamma: float = 2.3, maes_expansion_beta: int = 2,
+                 language_model: Optional[Dict[str, Any]] = None, softmax_temperature: float = 1.0,
+                 preserve_alignments: bool = False, ngram_lm_model: Optional[str] = None, ngram_lm_alpha: float = 0.0):
+        if beam_size < 1:
+            raise ValueError("Beam search size cannot be less than 1!")
+        if search_type not in ("default", "tsd", "alsd", "nsc", "maes"):
+            raise NotImplementedError(f"The search type ({search_type}) supplied is not supported!\n"
+                                      "Please use one of : (default, tsd, alsd, nsc)")
+        if beam_size > 1 and search_type != "default":
+            raise NotImplementedError(f"BeamRNNTInfer (B200): search_type={search_type!r} (only 'default' runs on the device)")
+        if language_model is not None or ngram_lm_model is not None:
+            raise NotImplementedError("BeamRNNTInfer (B200): language-model fusion")
+        if preserve_alignments:
+            raise NotImplementedError("BeamRNNTInfer (B200): preserve_alignments is a debugging aid of the reference")
+        if not softmax_temperature > 0:
+            raise ValueError("softmax_temperature must be positive")
+        if decoder_model.pred_hidden != joint_model.pred_hidden:
+            raise ValueError("decoder pred_hidden and joint pred_hidden differ")
+        if decoder_model.blank_idx != joint_model.num_classes_with_blank - 1:
+            raise ValueError("the decoder's blank index must be the joint's last class (blank_as_pad)")
+        self.decoder = decoder_model
+        self.joint = joint_model
+        self.blank = decoder_model.blank_idx
+        self.vocab_size = decoder_model.vocab_size
+        self.search_type = search_type
+        self.return_best_hypothesis = return_best_hypothesis
+        self.beam_size = beam_size
+        self.score_norm = score_norm
+        self.max_candidates = beam_size
+        self.softmax_temperature = float(softmax_temperature)
+        self.preserve_alignments = False
+        self._blank_index = self.blank
+        self._packed = None
+        self._scratch = None
+
+    # the fp32 weight copies and their refresh are those of the greedy decode
+    _sources = GreedyBatchedRNNTInfer._sources
+    _fingerprint = GreedyBatchedRNNTInfer._fingerprint
+    _prepare = GreedyBatchedRNNTInfer._prepare
+    invalidate = GreedyBatchedRNNTInfer.invalidate
+
+    def __call__(self, *args, **kwargs):
+        return self.forward(*args, **kwargs)
+
+    def widths(self) -> Tuple[int, int]:
+        """(beam, beam_k) of default_beam_search: hypotheses that end a frame, non-blank candidates per expansion."""
+        beam = min(self.beam_size, self.vocab_size + 1)
+        return beam, min(beam, self.vocab_size)
+
+    def default_caps(self, t: int) -> Dict[str, int]:
+        """First-try capacities for T frames; the decode is repeated with larger ones when an utterance outgrows them."""
+        beam, beam_k = self.widths()
+        x = 8 * beam + 8
+        return dict(max_expansions=x, max_hyps=min(x * (beam_k + 1) + 8, _MAX_HYPS), max_nodes=(t + 1) * 2 * beam * beam_k + 64,
+                    max_states=(t + 1) * beam + 64, max_len=t + 64)
+
+    @torch.no_grad()
+    def decode_arrays(self, encoder_output: torch.Tensor, encoded_lengths: torch.Tensor, caps: Optional[Dict[str, int]] = None):
+        """Device-side result (enqueue-only): n_hyps (B), lengths (B, X), tokens / timesteps (B, X, L) int32, scores (B, X)
+        fp64, h / c (B, X, H) fp32, stats (B, 4) int32, flags (1); X = max_expansions, L = max_len of ``caps``."""
+        jn = self.joint
+        if encoder_output.dim() != 3 or encoder_output.size(1) != jn.encoder_hidden:
+            raise TypeError(f"encoder_output must be (B, {jn.encoder_hidden}, T), got {tuple(encoder_output.shape)}")
+        if not encoder_output.is_cuda:
+            raise RuntimeError("BeamRNNTInfer (B200) has no CPU path: encoder_output must be a CUDA tensor")
+        device = encoder_output.device
+        if self._packed is None or self._packed[2] != device or self._packed[3] != self._fingerprint():
+            self._prepare(device)
+        w = self._packed[0]
+        b, d, t = encoder_output.shape
+        caps = dict(self.default_caps(t), **(caps or {}))
+        c = _lib.CfbRnntBeamCaps()
+        for k, v in caps.items():
+            setattr(c, k, int(v))
+        x = encoder_output.transpose(1, 2)
+        if x.dtype not in (torch.float32, torch.bfloat16):
+            x = x.float()
+        x = x.contiguous()
+        lens = encoded_lengths.to(device=device, dtype=torch.int32).contiguous()
+        lib = _lib.load_library()
+        need = lib.cfb_rnnt_beam_scratch_bytes(d, w.pred_hidden, w.joint_hidden, w.num_classes_with_blank, b, t,
+                                               ctypes.byref(c)) + 256
+        if self._scratch is None or self._scratch.numel() < need or self._scratch.device != device:
+            self._scratch = torch.empty(need, dtype=torch.uint8, device=device)
+        sptr = (self._scratch.data_ptr() + 255) // 256 * 256
+        X, L, H = c.max_expansions, c.max_len, w.pred_hidden
+        i32 = dict(dtype=torch.int32, device=device)
+        out = dict(n_hyps=torch.empty(b, **i32), lengths=torch.zeros(b, X, **i32), tokens=torch.empty(b, X, L, **i32),
+                   timesteps=torch.empty(b, X, L, **i32), scores=torch.empty(b, X, dtype=torch.float64, device=device),
+                   h=torch.empty(b, X, H, dtype=torch.float32, device=device),
+                   c=torch.empty(b, X, H, dtype=torch.float32, device=device), stats=torch.empty(b, 4, **i32),
+                   flags=torch.zeros(1, **i32))
+        vp = lambda tensor: ctypes.c_void_p(tensor.data_ptr())
+        with torch.cuda.device(device):
+            rc = lib.cfb_op_rnnt_beam(ctypes.byref(w), vp(x), _lib.CFB_F32 if x.dtype == torch.float32 else _lib.CFB_BF16,
+                                      vp(lens), b, t, self.beam_size, int(bool(self.score_norm)), self.softmax_temperature,
+                                      ctypes.byref(c), vp(out["n_hyps"]), vp(out["lengths"]), vp(out["tokens"]),
+                                      vp(out["timesteps"]), vp(out["scores"]), vp(out["h"]), vp(out["c"]), vp(out["stats"]),
+                                      vp(out["flags"]), ctypes.c_void_p(sptr), need - 256,
+                                      ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream))
+        _lib.check(rc, None, "cfb_op_rnnt_beam")
+        out["_keepalive"] = (x, lens)
+        out["caps"] = caps
+        off = sptr - self._scratch.data_ptr()
+        out["phase_cycles"] = self._scratch[off + 64:off + 192].view(torch.int64)  # CTA 0's clocks per phase (debugging)
+        return out
+
+    @torch.no_grad()
+    def forward(self, encoder_output: torch.Tensor, encoded_lengths: torch.Tensor,
+                partial_hypotheses: Optional[List[Hypothesis]] = None):
+        if partial_hypotheses is not None:
+            raise NotImplementedError("BeamRNNTInfer (B200): partial_hypotheses")
+        t = encoder_output.size(2)
+        caps = self.default_caps(t)
+        for _ in range(24):
+            out = self.decode_arrays(encoder_output, encoded_lengths, caps)
+            flags = int(out["flags"].cpu())  # the one synchronisation of the decode
+            if flags == 0:
+                break
+            # some utterance outgrew a capacity: run again with the exhausted ones grown
+            if flags & 4 and caps["max_hyps"] >= _MAX_HYPS:
+                raise NotImplementedError(f"BeamRNNTInfer (B200): a frame needs more than {_MAX_HYPS} list entries "
+                                          "(the hypothesis lists live in shared memory)")
+            caps = dict(caps)
+            for bit, k in ((2, "max_expansions"), (4, "max_hyps"), (8, "max_nodes"), (16, "max_states"), (32, "max_len")):
+                if flags & bit:
+                    caps[k] *= 4
+            if flags & 2:  # more expansions per frame also need longer lists
+                caps["max_hyps"] = max(caps["max_hyps"], caps["max_expansions"] * (self.widths()[1] + 1) + 8)
+            caps["max_hyps"] = min(caps["max_hyps"], _MAX_HYPS)
+        else:
+            raise RuntimeError(f"BeamRNNTInfer (B200): capacities still exceeded after growing them to {caps}")
+        self.last_caps = caps  # what this batch needed (pass to decode_arrays to skip the growth next time)
+        n = out["n_hyps"].cpu()
+        lengths, tokens, steps = out["lengths"].cpu(), out["tokens"].cpu(), out["timesteps"].cpu()
+        scores, h, c = out["scores"].cpu(), out["h"].cpu(), out["c"].cpu()
+        lens_cpu = encoded_lengths.to("cpu")
+        greedy = self.beam_size == 1
+        H = h.size(-1)
+        hypotheses = []
+        for i in range(n.size(0)):
+            nbest = []
+            for r in range(int(n[i])):
+                k = int(lengths[i, r])
+                emitted = k > 0
+                state = (h[i, r].view(1, 1, H).clone(), c[i, r].view(1, 1, H).clone()) if (emitted or not greedy) else None
+                nbest.append(Hypothesis(score=float(scores[i, r]), y_sequence=tokens[i, r, :k].long().clone(),
+                                        timestep=steps[i, r, :k].tolist(), dec_state=state, length=lens_cpu[i]))
+            hypotheses.append(nbest[0] if self.return_best_hypothesis else NBestHypotheses(nbest))
+        return (hypotheses,)
 
 
 class GreedyRNNTInfer(GreedyBatchedRNNTInfer):

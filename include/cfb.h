@@ -252,6 +252,47 @@ CFB_API int cfb_op_rnnt_greedy(const cfb_rnnt_weights* w, const void* encoded, i
                        float* scores, float* h_out, float* c_out, int32_t* flags, void* scratch, size_t scratch_bytes,
                        cfb_stream stream);
 
+/* ---- Transducer beam search on the encoder output (decoding.strategy = beam, search_type = default) ---------------------
+ * BeamRNNTInfer.default_beam_search, and greedy_search for beam_size == 1, with sort_nbest, run for every utterance of the
+ * batch (parts/submodules/rnnt_beam_decoding.py; restated in oracle/rnnt_beam_oracle.py) in one persistent cooperative
+ * kernel (csrc/rnnt_beam.cu).  Same weights (cfb_rnnt_weights) and joint.enc GEMM as cfb_op_rnnt_greedy.
+ * Capacities bound the per-utterance device state; an utterance that would exceed one stops and sets flags bit 0, and the
+ * caller runs the call again with larger capacities (stats tells how much was used). */
+typedef struct cfb_rnnt_beam_caps {
+  int32_t max_expansions; /* hypotheses expanded per frame; also the n-best rows per utterance of the outputs        */
+  int32_t max_hyps;       /* entries of each of the `hyps` / `kept` lists (<= 2048; kept in shared memory)           */
+  int32_t max_nodes;      /* prefix-tree nodes per utterance (one per non-blank extension, plus the initial blank)    */
+  int32_t max_states;     /* prediction-network outputs per utterance (one per distinct label sequence expanded)      */
+  int32_t max_len;        /* labels per output hypothesis (y_sequence, its leading blank included)                    */
+  int32_t reserved[3];
+} cfb_rnnt_beam_caps;
+
+CFB_API size_t cfb_rnnt_beam_scratch_bytes(int enc_hidden, int pred_hidden, int joint_hidden, int num_classes_with_blank, int B,
+                                   int T, const cfb_rnnt_beam_caps* caps);
+/*   encoded      (B, T, E) row-major = the contiguous encoder output, CFB_F32 or CFB_BF16;  encoded_len (B) int32
+ *   beam_size    BeamRNNTInfer's beam_size (>= 1; 1 = greedy_search, up to 5 labels per frame);  beam = min(beam_size, V + 1)
+ *                hypotheses end a frame, beam_k = min(beam, V) non-blank candidates extend each expansion (<= 64)
+ *   score_norm   sort the n-best list by score / len(y_sequence) (non-zero) or by score
+ *   temperature  softmax_temperature: log_softmax(joint / temperature) (> 0)
+ *   caps         host pointer, read during the call only
+ * Outputs (device), X = caps->max_expansions, L = caps->max_len; row (b, r) is the r-th hypothesis of sort_nbest's list:
+ *   n_hyps       (B) int32 hypotheses in the list (0 for an utterance that stopped on a capacity)
+ *   lengths      (B, X) int32 labels of each hypothesis;  tokens, timesteps (B, X, L) int32 = Hypothesis.y_sequence and
+ *                .timestep (beam: the leading blank and its -1 included; greedy_search: neither)
+ *   scores       (B, X) double = Hypothesis.score (accumulated in double, like the reference's Python floats)
+ *   h_out, c_out (B, X, H) = Hypothesis.dec_state: the LSTM state the hypothesis's last label is predicted from (zeros for
+ *                the initial hypothesis)
+ *   stats        (B, 4) int32: expansions, prefix-tree nodes, state slots, most expansions at one frame
+ *   flags        (1) int32, caller-zeroed; bit 0: some utterance exceeded a capacity, and which one: bit 1 max_expansions,
+ *                bit 2 max_hyps, bit 3 max_nodes, bit 4 max_states, bit 5 max_len
+ *   scratch      >= cfb_rnnt_beam_scratch_bytes(...), 256-byte aligned.  Enqueue-only on `stream`; CFB_ERR_UNSUPPORTED when
+ *                the device has no cooperative launch, the fp32 weights and lists do not fit in the SMs' shared memory, or
+ *                beam_k / max_hyps exceed the limits above. */
+CFB_API int cfb_op_rnnt_beam(const cfb_rnnt_weights* w, const void* encoded, int x_dtype, const int32_t* encoded_len, int B,
+                     int T, int beam_size, int score_norm, float temperature, const cfb_rnnt_beam_caps* caps,
+                     int32_t* n_hyps, int32_t* lengths, int32_t* tokens, int32_t* timesteps, double* scores, float* h_out,
+                     float* c_out, int32_t* stats, int32_t* flags, void* scratch, size_t scratch_bytes, cfb_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -160,6 +160,9 @@ int launch_subsample_first(const void* feats, bool feats_bf16, const float* w9, 
                            bool out_bf16, int B, int F, int T, int C, int T1, int F1, int Th, int Fh, cudaStream_t st);
 // tensor-core form of the first conv: rows [x_hi(9) | x_lo(9) | 1 | 1 | 0 x 4] (bf16, 24 columns) in y1's row order
 constexpr int kConv0Cols = 24;
+// The gather kernels of the first conv (subsample_first_kernel, conv0_im2col_kernel, conv0_im2col_packed_kernel) stage
+// (F + 2) x 34 fp32 features of a block in shared memory, inside the 48 KB a launch gets without opting in: F <= 359.
+constexpr int kMaxFeatIn = 359;
 int launch_conv0_im2col(const void* feats, bool feats_bf16, void* a0, int B, int F, int T, int T1, int F1, int Th, int Fh,
                         cudaStream_t st);
 // validation path: gather the 3x3/s2 patches of a parity-split tensor into a dense (rows x 9*C) fp32 matrix

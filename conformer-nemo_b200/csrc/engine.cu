@@ -263,6 +263,9 @@ int cfb_create(const cfb_config* cfg, int device, cfb_handle** out) {
   };
   if (cfg->feat_in < 1 || cfg->n_layers < 1 || cfg->d_model < 16 || cfg->n_heads < 1 || cfg->ff_expansion_factor < 1)
     return bad(CFB_ERR_INVALID_ARG, "feat_in, n_layers, d_model, n_heads and ff_expansion_factor must be positive");
+  if (cfg->feat_in > kMaxFeatIn)
+    return bad(CFB_ERR_UNSUPPORTED, "feat_in > " + std::to_string(kMaxFeatIn) +
+                                        " is not supported (the first conv stages (feat_in + 2) x 34 fp32 features of a block in 48 KB of shared memory)");
   if (cfg->d_model % cfg->n_heads) return bad(CFB_ERR_INVALID_ARG, "d_model must be divisible by n_heads");
   if (cfg->subsampling_factor != 4)
     return bad(CFB_ERR_UNSUPPORTED, "only subsampling_factor=4 (two strided convolutions) is supported");
@@ -1216,6 +1219,12 @@ int cfb_op_layernorm(const float* x, const float* gamma, const float* beta, void
   int rc = launch_layernorm(x, gamma, beta, out, out_dtype == CFB_BF16, rows, d, lens, frames_per_seq > 0 ? frames_per_seq : 1,
                             reinterpret_cast<cudaStream_t>(stream));
   return rc == 0 ? CFB_OK : op_fail(rc, rc == -1 ? "layernorm: d must be a multiple of 4 and <= 1024" : "");
+}
+
+int cfb_op_layernorm_dual(const float* x, const float* g1, const float* b1, float* out1, const float* g2, const float* b2,
+                          void* out2_bf16, int rows, int d, cfb_stream stream) {
+  int rc = launch_layernorm_dual(x, g1, b1, out1, g2, b2, out2_bf16, rows, d, reinterpret_cast<cudaStream_t>(stream));
+  return rc == 0 ? CFB_OK : op_fail(rc, rc == -1 ? "layernorm_dual: d must be a multiple of 4 and <= 1024" : "");
 }
 
 int cfb_op_depthwise(const void* x, const float* taps, const float* bias, void* out, int dtype, int B, int T, int d,

@@ -79,6 +79,7 @@ __global__ void __launch_bounds__(kPlanThreads) packed_plan_kernel(const long lo
 // Same row format as conv0_im2col_kernel (elementwise.cu): [x_hi (9) | x_lo (9) | 1 | 1 | 0 0 0 0] per output position,
 // in the row order of the parity-split y1 of ONE virtual sequence of 2 * n_rows first-conv rows.
 constexpr int kS1T = 16;  // t1 rows per block = kPackAlign token rows
+static_assert((kMaxFeatIn + 2) * (2 * kS1T + 2) * sizeof(float) <= 48 * 1024, "feature patch must fit the default shared memory");
 constexpr int kA0Cols = kConv0Cols;
 
 template <typename TIn>

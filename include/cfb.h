@@ -54,7 +54,7 @@ typedef enum cfb_precision {
 /* Mirrors the keyword arguments of ConformerEncoder.__init__ (conformer_encoder.py:111-132).  Dropouts are
  * identity at inference and have no field.  Unsupported values make cfb_create return CFB_ERR_UNSUPPORTED. */
 typedef struct cfb_config {
-  int32_t feat_in;                   /* mel bins, e.g. 80                                                     */
+  int32_t feat_in;                   /* mel bins, e.g. 80; 1 ... 359                                          */
   int32_t n_layers;
   int32_t d_model;
   int32_t feat_out;                  /* -1 (or == d_model): no out_proj (conformer_encoder.py:209-214)         */
@@ -164,6 +164,11 @@ CFB_API int cfb_op_gemm(int use_tensor_cores, int epilogue, const void* A, int64
  * out_dtype CFB_BF16 / CFB_F32.  lens != NULL: rows at frames >= lens[seq] are written as zeros. */
 CFB_API int cfb_op_layernorm(const float* x, const float* gamma, const float* beta, void* out, int out_dtype, int rows,
                      int d, const int32_t* lens, int frames_per_seq, cfb_stream stream);
+
+/* norm_out of one layer followed by norm_feed_forward1 of the next (conformer_modules.py:120, :98) in one pass:
+ * out1 = LayerNorm(x; g1, b1) fp32 (may alias x), out2 = LayerNorm(out1; g2, b2) bf16.  rows x d, d % 4 == 0, d <= 1024. */
+CFB_API int cfb_op_layernorm_dual(const float* x, const float* g1, const float* b1, float* out1, const float* g2,
+                                  const float* b2, void* out2_bf16, int rows, int d, cfb_stream stream);
 
 /* Depth-wise time convolution with folded BatchNorm + Swish (conformer_modules.py:168-177).
  * x, out: (B, T, d) in `dtype` (CFB_BF16 / CFB_F32); taps (ksize, d) fp32, tap-major; bias (d) fp32; zero padding at

@@ -41,6 +41,16 @@ def op_layernorm(x, gamma, beta, out, lens=None, frames_per_seq=1):
     return out
 
 
+def op_layernorm_dual(x, g1, b1, out1, g2, b2, out2):
+    """out1 = LN(x; g1, b1) fp32 (may be x itself), out2 = LN(out1; g2, b2) bf16 (cfb_op_layernorm_dual)."""
+    lib = _lib.load_library()
+    rows, d = x.shape
+    rc = lib.cfb_op_layernorm_dual(ptr(x), ptr(g1), ptr(b1), ptr(out1), ptr(g2), ptr(b2), ptr(out2), rows, d, stream())
+    assert rc == 0, _lib.last_error(None)
+    torch.cuda.synchronize()
+    return out1, out2
+
+
 def op_depthwise(x, taps, bias, out):
     """taps given as (d, ksize) like the reference's depthwise_conv.weight; the kernel wants them tap-major."""
     lib = _lib.load_library()

@@ -6,7 +6,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from gpu_util import err_stats, op_depthwise, op_layernorm, op_lengths
+from gpu_util import err_stats, op_depthwise, op_layernorm, op_layernorm_dual, op_lengths
 
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
@@ -68,3 +68,47 @@ def test_lengths_bit_exact_against_reference_golden():
     # length=None: every row is T_full
     got = op_lengths(None, 5, 2001, 2)
     assert got.tolist() == [501] * 5
+
+
+def _bf16_ulp(got, want):
+    _, e = torch.frexp(torch.maximum(got.abs(), want.abs()))
+    return torch.ldexp(torch.ones_like(got), e - 8)
+
+
+@pytest.mark.parametrize("d", [16, 64, 144, 176, 256, 512, 1024])
+@pytest.mark.parametrize("offset,scale", [(0.0, 1.0), (1e3, 0.1)])
+def test_layernorm_dual_in_place_against_fp64(d, offset, scale):
+    """norm_out + the next layer's norm_feed_forward1 in one kernel, in place as the engine runs it (out1 == x), against
+    LN2(LN1(x)) in fp64.  A large common offset (mean 1e3, std 0.1) is where a plain fp32 sum of the row loses the
+    mean (~1e-3 at the output); the kernel sums x - x[0] instead."""
+    torch.manual_seed(d)
+    rows = 333  # not a multiple of the 8 rows of a block
+    x = torch.randn(rows, d, device="cuda", dtype=torch.float64) * scale + offset
+    x = x.float()
+    g1, b1 = torch.randn(d, device="cuda"), torch.randn(d, device="cuda")
+    g2, b2 = torch.randn(d, device="cuda"), torch.randn(d, device="cuda")
+
+    def ln64(v, g, b):
+        v = v.double()
+        m = v.mean(-1, keepdim=True)
+        return (v - m) / torch.sqrt(((v - m) ** 2).mean(-1, keepdim=True) + 1e-5) * g.double() + b.double()
+
+    want1 = ln64(x, g1, b1)
+    want2 = ln64(want1, g2, b2)
+    y = x.clone()
+    out2 = torch.full((rows, d), float("nan"), device="cuda", dtype=torch.bfloat16)
+    op_layernorm_dual(y, g1, b1, y, g2, b2, out2)
+    assert float((y.double() - want1).abs().max()) < 2e-5
+    o2 = out2.double()
+    assert not torch.isnan(o2).any()
+    assert torch.all((o2 - want2).abs() <= _bf16_ulp(o2, want2) + 2e-5)
+    # Against cfb_op_layernorm applied twice: the same formula, but not the same bits.  The dual kernel gives lane l the
+    # float4 columns l, l + 32, ... and sums x - x[0]; layernorm_kernel gives it the pairs 2l, 2l + 1, 2l + 64, ... and
+    # sums x itself, so the two reductions round differently.  Without the offset both meet the same fp64 bound.
+    if offset == 0.0:
+        t1 = torch.empty_like(x)
+        t2 = torch.empty(rows, d, device="cuda", dtype=torch.bfloat16)
+        op_layernorm(x, g1, b1, t1)
+        op_layernorm(t1, g2, b2, t2)
+        assert float((t1.double() - want1).abs().max()) < 2e-5
+        assert torch.all((t2.double() - want2).abs() <= _bf16_ulp(t2.double(), want2) + 2e-5)

@@ -440,3 +440,57 @@ def test_profile_report_from_eager_brackets_and_from_graph_nodes():
     assert {k: v[0] for k, v in nodes.items()} == {k: v[0] for k, v in eager.items()}
     assert all(v[1] > 0.0 for v in nodes.values())
     assert torch.equal(y2, y0)
+
+
+# The configuration surface cfb_create accepts beyond the shipped recipes: any feat_in <= 359 (odd ones pad the
+# odd-f1 plane and leave a partial output tile in the second conv), subsampling channels C that leave a partial 64-channel
+# chunk, head dimensions 48 / 40 / 36 / 4, d_model 1024 (LayerNorm at its widest, no fused conv tail, d_ff 4096), odd
+# kernel sizes down to 1, ff_expansion_factor 1 and 3, and feat_out below and above d_model.
+# feat_in, C, d_model, heads, layers, conv_kernel_size, ff_expansion_factor, feat_out, T, lengths
+SURFACE = [
+    (64, 8, 80, 2, 2, 31, 4, -1, 203, [203, 150]),
+    (128, 24, 144, 4, 1, 3, 1, -1, 160, [160, 97, 0]),
+    (81, 72, 48, 1, 2, 1, 3, -1, 333, [333, 1, 200]),
+    (41, -1, 64, 16, 2, 31, 4, 8, 120, [120, 77]),
+    (359, 8, 64, 4, 1, 31, 4, -1, 99, [99, 64, 33]),
+    (80, 72, 1024, 16, 1, 31, 4, -1, 140, [140, 101]),
+    (81, 24, 176, 4, 1, 3, 3, 640, 257, [257, 190, 2]),
+    (41, 8, 96, 2, 2, 1, 1, -1, 400, [400, 311]),
+]
+
+
+@pytest.mark.parametrize("row", SURFACE, ids=[f"F{r[0]}-C{r[1]}-d{r[2]}h{r[3]}L{r[4]}-k{r[5]}-ff{r[6]}-out{r[7]}" for r in SURFACE])
+def test_accepted_configuration_surface_against_oracle(row):
+    feat_in, C, d, heads, layers, ks, ff, feat_out, t, lens = row
+    cfg = oc.EncoderConfig(feat_in=feat_in, n_layers=layers, d_model=d, n_heads=heads, subsampling_conv_channels=C,
+                           conv_kernel_size=ks, ff_expansion_factor=ff, feat_out=feat_out)
+    sd = oc.random_state_dict(cfg, 80 + feat_in)
+    x, length = oc.synthetic_batch(len(lens), feat_in, t, lens, seed=90 + feat_in)
+    g = torch.Generator().manual_seed(feat_in)
+    for b, n in enumerate(lens):  # non-zero features behind every utterance: the convolutions run over the padded batch
+        x[b, :, n:] = torch.randn(feat_in, t - n, generator=g)
+    want, want_len = oc.encoder_forward(sd, cfg, x, length)
+    for prec in ("fp32_validate", "bf16"):
+        enc = build(cfg, sd, prec)
+        enc.packed = False
+        y, ylen = enc(audio_signal=x.cuda(), length=length.cuda())
+        torch.cuda.synchronize()
+        assert torch.equal(ylen.cpu(), want_len), (prec, ylen, want_len)
+        st = compare(y.cpu(), want, ylen)
+        if prec == "fp32_validate":
+            assert st["nan"] == 0 and st["rel_l2"] < 1e-4 and st["max_abs"] < 1e-4 * max(1.0, float(want.abs().max())), st
+        else:
+            assert st["nan"] == 0 and st["rel_l2"] <= 1e-2 and st["max_abs"] <= 5e-2, st
+        m = valid_mask(ylen, y.shape[2])[:, None, :].expand_as(y)
+        assert torch.all(y.cpu()[~m] == 0)
+    if feat_out > 0 and feat_out != d:
+        return  # out_proj runs dense batches only
+    yd = y.clone()
+    enc.packed = True
+    yp, ylp = enc(audio_signal=x.cuda(), length=length.cuda(), length_host=lens)
+    torch.cuda.synchronize()
+    assert torch.equal(ylp, ylen)
+    for b in range(len(lens)):
+        n = int(ylen[b])
+        assert torch.equal(yd[b, :, :n], yp[b, :, :n]), (b, float((yd[b, :, :n] - yp[b, :, :n]).abs().max()))
+        assert n == yp.shape[2] or float(yp[b, :, n:].abs().max()) == 0.0

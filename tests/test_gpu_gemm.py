@@ -32,7 +32,9 @@ def test_tc_linear_exact_on_integers(M, N, K):
 
 
 @pytest.mark.parametrize("use_tc", [False, True])
-@pytest.mark.parametrize("M,N,K", [(300, 192, 176), (513, 512, 512)])
+@pytest.mark.parametrize("M,N,K", [(300, 192, 176), (513, 512, 512),
+                                   # pre_encode.out: K = F2 * C (F2 = 20 at 80 mel bins; 21 at 81, 11 at 41)
+                                   (406, 256, 5120), (300, 176, 3696), (77, 64, 168), (1000, 512, 10240)])
 def test_linear_bias(use_tc, M, N, K):
     A, W = _mk(M, N, K, seed=1)
     bias = torch.randn(N, device="cuda")
@@ -43,6 +45,15 @@ def test_linear_bias(use_tc, M, N, K):
         op_gemm(True, _lib.EPI_LINEAR, Ab, Wb, bias=bias, out=out)
         st = err_stats(out.float(), want)
         assert st["nan"] == 0 and st["rel_l2"] < 4e-3, st
+        # fp32 output (as pre_encode.out writes the residual stream): K products and the bias summed in fp32 are off by
+        # at most K * 2^-24 * sum |a w| (+ |bias|) from the exact sum of the bf16 operands
+        out32 = torch.full((M, N), float("nan"), device="cuda")
+        op_gemm(True, _lib.EPI_LINEAR, Ab, Wb, bias=bias, out=out32)
+        a64, w64 = Ab.double(), Wb.double()
+        want64 = a64 @ w64.t() + bias.double()
+        bound = K * 2.0 ** -24 * (a64.abs() @ w64.abs().t() + bias.double().abs())
+        bad = (out32.double() - want64).abs() > bound
+        assert not torch.isnan(out32).any() and not bad.any(), f"{int(bad.sum())} elements out of bound, first {bad.nonzero()[:4].tolist()}"
     else:
         want = A @ W.t() + bias
         out = torch.zeros(M, N, device="cuda")

@@ -111,6 +111,11 @@ def test_unsupported_config_is_rejected_by_the_library(lib):
     cfg.d_model = 60
     assert lib.cfb_create(ctypes.byref(cfg), 0, ctypes.byref(handle)) in (1, 2)
     assert lib.cfb_create(None, 0, ctypes.byref(handle)) == 1
+    # the first conv's gathers stage (feat_in + 2) x 34 fp32 values in 48 KB of shared memory: feat_in <= 359
+    cfg.d_model = 64
+    cfg.feat_in = 360
+    assert lib.cfb_create(ctypes.byref(cfg), 0, ctypes.byref(handle)) == 2
+    assert "feat_in > 359" in _lib.last_error(None)
 
 
 def test_constructor_surface_and_errors():

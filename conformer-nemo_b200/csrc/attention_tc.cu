@@ -68,8 +68,6 @@ struct AttnParams {
   int T, Dp;
   const int4* tiles;  // packed batches: blockIdx.x -> (sequence, i0, first token row of its slot, rows in the slot)
   float scale_log2;  // log2(e) / sqrt(dk)
-  int debug;         // CFB_ATTN_DEBUG ablation bits (timing experiments only; results are wrong when non-zero)
-  long long* trace;  // CFB_ATTN_TRACE=1: clock64 trace of CTA (0,0,0) (timing experiments only)
 };
 
 __device__ __forceinline__ float fast_exp2(float x) {
@@ -121,8 +119,6 @@ __host__ __device__ constexpr uint32_t make_idesc_f16_f16acc(int m, int n) {
   return (static_cast<uint32_t>(n >> 3) << 17) | (static_cast<uint32_t>(m >> 4) << 24);
 }
 
-// kInstr: clock trace + ablation switches (timing experiments only)
-template <bool kInstr>
 __global__ void __launch_bounds__(kThreads, 1)
 rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_constant__ CUtensorMap tmP,
                    const AttnParams p) {
@@ -134,10 +130,6 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
   // warp and lane index -- several times per key tile in the softmax warps (ncu source page); a shuffle result it keeps.
   const int warp = __shfl_sync(0xffffffffu, static_cast<int>(tid >> 5), 0);
   const int lane = __shfl_sync(0xffffffffu, static_cast<int>(tid & 31), static_cast<int>(tid & 31));
-  const bool trc = kInstr && p.trace != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && lane == 0;
-  const int dbg = kInstr ? p.debug : 0;
-#define CFB_TR(slot) do { if (kInstr && trc) p.trace[slot] = clock64(); } while (0)
-  if (warp == 4) CFB_TR(0);
 
   extern __shared__ uint8_t smem_raw[];
   // every shared-memory object is addressed through a 32-bit shared address derived once from this base
@@ -244,7 +236,6 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
   ptx::tc_fence_after();
   uint32_t tmem_base;
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
-  if (warp == 4) CFB_TR(1);
 
   if (!active) {
     if (warp >= 4 && warp < 8) {
@@ -294,28 +285,22 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
       int it = 0;
       for (int kt = s; kt < n_kt; kt += 2, ++it) {
         const int kvs = kt % kKVStages;
-        const bool ti = kInstr && s == 0 && it < 30;
         const uint32_t st = sbase + kOffKV + kvs * kKVBytes;
         const uint64_t dK = ptx::make_sdesc_sw128(st, 16, 1024);
         // V tile: 64 keys (K of this MMA) x 64 dk (N), 128-byte rows along N -> MN-major, 8-key groups 1 KB apart
         const uint64_t dV = ptx::make_sdesc_sw128(st + kKBytes, 1024, 1024);
-        if (ti) CFB_TR(512 + it * 8 + 0);
         ptx::mbar_wait_a(kv_full + 8 * kvs, (kt / kKVStages) & 1);
-        if (ti) CFB_TR(512 + it * 8 + 1);
         ptx::mbar_wait_a(s_free + 8 * s, (it & 1) ^ 1);
         ptx::tc_fence_after();
-        if (ti) CFB_TR(512 + it * 8 + 2);
         if (ptx::elect_one()) {
 #pragma unroll
           for (int k = 0; k < kDK / 16; ++k) ptx::umma_bf16_ts(tS, tQu + 8 * k, dK + 2 * k, idesc_s, k != 0);
           ptx::tc_commit_a(sg_full + 8 * s);
         }
         __syncwarp();
-        if (ti) CFB_TR(512 + it * 8 + 3);
         // ---- O_part = P V once the set has stored its probabilities (P is a TMEM A operand: 8 columns per K=16)
         ptx::mbar_wait_a(p_ready + 8 * s, it & 1);
         ptx::tc_fence_after();
-        if (ti) CFB_TR(512 + it * 8 + 4);
         if (ptx::elect_one()) {
 #pragma unroll
           for (int k = 0; k < kBN / 16; ++k)
@@ -324,7 +309,6 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
           ptx::tc_commit_a(kv_empty + 8 * kvs);
         }
         __syncwarp();
-        if (ti) CFB_TR(512 + it * 8 + 5);
       }
     } else {
       // ---------------------------------------------------------------------------------- G ring issuer
@@ -351,7 +335,6 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
         ptx::tc_commit_a(band_empty + 16);
       }
       __syncwarp();
-      CFB_TR(800 + 2);
       for (int g = 3; g < n_gb; ++g) {
         const int bs = g % kBandSlots;
         const uint64_t dB = ptx::make_sdesc_sw128(band_base + bs * kBlockBytes, 16, 1024);
@@ -369,7 +352,6 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
           ptx::tc_commit_a(band_empty + 8 * bs);
         }
         __syncwarp();
-        if (g < 30) CFB_TR(800 + g);
       }
     }
   } else {
@@ -396,7 +378,6 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
     ptx::tc_fence_before();
     __syncwarp();
     if (lane == 0) ptx::mbar_arrive_a(set == 0 ? qu_ready : qv_ready);
-    if (warp == 4) CFB_TR(2);
 
     // rel_shift: row ii needs window column (31 - lane) + jj of the 96 columns starting at ring column
     // 64 kt + 96 - 32 quarter.  The window goes through a private fp32 shared-memory row: stored with 16-byte
@@ -408,36 +389,27 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
                                static_cast<uint32_t>(((lane >> 1) + 4 * (lane & 1)) & 7) * 16;
     const int wcol = 96 - 32 * quarter;  // window start inside the concatenation of ring blocks kt, kt+1, kt+2
 
-    auto fetch_window = [&](int kt, int tslot) {
+    auto fetch_window = [&](int kt) {
       ptx::mbar_wait_a(g_full + 8 * ((kt + 2) % kGSlots), ((kt + 2) / kGSlots) & 1);  // blocks complete in order
       ptx::tc_fence_after();
-      if (tslot) CFB_TR(tslot);
       uint32_t w[49];
-      if (dbg & 32) {
 #pragma unroll
-        for (int c = 0; c < 48; ++c) w[c] = 0u;
-      } else {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-          const int wc = wcol + 32 * c;
-          const int blk = kt + (wc >> 6);
-          ptx::tmem_ld_x16_pack16(t_lane + kColG + (blk % kGSlots) * 64 + (wc & 63), &w[16 * c]);
-        }
-        ptx::tc_wait_ld();
+      for (int c = 0; c < 3; ++c) {
+        const int wc = wcol + 32 * c;
+        const int blk = kt + (wc >> 6);
+        ptx::tmem_ld_x16_pack16(t_lane + kColG + (blk % kGSlots) * 64 + (wc & 63), &w[16 * c]);
       }
+      ptx::tc_wait_ld();
       w[48] = 0u;
-      if (tslot) CFB_TR(tslot + 1);
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive_a(g_free + 8 * set);
-      if (!(dbg & 2)) {
-        // odd shifts: move the row down by one half so that the halves (31 - lane) + 2 j, + 2 j + 1 share a word
-        const uint32_t sel = (sh & 1) ? 0x5432u : 0x3210u;
+      // odd shifts: move the row down by one half so that the halves (31 - lane) + 2 j, + 2 j + 1 share a word
+      const uint32_t sel = (sh & 1) ? 0x5432u : 0x3210u;
 #pragma unroll
-        for (int m = 0; m < 48; ++m) w[m] = prmt(w[m], w[m + 1], sel);
+      for (int m = 0; m < 48; ++m) w[m] = prmt(w[m], w[m + 1], sel);
 #pragma unroll
-        for (int q = 0; q < 12; ++q) ptx::sts128(shift_row + q * 16, w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
-      }
+      for (int q = 0; q < 12; ++q) ptx::sts128(shift_row + q * 16, w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
     };
 
     float o_acc[kDK];
@@ -446,31 +418,21 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
     float m_run = -INFINITY, l_run = 0.f;
     const float scale = p.scale_log2;
 
-    if (set < n_kt) fetch_window(set, 0);
-    if (warp == 4) CFB_TR(3);
+    if (set < n_kt) fetch_window(set);
     int it = 0;
     for (int kt = set; kt < n_kt; kt += 2, ++it) {
       const int j0 = kt * kBN;
-      const bool ts = kInstr && warp == 4 && it < 30;
-      if (ts) CFB_TR(16 + it * 16 + 0);
       // the shifted window row was stored a whole P V MMA ago: read it while the S MMA of this tile is still in flight
       uint32_t gw[32];
-      if (dbg & 4) {
-#pragma unroll
-        for (int c = 0; c < 32; ++c) gw[c] = 0u;
-      } else {
-        lds_u32x32(shift_row + (sh >> 1) * 4, gw);
-      }
+      lds_u32x32(shift_row + (sh >> 1) * 4, gw);
       ptx::mbar_wait_a(sg_full + 8 * set, it & 1);
       ptx::tc_fence_after();
-      if (ts) CFB_TR(16 + it * 16 + 1);
       float sv[kBN];
       {
         uint32_t s0r[32], s1r[32];
         ptx::tmem_ld_x32(tS, s0r);
         ptx::tmem_ld_x32(tS + 32, s1r);
         ptx::tc_wait_ld();
-        if (ts) CFB_TR(16 + it * 16 + 10);
 #pragma unroll
         for (int c = 0; c < 16; ++c) {  // s + 16 g, g an fp16 half of the packed window word (FHFMA: no conversion)
           ptx::fhfma_pair(gw[c], kGScaleH, __uint_as_float(s0r[2 * c]), __uint_as_float(s0r[2 * c + 1]), sv[2 * c], sv[2 * c + 1]);
@@ -478,7 +440,6 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
                           sv[32 + 2 * c + 1]);
         }
       }
-      if (ts) CFB_TR(16 + it * 16 + 2);
       if (j0 + kBN > len) {  // only the last key tile can contain masked keys
 #pragma unroll
         for (int c = 0; c < kBN; ++c)
@@ -487,8 +448,7 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
       // The exponentials of consecutive key tiles take turns on the MUFU pipe (tile kt after tile kt-1): the two
       // sets then stay in anti-phase, one in its MUFU phase while the other is in its shared-memory / TMEM phases,
       // instead of drifting into lock-step and halving each other's throughput in every phase.
-      if (kt > 0 && !(dbg & 8)) ptx::mbar_wait_a(exp_done + 8 * (set ^ 1), (set == 0 ? it - 1 : it) & 1);
-      if (ts) CFB_TR(16 + it * 16 + 11);
+      if (kt > 0) ptx::mbar_wait_a(exp_done + 8 * (set ^ 1), (set == 0 ? it - 1 : it) & 1);
       float mx4[4] = {sv[0], sv[1], sv[2], sv[3]};  // four independent chains instead of one 64-deep one
 #pragma unroll
       for (int c = 4; c < kBN; ++c) mx4[c & 3] = fmaxf(mx4[c & 3], sv[c]);
@@ -504,14 +464,13 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
 #pragma unroll
       for (int m = 0; m < 32; ++m) {
         const float2 a = ptx::ffma2(make_float2(sv[2 * m], sv[2 * m + 1]), scale2, nms2);
-        const float2 e = make_float2((dbg & 1) ? a.x : fast_exp2(a.x), (dbg & 1) ? a.y : fast_exp2(a.y));
+        const float2 e = make_float2(fast_exp2(a.x), fast_exp2(a.y));
         rs4[m & 3] = ptx::fadd2(rs4[m & 3], e);
         // bf16 pair without the conversion unit (it shares the MUFU pipe): round half up with integer adds, one PRMT
         pw[m] = prmt(__float_as_uint(e.x) + 0x8000u, __float_as_uint(e.y) + 0x8000u, 0x7632u);
       }
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive_a(exp_done + 8 * set);
-      if (ts) CFB_TR(16 + it * 16 + 3);
       ptx::tmem_st_x32(tP, pw);
       const float2 rs2 = ptx::fadd2(ptx::fadd2(rs4[0], rs4[1]), ptx::fadd2(rs4[2], rs4[3]));
       const float rsum = rs2.x + rs2.y;
@@ -521,24 +480,16 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive_a(p_ready + 8 * set);
-      if (ts) CFB_TR(16 + it * 16 + 4);
       // ---- the G window of this set's next tile, while the P V MMA runs
-      if (kt + 2 < n_kt) fetch_window(kt + 2, ts ? 16 + it * 16 + 8 : 0);
-      if (ts) CFB_TR(16 + it * 16 + 5);
+      if (kt + 2 < n_kt) fetch_window(kt + 2);
       // ---- o_acc = o_acc * alpha + O_part (the S columns of this set)
       ptx::mbar_wait_a(o_full + 8 * set, it & 1);
       ptx::tc_fence_after();
-      if (ts) CFB_TR(16 + it * 16 + 6);
       {
         uint32_t a0[32], a1[32];
-        if (dbg & 16) {
-#pragma unroll
-          for (int c = 0; c < 32; ++c) a0[c] = a1[c] = 0u;
-        } else {
-          ptx::tmem_ld_x32(tS, a0);
-          ptx::tmem_ld_x32(tS + 32, a1);
-          ptx::tc_wait_ld();
-        }
+        ptx::tmem_ld_x32(tS, a0);
+        ptx::tmem_ld_x32(tS + 32, a1);
+        ptx::tc_wait_ld();
 #pragma unroll
         for (int c = 0; c < 16; ++c) {
           const float2 x = ptx::ffma2(make_float2(o_acc[2 * c], o_acc[2 * c + 1]), alpha2,
@@ -551,13 +502,11 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive_a(s_free + 8 * set);  // the S columns may now receive the next tile's scores
-      if (ts) CFB_TR(16 + it * 16 + 7);
     }
 
     // ---- merge the two sets (log-sum-exp) and write the context rows.  Every MMA of the CTA has completed once
     // both sets are past their last o_full wait, so the K/V ring can carry the exchange (16-byte accesses,
     // 17-quad row pitch: conflict-free).
-    if (warp == 4) CFB_TR(4);
     asm volatile("bar.sync 1, 256;" ::: "memory");
     const uint32_t xrow = sbase + kOffKV + ii * kXPitch * 4;
     if (set == 1) {
@@ -592,18 +541,13 @@ rel_attn_tc_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_consta
     }
   }
 
-  if (warp == 4) CFB_TR(5);
   ptx::tc_fence_before();
   __syncthreads();
   if (warp == 1) {
     ptx::tc_fence_after();
     ptx::tmem_dealloc(tmem_base, kTmemCols);
   }
-  if (warp == 4) CFB_TR(6);
-#undef CFB_TR
 }
-
-long long* g_attn_trace = nullptr;
 
 }  // namespace
 
@@ -626,13 +570,6 @@ const void* attn_pos_f16(const AttnDesc& a, int Dp, cudaStream_t st) {
   return scratch[dev & 63];
 }
 
-// debug: copies the clock trace of the last traced launch to the host (1024 values)
-extern "C" __attribute__((visibility("default"))) int cfb_debug_attn_trace(long long* host_out) {
-  if (!g_attn_trace) return 1;
-  cudaDeviceSynchronize();
-  return cudaMemcpy(host_out, g_attn_trace, 1024 * sizeof(long long), cudaMemcpyDeviceToHost) == cudaSuccess ? 0 : 2;
-}
-
 int launch_attn_tc(const AttnDesc& a, cudaStream_t st, std::string* err) {
   if ((a.tiles == nullptr && a.B <= 0) || a.T <= 0) return 0;
   {
@@ -640,11 +577,10 @@ int launch_attn_tc(const AttnDesc& a, cudaStream_t st, std::string* err) {
     // 93.3 -> 92.1 us, 1 x 7500 x 8 477 -> 504 us: it removes the per-CTA setup, which matters for short sequences; the
     // per-item time is set by the softmax warps' serial work either way.  CFB_ATTN_PERSIST=1 / 0 forces.
     const char* pv = getenv("CFB_ATTN_PERSIST");
-    const bool instrumented = getenv("CFB_ATTN_TRACE") != nullptr || getenv("CFB_ATTN_DEBUG") != nullptr;
     // packed batches: the tiles of one launch differ widely in length, which the hardware's dynamic CTA scheduling
     // absorbs and a static item walk does not -- per-item form unless forced
     const bool want = pv != nullptr ? atoi(pv) != 0 : (a.tiles == nullptr && a.T <= 512);
-    if (want && !instrumented) return launch_attn_tcp(a, st, err);
+    if (want) return launch_attn_tcp(a, st, err);
   }
   const int Dp = a.H * a.dkp;
   const long long rows = a.tiles != nullptr ? a.rows : static_cast<long long>(a.B) * a.T;
@@ -667,9 +603,7 @@ int launch_attn_tc(const AttnDesc& a, cudaStream_t st, std::string* err) {
   int dev = 0;
   cudaGetDevice(&dev);
   if (!configured[dev & 63]) {
-    cudaError_t e = cudaFuncSetAttribute(rel_attn_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(rel_attn_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal);
+    const cudaError_t e = cudaFuncSetAttribute(rel_attn_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal);
     if (e != cudaSuccess) {
       if (err) *err = std::string("cudaFuncSetAttribute(attn_tc): ") + cudaGetErrorString(e);
       return static_cast<int>(e);
@@ -684,25 +618,9 @@ int launch_attn_tc(const AttnDesc& a, cudaStream_t st, std::string* err) {
   p.Dp = Dp;
   p.tiles = a.tiles;
   p.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(a.dk));
-  p.trace = nullptr;
-  {
-    const char* dbg = getenv("CFB_ATTN_DEBUG");
-    p.debug = dbg ? atoi(dbg) : 0;
-  }
-  if (getenv("CFB_ATTN_TRACE")) {
-    if (!g_attn_trace) {
-      cudaMalloc(&g_attn_trace, 1024 * sizeof(long long));
-      cudaMemset(g_attn_trace, 0, 1024 * sizeof(long long));
-    }
-    p.trace = g_attn_trace;
-  }
   dim3 grid((a.T + kBM - 1) / kBM, a.H, a.B);
   if (a.tiles != nullptr) grid = dim3(a.n_tiles, a.H, 1);
-  cudaError_t e;
-  if (p.trace != nullptr || p.debug != 0)
-    e = launch_pdl(rel_attn_tc_kernel<true>, grid, dim3(kThreads), kSmemTotal, st, tmKV, tmP, p);
-  else
-    e = launch_pdl(rel_attn_tc_kernel<false>, grid, dim3(kThreads), kSmemTotal, st, tmKV, tmP, p);
+  const cudaError_t e = launch_pdl(rel_attn_tc_kernel, grid, dim3(kThreads), kSmemTotal, st, tmKV, tmP, p);
   if (e != cudaSuccess) {
     if (err) *err = std::string("attn_tc launch: ") + cudaGetErrorString(e);
     return static_cast<int>(e);

@@ -104,8 +104,8 @@ int launch_layernorm_scatter(const float* x, const float* gamma, const float* be
 // TMEM allocation, descriptor prefetch) while the previous kernel of the stream drains, and they call pdl_wait()
 // before their first global-memory access -- it returns once the previous kernel has completed and flushed.
 // pdl_launch_dependents() at the top of a kernel lets the NEXT kernel start the same way.  The forward is a chain
-// of ~260 short dependent launches, so this can hide launch latency + prologue per link.  Opt-in (CFB_PDL=1): see
-// pdl_enabled() for the measurement.
+// of ~260 short dependent launches, so this can hide launch latency + prologue per link.  The engine turns it on per
+// forward for small batches: see pdl_enabled() for the measurement.
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
@@ -133,8 +133,6 @@ int launch_gemm_tc(const GemmDesc& g, cudaStream_t st, std::string* err);
 // CTA-pair (cta_group::2) variant for N % 256 == 0 (gemm_tc2.cu); launch_gemm_tc picks it by shape / CFB_GEMM_2CTA
 bool gemm_tc2_supported(const GemmDesc& g);
 int launch_gemm_tc2(const GemmDesc& g, cudaStream_t st, std::string* err);
-long long* g_gemm_trace_view();
-long long* gemm_trace_buffer(cudaStream_t st);
 int launch_conv_tc(const ConvDesc& c, cudaStream_t st, std::string* err);
 int launch_gemm_simt(const GemmDesc& g, float* scratch, cudaStream_t st, std::string* err);
 int launch_attn_tc(const AttnDesc& a, cudaStream_t st, std::string* err);

@@ -19,7 +19,6 @@
 // Arithmetic order is the stand-alone kernels' (taps ascending, k-blocks ascending): results are bit-identical to
 // depthwise_kernel + gemm_tc_kernel<EPI_RESID>.
 #include <stdio.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "ptx.cuh"
@@ -62,16 +61,7 @@ struct DwPwParams {
   int T, d, num_kb, nc, bnc, tblocks;
   uint32_t tmem_cols;
   const float* bias2;
-  long long* trace;  // CFB_TAIL_TRACE=1 (instrumented instance only): clock marks of CTA 0
 };
-// trace slots: [0] start, [1] end of main loop (warp 2), [2] acc_full seen, [3] epilogue done;
-// 16 + 4 kb + {0..3}: TMA warp (g_empty seen, g issued, w issued);  64 + 4 kb + {0..3}: MMA warp (a_full seen, w seen,
-// committed);  128 + 64 group + 8 i + {0..3}: producer warp strip 0 of the group (g_full seen, FMAs done, a_empty seen,
-// a_full arrived)
-#define CFB_MARK(slot)                                   \
-  do {                                                   \
-    if (TRACE && p.trace != nullptr && blockIdx.x == 0) p.trace[slot] = clock64(); \
-  } while (0)
 
 __device__ __forceinline__ float2 lds64f(uint32_t addr) {
   float2 v;
@@ -104,7 +94,6 @@ __device__ __forceinline__ float swish_fast(float v) {  // swish(v) = h + h tanh
   return fmaf(h, t, h);
 }
 
-template <bool TRACE>
 __global__ void __launch_bounds__(kThreads, 1)
 dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CUtensorMap tmT,
              const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmO, const DwPwParams p) {
@@ -157,7 +146,6 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
   const uint32_t tmem_base = *tmem_slot;
   pdl_launch_dependents();
   pdl_wait();
-  if (threadIdx.x == 0) CFB_MARK(0);
 
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer: halo tiles of g + tap blocks
@@ -166,7 +154,6 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
       uint32_t gphase = 0;
       for (int kb = 0; kb < p.num_kb; ++kb) {
         ptx::mbar_wait_a(g_empty + 8 * gs, gphase ^ 1);
-        CFB_MARK(16 + 4 * kb + 0);
         ptx::mbar_arrive_expect_tx_a(g_full + 8 * gs, kGBytes + kTapBytes);
         ptx::tma_load_3d(smem + kOffG + gs * kGStage, &tmG, reinterpret_cast<uint64_t*>(smem + kOffBar + 8 * gs),
                          kb * kKC, t0 - kHalo, b);
@@ -176,7 +163,6 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
           gs = 0;
           gphase ^= 1;
         }
-        CFB_MARK(16 + 4 * kb + 1);
       }
     }
   } else if (warp == 2) {
@@ -196,7 +182,6 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
             wphase ^= 1;
           }
         }
-        CFB_MARK(16 + 4 * kb + 2);
       }
     }
   } else if (warp == 1) {
@@ -209,12 +194,10 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
         const int s = kb & 1;
         ptx::mbar_wait_a(a_full + 8 * s, (kb >> 1) & 1);
         ptx::tc_fence_after();
-        CFB_MARK(64 + 4 * kb + 0);
         const uint64_t da = ptx::make_sdesc_sw128(sbase + kOffA + s * kAStage, 16, 1024);
         for (int nh = 0; nh < p.nc; ++nh) {
           ptx::mbar_wait_a(w_full + 8 * wslot, wphase);
           ptx::tc_fence_after();
-          CFB_MARK(64 + 4 * kb + 1);
           const uint64_t db = ptx::make_sdesc_sw128(sbase + kOffW + wslot * kWStage, 16, 1024);
           const uint32_t d_tmem = tmem_base + nh * p.bnc;
 #pragma unroll
@@ -226,7 +209,6 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
           }
         }
         ptx::tc_commit_a(a_empty + 8 * s);
-        CFB_MARK(64 + 4 * kb + 2);
       }
       ptx::tc_commit_a(acc_full);
     }
@@ -242,10 +224,7 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
       const int s = kb & 1;  // A slot (= group)
       const uint32_t ph = (kb >> 1) & 1;
       const int gs = kb % kGStages;
-      const bool tr = TRACE && strip == 0 && lane == 0;
-      const int tb = 128 + 64 * group + 8 * (kb >> 1);
       ptx::mbar_wait_a(g_full + 8 * gs, (kb / kGStages) & 1);
-      if (tr) CFB_MARK(tb + 0);
       const uint32_t tp = sbase + kOffT + gs * kTapBytes + lane * 8;
       float2 w[kTaps];
 #pragma unroll
@@ -266,10 +245,8 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
         }
       }
       __syncwarp();
-      if (tr) CFB_MARK(tb + 1);
       if (lane == 0) ptx::mbar_arrive_a(g_empty + 8 * gs);  // halo tile and taps of this stage are in registers
       ptx::mbar_wait_a(a_empty + 8 * s, ph ^ 1);           // the MMAs that read this A slot two k-blocks ago are done
-      if (tr) CFB_MARK(tb + 2);
       const uint32_t ap = sbase + kOffA + s * kAStage + (strip * kStrip) * 128 + a_lane;
 #pragma unroll
       for (int o = 0; o < kStrip; ++o) {
@@ -279,9 +256,7 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
       ptx::fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive_a(a_full + 8 * s);
-      if (tr) CFB_MARK(tb + 3);
     }
-    if (pw == 0 && lane == 0) CFB_MARK(1);
 
     // ------------------------------------------------------------------ epilogue: x += acc + b2
     const int quarter = warp & 3;           // TMEM lanes this warp may read
@@ -289,7 +264,6 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
     const int row0 = t0 + quarter * 32;
     ptx::mbar_wait_a(acc_full, 0);
     ptx::tc_fence_after();
-    if (pw == 0 && lane == 0) CFB_MARK(2);
     if (row0 < p.T) {
       uint8_t* stage_base = smem + pw * 8192;
       const uint32_t swz = static_cast<uint32_t>(lane & 7);
@@ -325,7 +299,6 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
       // the staging boxes must outlive their reads; the global side of the reductions completes with the grid
       if (lane == 0) ptx::bulk_wait_read<0>();
     }
-    if (pw == 0 && lane == 0) CFB_MARK(3);
   }
 
   ptx::tc_fence_before();
@@ -337,8 +310,6 @@ dw_pw_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CU
 }
 
 }  // namespace
-
-long long* g_tail_trace = nullptr;
 
 bool dw_pw_supported(int d) { return d >= 64 && d % 64 == 0 && d <= 512; }
 
@@ -388,24 +359,15 @@ int launch_dw_pw(const DwPwDesc& c, cudaStream_t st, std::string* err) {
   int dev = 0;
   cudaGetDevice(&dev);
   if (!configured[dev & 63]) {
-    cudaError_t e = cudaFuncSetAttribute(dw_pw_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(dw_pw_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal);
+    const cudaError_t e = cudaFuncSetAttribute(dw_pw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal);
     if (e != cudaSuccess) {
       if (err) *err = std::string("cudaFuncSetAttribute(dw_pw): ") + cudaGetErrorString(e);
       return static_cast<int>(e);
     }
     configured[dev & 63] = true;
   }
-  cudaError_t e;
-  if (getenv("CFB_TAIL_TRACE")) {
-    if (!g_tail_trace) cudaMalloc(&g_tail_trace, 512 * sizeof(long long));
-    cudaMemsetAsync(g_tail_trace, 0, 512 * sizeof(long long), st);
-    p.trace = g_tail_trace;
-    e = launch_pdl(dw_pw_kernel<true>, dim3(c.B * p.tblocks), dim3(kThreads), kSmemTotal, st, tmG, tmT, tmW, tmO, p);
-  } else {
-    e = launch_pdl(dw_pw_kernel<false>, dim3(c.B * p.tblocks), dim3(kThreads), kSmemTotal, st, tmG, tmT, tmW, tmO, p);
-  }
+  const cudaError_t e =
+      launch_pdl(dw_pw_kernel, dim3(c.B * p.tblocks), dim3(kThreads), kSmemTotal, st, tmG, tmT, tmW, tmO, p);
   if (e != cudaSuccess) {
     if (err) *err = std::string("dw_pw launch: ") + cudaGetErrorString(e);
     return static_cast<int>(e);
@@ -413,13 +375,4 @@ int launch_dw_pw(const DwPwDesc& c, cudaStream_t st, std::string* err) {
   return 0;
 }
 
-long long* g_tail_trace_view() { return g_tail_trace; }
-
 }  // namespace cfb
-
-// debug: clock marks of the last traced launch (512 values; CFB_TAIL_TRACE=1)
-extern "C" __attribute__((visibility("default"))) int cfb_debug_tail_trace(long long* host_out) {
-  if (!cfb::g_tail_trace_view()) return 1;
-  cudaDeviceSynchronize();
-  return cudaMemcpy(host_out, cfb::g_tail_trace_view(), 512 * sizeof(long long), cudaMemcpyDeviceToHost) == cudaSuccess ? 0 : 2;
-}

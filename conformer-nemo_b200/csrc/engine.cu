@@ -198,11 +198,7 @@ PackedTables carve_tables(uint8_t* base, int B, int n_rows) {
 }
 
 // cfb_forward may run a batch as two half-batches on two streams, each half with its own plan
-bool micro_batching_enabled() {
-  static const bool on = !(getenv("CFB_MICROBATCH") != nullptr && atoi(getenv("CFB_MICROBATCH")) == 0);
-  return on;
-}
-int micro_split(const cfb_handle* h, int B) { return (!h->validate && micro_batching_enabled() && B >= 8) ? (B + 1) / 2 : 0; }
+int micro_split(const cfb_handle* h, int B) { return (!h->validate && B >= 8) ? (B + 1) / 2 : 0; }
 size_t workspace_need(const cfb_handle* h, int B, int T) {
   size_t need = make_plan(h, B, T).total;
   const int b0 = micro_split(h, B);
@@ -1081,7 +1077,7 @@ int cfb_forward(cfb_handle* h, const void* feats, int feats_dtype, const int64_t
 // A small packed batch runs as interleaved groups (utterances g, g + G, ...: balanced when the caller sorts by length,
 // as sharding.plan_shards does) on their own streams, like cfb_forward's half-batches: the groups' kernels
 // interleave on the GPU, which matters most for SMALL shares (a rank of an 8-GPU job), where every kernel is a fraction
-// of a wave and latency-bound.  CFB_MICROBATCH=0 keeps one group.
+// of a wave and latency-bound.
 // Measured (r5b / r5e, cfg3 shares, ms per step): 25 480 rows 13.31 with two groups / 13.25 with one, 6 500 rows 4.41 /
 // 4.17, 3 100 rows (an 8-GPU share) 2.80 with one or two groups, 2.73 with three -- it only pays once a launch no
 // longer fills the machine.
@@ -1091,7 +1087,7 @@ static int packed_groups(const cfb_handle* h, int B, int n_rows) {
   const char* force = getenv("CFB_PACKED_GROUPS");  // 1 .. 4 forces (read per call: tests switch it)
   int g = 1;
   if (force != nullptr) g = atoi(force);
-  else if (micro_batching_enabled() && n_rows <= kSmallBatchRows) g = 3;  // r5e: 1 / 2 / 3 / 4 groups 2.80 / 2.81 / 2.73 / 2.75 ms
+  else if (n_rows <= kSmallBatchRows) g = 3;  // r5e: 1 / 2 / 3 / 4 groups 2.80 / 2.81 / 2.73 / 2.75 ms
   if (h->profiling) g = 1;
   g = std::min(std::min(g, B), cfb_handle::kMaxGroups);
   return std::max(g, 1);

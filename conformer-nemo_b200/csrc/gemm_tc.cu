@@ -38,8 +38,6 @@ struct TcParams {
   int conv_tblocks;   // output tiles per sequence along time (32 frames each)
   int conv_fblocks;   // output tiles along frequency (4 bins each)
   int conv_To, conv_Fo;
-  int dbg_nofence;  // CFB_GEMM_NOFENCE=1: timing experiment only (results may be stale)
-  long long* trace;  // CFB_GEMM_TRACE=1: per-tile clock marks of CTA 0 (epilogue warp 2, MMA issuer)
   EpiParams ep;
 };
 
@@ -148,11 +146,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       int it = 0;
       for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
         const int buf = it & 1;
-        const bool trm = p.trace != nullptr && blockIdx.x == 0 && it < 16;
-        if (trm) p.trace[64 + it * 4 + 0] = clock64();
         ptx::mbar_wait(&acc_empty[buf], ((it >> 1) & 1) ^ 1);
         ptx::tc_fence_after();
-        if (trm) p.trace[64 + it * 4 + 1] = clock64();
         const uint32_t d_tmem = tmem_base + buf * BN;
         for (int kb = 0; kb < p.num_k_blocks; ++kb) {
           ptx::mbar_wait(&full_bar[stage], phase);
@@ -172,7 +167,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           }
         }
         ptx::tc_commit(&acc_full[buf]);
-        if (trm) p.trace[64 + it * 4 + 2] = clock64();
       }
     }
   } else {
@@ -214,8 +208,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         out_row = static_cast<long long>(m_blk) * kBlockM + row_in_tile;
         row_ok = out_row < p.ep.M;
       }
-      const bool trc = p.trace != nullptr && blockIdx.x == 0 && warp == 2 && lane == 0 && it < 16;
-      if (trc) p.trace[it * 4 + 0] = clock64();
       const bool keep = row_ok ? epi_keep<EPI>(p.ep, out_row) : true;  // its load is in flight during the accumulator wait
       // stage this tile's bias (BN floats) in shared memory while the accumulator is still being computed
       const uint32_t bias_a = bias_a0 + buf * BN * 4;
@@ -229,7 +221,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       }
       ptx::mbar_wait(&acc_full[buf], (it >> 1) & 1);
       ptx::tc_fence_after();
-      if (trc) p.trace[it * 4 + 1] = clock64();
       const uint32_t t_addr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + buf * BN;
 #pragma unroll 1
       for (int box = half; box < kBoxes; box += kEpiWarps / 4) {
@@ -239,15 +230,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll 1
         for (int pass = 0; pass < n_pass; ++pass) {
           uint8_t* sbuf = stage_base + (L::kSBuf == 2 ? (box_counter & 1u) * 4096 : 0u);
-          const bool trb = trc && it == 2;
-          const int tb0 = 32 + (box >> 1) * 8;
-          if (trb) p.trace[tb0 + 0] = clock64();
           if (lane == 0) {  // the store that last read this buffer has drained it
             if constexpr (L::kSBuf == 2) ptx::bulk_wait_read<1>();
             else ptx::bulk_wait_read<0>();
           }
           __syncwarp();
-          if (trb) p.trace[tb0 + 1] = clock64();
           const uint32_t srow = stage_a + static_cast<uint32_t>(sbuf - stage_base) + lane * 128;
 #pragma unroll
           for (int ch = 0; ch < kChunks; ++ch) {
@@ -289,10 +276,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               }
             }
           }
-          if (trb) p.trace[tb0 + 2] = clock64();
-          if (!p.dbg_nofence) ptx::fence_proxy_async_smem();
+          ptx::fence_proxy_async_smem();
           __syncwarp();
-          if (trb) p.trace[tb0 + 3] = clock64();
           if (lane == 0) {
             if constexpr (CONV) {
               ptx::tma_store_4d(&tmO, sbuf, acc_col0, cv_f0, cv_t0, cv_b);
@@ -311,13 +296,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             }
             ptx::bulk_commit();
           }
-          if (trb) p.trace[tb0 + 4] = clock64();
           ++box_counter;
         }
       }
       ptx::tc_fence_before();
       ptx::mbar_arrive(&acc_empty[buf]);
-      if (trc) p.trace[it * 4 + 2] = clock64();
     }
     if (lane == 0) ptx::bulk_wait_read<0>();  // staging boxes outlive their reads; the global side completes with the grid
   }
@@ -330,7 +313,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   }
 }
 
-long long* g_gemm_trace = nullptr;
 int g_num_sms = 0;
 int num_sms() {
   if (g_num_sms == 0) {
@@ -358,11 +340,7 @@ int launch_instance(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtens
     }
     configured[dev & 63] = true;
   }
-  int grid = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
-  if (const char* cap = getenv("CFB_GEMM_MAX_CTAS")) {  // timing experiments: fewer CTAs share the L2 (per-tile clocks via CFB_GEMM_TRACE)
-    const int c = atoi(cap);
-    if (c > 0 && c < grid) grid = c;
-  }
+  const int grid = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
   cudaError_t e = launch_pdl(kern, dim3(grid), dim3(kThreads), L::kTotal, st, tmA, tmB, tmO, p);
   if (e != cudaSuccess) {
     if (err) *err = std::string("gemm_tc launch: ") + cudaGetErrorString(e);
@@ -400,15 +378,6 @@ int dispatch_epi(int epi, bool out_bf16, const CUtensorMap& tmA, const CUtensorM
 
 }  // namespace
 
-long long* g_gemm_trace_view() { return g_gemm_trace; }
-// CFB_GEMM_TRACE=1: the 128-value clock trace buffer (cleared on the launch's stream), else null
-long long* gemm_trace_buffer(cudaStream_t st) {
-  if (!getenv("CFB_GEMM_TRACE")) return nullptr;
-  if (!g_gemm_trace) cudaMalloc(&g_gemm_trace, 128 * sizeof(long long));
-  cudaMemsetAsync(g_gemm_trace, 0, 128 * sizeof(long long), st);
-  return g_gemm_trace;
-}
-
 int launch_gemm_tc(const GemmDesc& g, cudaStream_t st, std::string* err) {
   if (g.M <= 0 || g.N <= 0 || g.K <= 0) return 0;
   if ((g.lda % 8) || (g.ldw % 8) || (g.K % 8)) {
@@ -419,9 +388,8 @@ int launch_gemm_tc(const GemmDesc& g, cudaStream_t st, std::string* err) {
   // Small M (a rank's share of a sharded batch, one of its groups): when 128-wide tiles still fit in one wave, every CTA
   // owns ONE tile and its time is fill + K loop + epilogue in series -- 128-wide tiles double the CTAs and halve both the
   // operand bytes per k-block and the epilogue per CTA (the tiles are latency-bound there, not operand-bound).  This
-  // also takes precedence over the CTA-pair kernel, whose 256 x 256 tiles are the coarsest.  CFB_GEMM_SMALL_BN=0 disables.
-  static const bool small_bn_on = !(getenv("CFB_GEMM_SMALL_BN") != nullptr && atoi(getenv("CFB_GEMM_SMALL_BN")) == 0);
-  const bool small_m = small_bn_on && g.N % 256 == 0 && 2 * m_tiles * (g.N / 256) <= num_sms();
+  // also takes precedence over the CTA-pair kernel, whose 256 x 256 tiles are the coarsest.
+  const bool small_m = g.N % 256 == 0 && 2 * m_tiles * (g.N / 256) <= num_sms();
   if (!small_m) {
     // CTA pairs (gemm_tc2.cu): CFB_GEMM_2CTA=0 never, =1 whenever the shape allows, unset = the measured default
     const char* v2 = getenv("CFB_GEMM_2CTA");
@@ -453,8 +421,6 @@ int launch_gemm_tc(const GemmDesc& g, cudaStream_t st, std::string* err) {
   p.num_n_tiles = n_tiles;
   p.num_tiles = m_tiles * n_tiles;
   p.num_k_blocks = (g.K + kBlockK - 1) / kBlockK;
-  p.dbg_nofence = getenv("CFB_GEMM_NOFENCE") != nullptr;
-  p.trace = gemm_trace_buffer(st);
   p.ep = g.ep;
   p.ep.M = g.M;
   p.ep.N = g.N;
@@ -534,10 +500,3 @@ int launch_conv_tc(const ConvDesc& c, cudaStream_t st, std::string* err) {
 }
 
 }  // namespace cfb
-
-// debug: clock marks of the last traced GEMM launch (128 values)
-extern "C" __attribute__((visibility("default"))) int cfb_debug_gemm_trace(long long* host_out) {
-  if (!cfb::g_gemm_trace_view()) return 1;
-  cudaDeviceSynchronize();
-  return cudaMemcpy(host_out, cfb::g_gemm_trace_view(), 128 * sizeof(long long), cudaMemcpyDeviceToHost) == cudaSuccess ? 0 : 2;
-}

@@ -40,7 +40,6 @@ struct Tc2Params {
   int num_tiles;      // 256 x 256 tiles
   int num_n_tiles;
   int num_k_blocks;
-  long long* trace;  // CFB_GEMM_TRACE=1: per-tile clock marks of pair 0's MMA issuer and epilogue warp 2 (layout of gemm_tc.cu)
   EpiParams ep;
 };
 
@@ -123,11 +122,8 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       int it = 0;
       for (int tile = pair; tile < p.num_tiles; tile += num_pairs, ++it) {
         const int buf = it & 1;
-        const bool trm = p.trace != nullptr && blockIdx.x == 0 && it < 16;
-        if (trm) p.trace[64 + it * 4 + 0] = clock64();
         ptx::mbar_wait_a(acc_empty + 8 * buf, ((it >> 1) & 1) ^ 1);
         ptx::tc_fence_after();
-        if (trm) p.trace[64 + it * 4 + 1] = clock64();
         const uint32_t d_tmem = tmem_base + buf * kBN;
         for (int kb = 0; kb < p.num_k_blocks; ++kb) {
           ptx::mbar_wait_a(full_bar + 8 * stage, phase);
@@ -145,7 +141,6 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           }
         }
         ptx::tc_commit_2cta(acc_full + 8 * buf);
-        if (trm) p.trace[64 + it * 4 + 2] = clock64();
       }
     }
   } else {
@@ -181,11 +176,8 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         asm volatile("bar.sync 1, %0;" ::"n"(32 * kEpiWarps) : "memory");
       }
       const bool keep = row_ok ? epi_keep<EPI>(p.ep, out_row) : true;  // its load is in flight during the accumulator wait
-      const bool trc = p.trace != nullptr && blockIdx.x == 0 && warp == 2 && lane == 0 && it < 16;
-      if (trc) p.trace[it * 4 + 0] = clock64();
       ptx::mbar_wait_a(acc_full + 8 * buf, (it >> 1) & 1);
       ptx::tc_fence_after();
-      if (trc) p.trace[it * 4 + 1] = clock64();
       const uint32_t t_addr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + buf * kBN;
 #pragma unroll 1
       for (int box = half; box < kBoxes; box += kEpiWarps / 4) {
@@ -260,7 +252,6 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive_leader(acc_empty + 8 * buf);  // one arrival per warp, on the leader's barrier
-      if (trc) p.trace[it * 4 + 2] = clock64();
     }
     if (lane == 0) ptx::bulk_wait_read<0>();  // the staging boxes must outlive their reads
   }
@@ -352,7 +343,6 @@ int launch_gemm_tc2(const GemmDesc& g, cudaStream_t st, std::string* err) {
   p.num_n_tiles = g.N / kBN;
   p.num_tiles = ((g.M + 2 * kBlockM - 1) / (2 * kBlockM)) * p.num_n_tiles;
   p.num_k_blocks = (g.K + kBlockK - 1) / kBlockK;
-  p.trace = gemm_trace_buffer(st);
   p.ep = g.ep;
   p.ep.M = g.M;
   p.ep.N = g.N;

@@ -1,6 +1,5 @@
 // cuTensorMapEncodeTiled without linking libcuda: the entry point is resolved through the CUDA runtime, so the
 // shared library loads (and exports its symbols) on a machine that has no driver installed.
-#include <stdlib.h>
 #include <string.h>
 
 #include <mutex>
@@ -112,11 +111,8 @@ thread_local int g_pdl_auto = 0;  // set by the engine per forward (small batche
 // Programmatic dependent launch.  Measured on cfg2 (r01q): 8.65 ms/step with PDL vs 8.53 without under CUDA-graph replay,
 // 8.84 vs 8.99 eager -- at full size launch gaps are not what separates the kernel sum from the step time.  For SMALL
 // batches they are: an 8-GPU share of cfg3 (~3000 token rows, every kernel a fraction of a wave) runs 2.93 -> 2.86 ms
-// (r5b).  So the engine turns it on per forward below a row count; CFB_PDL=0 / 1 forces it off / on.
-bool pdl_enabled() {
-  static const int forced = getenv("CFB_PDL") != nullptr ? (atoi(getenv("CFB_PDL")) != 0 ? 1 : 0) : -1;
-  return forced >= 0 ? forced == 1 : g_pdl_auto != 0;
-}
+// (r5b).  So the engine turns it on per forward below a row count.
+bool pdl_enabled() { return g_pdl_auto != 0; }
 void set_pdl_auto(bool on) { g_pdl_auto = on ? 1 : 0; }
 
 }  // namespace cfb

@@ -41,20 +41,3 @@ if B * H * T * T <= 64 * 1024 * 1024:
     want = (torch.softmax((ac + bd) / math.sqrt(dk), -1) @ v).permute(0, 2, 1, 3).reshape(B * T, Dp)
     diff = (ctx.float() - want).abs()
     print(f"max_abs {float(diff.max()):.4e} rel_l2 {float(diff.norm() / want.norm()):.4e}")
-
-if os.environ.get("CFB_ATTN_TRACE"):
-    import ctypes, numpy as np
-    buf = (ctypes.c_longlong * 1024)()
-    rc = lib.cfb_debug_attn_trace(buf)
-    a = np.array(buf[:], dtype=np.int64)
-    base = a[0]
-    rel = lambda x: int(x - base) if x > 0 else -1
-    print("cta: start, tmem_alloc+sync, q_stored, first_window, loop_end, merged+written, dealloc:", [rel(x) for x in a[:7]])
-    print("softmax set0 warp0: it | wait_S, S_ready, (S_loaded), sv_done, exp_done, p_arrived, (g_full ok, window_loaded), window_stored, o_full, folded")
-    for it in range(5):
-        r = [rel(x) for x in a[16 + it * 16: 32 + it * 16]]
-        print(it, [r[0], r[1], r[10], r[2], r[3], r[4], r[8], r[9], r[5], r[6], r[7]])
-    print("issuer set0: it | start, kv_full, s_free, S_issued, p_ready, PV_issued")
-    for it in range(5):
-        print(it, [rel(x) for x in a[512 + it * 8: 518 + it * 8]])
-    print("G issuer: block issue times", [rel(x) for x in a[800:812]])

@@ -37,20 +37,3 @@ def timeit(fn, name):
 timeit(fused, "fused dw+pw2")
 if "--once" not in sys.argv:
     timeit(split, "depthwise, then pw2 GEMM")
-
-if os.environ.get("CFB_TAIL_TRACE"):
-    import ctypes
-    fused(); torch.cuda.synchronize()
-    buf = (ctypes.c_longlong * 512)()
-    assert lib.cfb_debug_tail_trace(buf) == 0
-    t = list(buf); t0 = t[0]
-    rel = lambda v: (v - t0) if v else -1
-    nkb = d // 64
-    print(f"trace (cycles since CTA start): main loop end {rel(t[1])}  acc_full seen {rel(t[2])}  epilogue done {rel(t[3])}")
-    for kb in range(nkb):
-        tm = [rel(t[16 + 4 * kb + i]) for i in range(3)]
-        mm = [rel(t[64 + 4 * kb + i]) for i in range(3)]
-        grp, i = kb & 1, kb >> 1
-        pr = [rel(t[128 + 64 * grp + 8 * i + j]) for j in range(4)]
-        print(f"kb {kb}: TMA g_empty {tm[0]:6d} g_issued {tm[1]:6d} w_issued {tm[2]:6d} | producer g_full {pr[0]:6d} fma_done {pr[1]:6d} "
-              f"a_empty {pr[2]:6d} a_full {pr[3]:6d} | MMA a_full {mm[0]:6d} w_full {mm[1]:6d} commit {mm[2]:6d}")

@@ -42,21 +42,3 @@ for name, epi, N, K, od in CASES:
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / n
     print(f"{name:24s} N={N:5d} K={K:5d}: {ms * 1e3:7.1f} us  {2.0 * M * N * K / ms / 1e9:7.0f} TFLOP/s")
-    if os.environ.get("CFB_GEMM_TRACE"):
-        import ctypes
-        buf = (ctypes.c_longlong * 128)()
-        lib.cfb_debug_gemm_trace(buf)
-        t = list(buf)
-        if not any(v > 0 for v in t):
-            print("   (no trace: the CTA-pair kernel ran; CFB_GEMM_2CTA=0 forces the traced single-CTA kernel)")
-            continue
-        base = min(v for v in t if v > 0)
-        ep = [(t[i * 4] - base, t[i * 4 + 1] - base, t[i * 4 + 2] - base) for i in range(8) if t[i * 4] > 0]
-        mm = [(t[64 + i * 4] - base, t[64 + i * 4 + 1] - base, t[64 + i * 4 + 2] - base) for i in range(8) if t[64 + i * 4] > 0]
-        print("   epilogue warp (wait start, acc ready, tile done):", ep)
-        print("   mma issuer   (tile start, acc_empty ok, committed):", mm)
-        for bx in range(4):
-            v = t[32 + bx * 8: 32 + bx * 8 + 5]
-            if v[0] > 0:
-                print("   tile 2 box", bx, "(start | drained | ld+math+sts | fence | store issued):", [x - v[0] for x in v])
-

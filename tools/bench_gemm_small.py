@@ -1,6 +1,5 @@
 """Small-M GEMMs (one group of an 8-GPU share: ~1000 token rows) timed under CUDA-graph replay of a dependent chain, so the
-number is the kernel's latency in a chain and not the host's launch rate.  Run once per tile setting:
-    CFB_GEMM_TINY_BN=0 python tools/bench_gemm_small.py ; python tools/bench_gemm_small.py"""
+number is the kernel's latency in a chain and not the host's launch rate."""
 import ctypes, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
@@ -9,7 +8,6 @@ from gpu_util import ptr
 from conformer_nemo_b200 import _lib
 
 lib = _lib.load_library()
-print("CFB_GEMM_TINY_BN =", os.environ.get("CFB_GEMM_TINY_BN", "default (on)"))
 for M in (1059, 2118, 3176):
     for name, epi, N, K in (("linear2 (resid)", 3, 512, 2048), ("linear_out (resid)", 3, 512, 512), ("plain bf16", 0, 512, 512)):
         A = (torch.randn(M, K, device="cuda") * 0.5).bfloat16()

@@ -63,14 +63,12 @@ struct cfb_handle {
   size_t arena_bytes = 0;
   Slot sub_w1, sub_b1, sub_w1g, sub_w2, sub_b2, sub_w3, sub_b3, w_pos, div_term, w_oproj, b_oproj;
   std::vector<LayerW> layers;
+  int sms = 0;  // streaming multiprocessors of the device
   int launches = 0;
-  // two-stream micro-batching (see cfb_forward): the second half of a batch runs on an auxiliary stream
-  cudaStream_t aux_stream = nullptr;
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  // packed batches may run as up to kMaxGroups interleaved groups: group 0 on the caller's stream, g on group_stream[g]
+  // a batch may run as up to kMaxGroups parts (run_parts): part 0 on the caller's stream, part g on group_stream[g]
   static constexpr int kMaxGroups = 4;
   cudaStream_t group_stream[kMaxGroups] = {};
-  cudaEvent_t group_join[kMaxGroups] = {};
+  cudaEvent_t ev_fork = nullptr, group_join[kMaxGroups] = {};
   mutable std::string err;
   // optional per-launch event timing
   bool profiling = false;
@@ -100,11 +98,16 @@ size_t align_up(size_t v, size_t a = 256) { return (v + a - 1) / a * a; }
 
 int conv_out(int n) { return (n - 1) / 2 + 1; }  // k=3, s=2, p=1 (n >= 1)
 
+// a named region of the workspace
+struct Region {
+  size_t off = 0, bytes = 0;
+};
+
 struct Plan {
   int B, T, T1, T2, Th, N, P;  // P = 2*T2-1
-  size_t y1, y2, x, a, hbuf, qkv, ctx, g, c, pe, pos, a0, raw, cols, total;
-  size_t tables;  // packed batches only: the PackedTables arrays
-  int n_tiles;
+  Region y1, y2, x, a, hbuf, qkv, ctx, g, c, pe, pos, a0, raw, cols;
+  Region tables;  // packed batches only: the PackedTables arrays
+  size_t total;
 };
 
 // Layout of a packed batch, computed from host-side lengths with the integer arithmetic packed_plan_kernel uses.
@@ -113,7 +116,6 @@ struct PackedShape {
   int n_tiles = 0;  // attention query tiles
   int t2_max = 0;   // dense output extent T' of the padded batch
   int first = 0, step = 1, count = 0;  // the group of utterances first, first + step, ... (count of them) this layout holds
-  bool prologue = true;  // this range also computes encoded_len and clears the dense result
 };
 PackedShape packed_shape(const int64_t* lengths_host, int B, int T, int first = 0, int step = 1) {
   PackedShape ps;
@@ -133,13 +135,13 @@ PackedShape packed_shape(const int64_t* lengths_host, int B, int T, int first = 
   return ps;
 }
 
-// packed_rows > 0: one virtual sequence of 4 * packed_rows input frames (common.cuh, PackedTables) whose positional
-// table covers t2_pos frames; otherwise the dense (B, T) batch.
-Plan make_plan(const cfb_handle* h, int B, int T, int packed_rows = 0, int t2_pos = 0, int packed_B = 0, int n_tiles = 0) {
+// Workspace layout of the dense (B, T) batch, or with pk of the packed group pk: one virtual sequence of 4 * pk->n_rows
+// input frames (common.cuh, PackedTables) whose positional table covers pk->t2_max frames.
+Plan make_plan(const cfb_handle* h, int B, int T, const PackedShape* pk = nullptr) {
   Plan p{};
-  if (packed_rows > 0) {
+  if (pk) {
     B = 1;
-    T = 4 * packed_rows;
+    T = 4 * pk->n_rows;
   }
   p.B = B;
   p.T = T;
@@ -147,14 +149,13 @@ Plan make_plan(const cfb_handle* h, int B, int T, int packed_rows = 0, int t2_po
   p.T2 = conv_out(p.T1);
   p.Th = (p.T1 + 1) / 2;
   p.N = B * p.T2;
-  p.P = 2 * (packed_rows > 0 ? t2_pos : p.T2) - 1;
-  p.n_tiles = n_tiles;
+  p.P = 2 * (pk ? pk->t2_max : p.T2) - 1;
   const size_t e = h->esz();
   size_t off = 0;
   auto take = [&](size_t bytes) {
-    size_t o = off;
+    const Region r{off, bytes};
     off = align_up(off + bytes);
-    return o;
+    return r;
   };
   const size_t N = static_cast<size_t>(p.N);
   p.y1 = take(static_cast<size_t>(B) * 4 * p.Th * h->Fh * h->C * e);
@@ -168,8 +169,9 @@ Plan make_plan(const cfb_handle* h, int B, int T, int packed_rows = 0, int t2_po
   p.c = take(N * h->d * e);
   p.pe = take(static_cast<size_t>(p.P) * h->d * e);
   p.pos = take(static_cast<size_t>(p.P) * h->L * h->Dp * e);
-  p.a0 = h->validate ? 0 : take(static_cast<size_t>(B) * 4 * p.Th * h->Fh * kConv0Cols * 2);  // first conv's GEMM operand
-  if (h->validate) {
+  if (!h->validate) {
+    p.a0 = take(static_cast<size_t>(B) * 4 * p.Th * h->Fh * kConv0Cols * 2);  // first conv's GEMM operand
+  } else {
     size_t raw = N * h->dff;
     raw = std::max(raw, N * 3 * h->Dp);
     raw = std::max(raw, static_cast<size_t>(p.P) * h->L * h->Dp);
@@ -179,8 +181,8 @@ Plan make_plan(const cfb_handle* h, int B, int T, int packed_rows = 0, int t2_po
     p.raw = take(raw * 4);
     p.cols = take(N * h->F2 * 9 * h->C * 4);
   }
-  if (packed_rows > 0)
-    p.tables = take((static_cast<size_t>(2) * packed_B + 2 * N + N / kPackAlign + 8) * 4 + static_cast<size_t>(n_tiles) * 16 + 64);
+  if (pk)
+    p.tables = take((static_cast<size_t>(2) * pk->count + 2 * N + N / kPackAlign + 8) * 4 + static_cast<size_t>(pk->n_tiles) * 16 + 64);
   p.total = off;
   return p;
 }
@@ -197,13 +199,38 @@ PackedTables carve_tables(uint8_t* base, int B, int n_rows) {
   return t;
 }
 
-// cfb_forward may run a batch as two half-batches on two streams, each half with its own plan
-int micro_split(const cfb_handle* h, int B) { return (!h->validate && B >= 8) ? (B + 1) / 2 : 0; }
-size_t workspace_need(const cfb_handle* h, int B, int T) {
-  size_t need = make_plan(h, B, T).total;
-  const int b0 = micro_split(h, B);
-  if (b0 > 0) need = std::max(need, make_plan(h, b0, T).total + make_plan(h, B - b0, T).total);
+// cfb_forward runs a bf16 batch of B >= 8 as two half-batches on two streams (micro-batching)
+int dense_parts(const cfb_handle* h, int B) { return (!h->validate && B >= 8) ? 2 : 1; }
+// utterances [first, first + count) of part i when a dense batch of B runs as n contiguous parts
+struct Range {
+  int first, count;
+};
+Range dense_part(int B, int n, int i) {
+  const int per = (B + n - 1) / n;
+  return {i * per, std::min(per, B - i * per)};
+}
+
+// A batch split into n parts lays the parts' plans end to end in the workspace.  The workspace a call needs is the
+// largest such sum over the splits n = 1 .. max_parts it may take; plan(n, i) is the plan of part i of n.
+template <typename PartPlan>
+size_t workspace_need(int max_parts, PartPlan plan) {
+  size_t need = 0;
+  for (int n = 1; n <= max_parts; ++n) {
+    size_t sum = 0;
+    for (int i = 0; i < n; ++i) sum += plan(n, i).total;
+    need = std::max(need, sum);
+  }
   return need;
+}
+size_t dense_workspace(const cfb_handle* h, int B, int T) {
+  return workspace_need(dense_parts(h, B), [&](int n, int i) { return make_plan(h, dense_part(B, n, i).count, T); });
+}
+// any group count up to min(B, kMaxGroups): CFB_PACKED_GROUPS can force each of them
+size_t packed_workspace(const cfb_handle* h, const int64_t* lengths_host, int B, int T) {
+  return workspace_need(std::min(B, cfb_handle::kMaxGroups), [&](int n, int i) {
+    const PackedShape ps = packed_shape(lengths_host, B, T, i, n);
+    return make_plan(h, B, T, &ps);
+  });
 }
 
 const HostTensor* find(const cfb_handle* h, const std::string& key) {
@@ -278,13 +305,14 @@ int cfb_create(const cfb_config* cfg, int device, cfb_handle** out) {
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev)
     return bad(CFB_ERR_CUDA, "no such CUDA device (this library has no CPU fallback)");
-  cudaDeviceProp prop;
+  cudaDeviceProp prop{};
   cudaGetDeviceProperties(&prop, device);
   if (prop.major != 10) return bad(CFB_ERR_UNSUPPORTED, "the kernels are built for sm_100a (Blackwell B200) only");
 
   cfb_handle* h = new cfb_handle();
   h->cfg = *cfg;
   h->device = device;
+  h->sms = prop.multiProcessorCount;
   h->validate = cfg->precision == CFB_PREC_FP32_VALIDATE;
   h->d = cfg->d_model;
   h->C = C;
@@ -306,20 +334,13 @@ int cfb_create(const cfb_config* cfg, int device, cfb_handle** out) {
     return bad(CFB_ERR_UNSUPPORTED, "d_ff and feat_out must be multiples of 8");
   }
   cudaSetDevice(device);
-  if (cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
-      cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming) != cudaSuccess) {
-    delete h;
-    return bad(CFB_ERR_CUDA, "could not create the auxiliary stream / events");
-  }
-  h->group_stream[1] = h->aux_stream;
-  h->group_join[1] = h->ev_join;
-  for (int g = 2; g < cfb_handle::kMaxGroups; ++g) {
-    if (cudaStreamCreateWithFlags(&h->group_stream[g], cudaStreamNonBlocking) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->group_join[g], cudaEventDisableTiming) != cudaSuccess) {
-      delete h;
-      return bad(CFB_ERR_CUDA, "could not create the group streams / events");
-    }
+  bool ok = cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming) == cudaSuccess;
+  for (int g = 1; ok && g < cfb_handle::kMaxGroups; ++g)
+    ok = cudaStreamCreateWithFlags(&h->group_stream[g], cudaStreamNonBlocking) == cudaSuccess &&
+         cudaEventCreateWithFlags(&h->group_join[g], cudaEventDisableTiming) == cudaSuccess;
+  if (!ok) {
+    cfb_destroy(h);
+    return bad(CFB_ERR_CUDA, "could not create the group streams / events");
   }
   *out = h;
   return CFB_OK;
@@ -329,13 +350,11 @@ void cfb_destroy(cfb_handle* h) {
   if (!h) return;
   cudaSetDevice(h->device);
   if (h->arena) cudaFree(h->arena);
-  if (h->aux_stream) cudaStreamDestroy(h->aux_stream);
-  for (int g = 2; g < cfb_handle::kMaxGroups; ++g) {
+  for (int g = 1; g < cfb_handle::kMaxGroups; ++g) {
     if (h->group_stream[g]) cudaStreamDestroy(h->group_stream[g]);
     if (h->group_join[g]) cudaEventDestroy(h->group_join[g]);
   }
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-  if (h->ev_join) cudaEventDestroy(h->ev_join);
   for (auto& e : h->ev_pool) cudaEventDestroy(e);
   delete h;
 }
@@ -602,7 +621,7 @@ int cfb_output_frames(const cfb_handle* h, int T, int* t_out) {
 
 int cfb_workspace_bytes(const cfb_handle* h, int B, int T, size_t* out) {
   if (!h || !out || B < 1 || T < 1) return fail(h, CFB_ERR_INVALID_ARG, "cfb_workspace_bytes: bad argument");
-  *out = workspace_need(h, B, T);
+  *out = dense_workspace(h, B, T);
   return CFB_OK;
 }
 
@@ -653,98 +672,139 @@ int cfb_profile_report(cfb_handle* h, char* buf, size_t cap) {
 
 int cfb_debug_buffer(const cfb_handle* h, int B, int T, const char* name, size_t* offset, size_t* bytes) {
   if (!h || !name || !offset || !bytes || B < 1 || T < 1) return fail(h, CFB_ERR_INVALID_ARG, "cfb_debug_buffer: bad argument");
+  if (dense_parts(h, B) > 1)
+    return fail(h, CFB_ERR_INVALID_ARG, "cfb_debug_buffer: a bf16 batch of B >= 8 runs as two half-batches, each with a "
+                                        "workspace plan of its own; ask for B <= 7, or use fp32_validate");
+  static const struct {
+    const char* name;
+    Region Plan::*region;
+  } named[] = {{"y1", &Plan::y1},   {"y2", &Plan::y2}, {"x", &Plan::x}, {"a", &Plan::a},   {"h", &Plan::hbuf},
+               {"qkv", &Plan::qkv}, {"ctx", &Plan::ctx}, {"g", &Plan::g}, {"c", &Plan::c}, {"pe", &Plan::pe},
+               {"pos", &Plan::pos}};
   const Plan p = make_plan(h, B, T);
-  const size_t e = h->esz();
-  const size_t N = static_cast<size_t>(p.N);
-  const std::string n(name);
-  struct { const char* name; size_t off, bytes; } tab[] = {
-      {"y1", p.y1, static_cast<size_t>(B) * 4 * p.Th * h->Fh * h->C * e},
-      {"y2", p.y2, N * h->F2 * h->C * e},
-      {"x", p.x, N * h->d * 4},
-      {"a", p.a, N * h->d * e},
-      {"h", p.hbuf, N * h->dff * e},
-      {"qkv", p.qkv, N * 4 * h->Dp * e},
-      {"ctx", p.ctx, N * h->Dp * e},
-      {"g", p.g, N * h->d * e},
-      {"c", p.c, N * h->d * e},
-      {"pe", p.pe, static_cast<size_t>(p.P) * h->d * e},
-      {"pos", p.pos, static_cast<size_t>(p.P) * h->L * h->Dp * e},
-  };
-  for (auto& t : tab)
-    if (n == t.name) {
-      *offset = t.off;
-      *bytes = t.bytes;
+  for (const auto& n : named)
+    if (strcmp(name, n.name) == 0) {
+      *offset = (p.*n.region).off;
+      *bytes = (p.*n.region).bytes;
       return CFB_OK;
     }
-  return fail(h, CFB_ERR_INVALID_ARG, "cfb_debug_buffer: unknown buffer " + n);
+  return fail(h, CFB_ERR_INVALID_ARG, std::string("cfb_debug_buffer: unknown buffer ") + name);
 }
 
 }  // extern "C"
 
-// One contiguous range of the batch on one stream (the whole batch, or one half of it).
-// pk != nullptr: the batch runs in the packed layout (every utterance in its own slot of token rows, no padding).
-static int forward_range(cfb_handle* h, const void* feats, int feats_dtype, const int64_t* lengths, int B, int T,
-                         void* encoded, int out_dtype, int32_t* encoded_len, void* workspace, cudaStream_t st,
-                         int* launches_out, int B_total, const PackedShape* pk = nullptr) {
-  const Plan pl = pk ? make_plan(h, B, T, pk->n_rows, pk->t2_max, pk->count, pk->n_tiles) : make_plan(h, B, T);
+namespace {
+
+// Enqueues the launch groups of one forward call.  Each group gets an NVTX range named like its label in the profile
+// report (nsys / ncu --nvtx group kernels by them) and, while profiling is on, a CUDA event on either side; its kernels
+// are added to the call's launch count, and its failure becomes the handle's error text.  After a failure nothing more
+// is enqueued: every later group returns the same status, which the call returns.
+struct Enqueue {
+  cfb_handle* h;
+  unsigned int ev_flags = cudaEventRecordDefault;
+  int rc = CFB_OK;
+  std::string err;  // a launcher's own description of its failure
+
+  Enqueue(cfb_handle* h_, cudaStream_t st) : h(h_) {
+    h->launches = 0;
+    if (!h->profiling) return;
+    // A profiled forward runs on the caller's stream alone.  Under stream capture the brackets become event-record NODES
+    // of the graph (cudaEventRecordExternal): every replay re-records them on the GPU's own timeline, so the intervals
+    // hold the kernel and the node-to-node launch latency the replayed step really pays, but none of the host's enqueue
+    // cost (eager brackets around a 5 us kernel measure mostly how fast the host enqueues: the GPU runs ahead of it).
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusActive) ev_flags = cudaEventRecordExternal;
+    // calibration of the brackets themselves: two event records with nothing between them (a bracket around a kernel
+    // holds the same fixed cost on top of the kernel's launch latency and run time)
+    (*this)(st, "(empty bracket)", 0, [] { return 0; });
+  }
+
+  // launch() enqueues n kernels on st and returns 0 or an error code
+  template <typename Launch>
+  int operator()(cudaStream_t st, const char* label, int n, Launch&& launch) {
+    if (rc != CFB_OK) return rc;
+    nvtxRangePushA(label);
+    const bool timed = h->profiling && h->ev_used + 2 <= h->ev_pool.size();
+    const size_t e0 = h->ev_used;
+    if (timed) cudaEventRecordWithFlags(h->ev_pool[e0], st, ev_flags);
+    const int r = launch();
+    nvtxRangePop();
+    if (timed) {
+      cudaEventRecordWithFlags(h->ev_pool[e0 + 1], st, ev_flags);
+      h->recs.push_back({label, e0, e0 + 1});
+      h->ev_used += 2;
+    }
+    if (r != 0)
+      return rc = fail(h, CFB_ERR_CUDA, std::string("cfb_forward: ") + label + " failed: " +
+                                           (err.empty() ? cudaGetErrorString(static_cast<cudaError_t>(r)) : err));
+    h->launches += n;
+    return CFB_OK;
+  }
+};
+
+// Runs a batch as n parts: part 0 on the caller's stream st, part g on group_stream[g], forked from st with one event
+// and joined back into it (capturable).  part(g, stream) enqueues part g and returns its status.  The parts' kernels
+// interleave on the GPU: one part's memory-bound kernels and kernel tails overlap another part's GEMMs.  The join
+// happens even after an error, so that a capture in progress is not left with a dangling branch.
+template <typename Part>
+int run_parts(cfb_handle* h, cudaStream_t st, int n, Part&& part) {
+  if (n == 1) return part(0, st);
+  int forked = 1;  // streams waiting on the fork, st included
+  if (cudaEventRecord(h->ev_fork, st) == cudaSuccess)
+    while (forked < n && cudaStreamWaitEvent(h->group_stream[forked], h->ev_fork, 0) == cudaSuccess) ++forked;
+  int rc = forked == n ? CFB_OK : fail(h, CFB_ERR_CUDA, "cfb_forward: stream fork failed");
+  for (int g = 0; g < n && rc == CFB_OK; ++g) rc = part(g, g == 0 ? st : h->group_stream[g]);
+  for (int g = 1; g < forked; ++g) {
+    cudaEventRecord(h->group_join[g], h->group_stream[g]);
+    cudaStreamWaitEvent(st, h->group_join[g], 0);
+  }
+  return rc;
+}
+
+// Whether a forward runs the conv-module tail as one kernel (conv_tail.cu) instead of two.  CFB_FUSED_TAIL=0 keeps the
+// two launches, =2 fuses whenever the shape allows, unset leaves it to the heuristic; it is read on every call (tests
+// switch it between forwards).  The fused kernel runs one CTA per 128 frames of a sequence: worth it when the `ctas` of
+// the whole batch (its parts run concurrently) fill most of the machine; a CTA takes ~29 us however few there are
+// (measured r02f: 128 CTAs 29 us vs 39 us for the two kernels, 59 CTAs 29 us vs 25 us).
+bool use_fused_tail(const cfb_handle* h, long long ctas) {
+  const char* var = getenv("CFB_FUSED_TAIL");
+  const int mode = var != nullptr ? atoi(var) : 1;
+  if (mode == 0 || h->validate || !dw_pw_supported(h->d)) return false;
+  if (mode == 2) return true;
+  const long long waves = (ctas + h->sms - 1) / h->sms;
+  return ctas * 100 >= waves * h->sms * 65;
+}
+
+// The checks cfb_forward and cfb_forward_packed (`fn` in the messages) share.
+int check_forward(cfb_handle* h, const char* fn, const void* feats, int feats_dtype, const void* encoded, int out_dtype,
+                  const int32_t* encoded_len, const void* workspace, int B, int T) {
+  if (!h) return CFB_ERR_INVALID_ARG;
+  auto bad = [&](int code, const char* msg) { return fail(h, code, std::string(fn) + msg); };
+  if (!h->finalized) return bad(CFB_ERR_STATE, ": weights are not finalized");
+  if (!feats || !encoded || !encoded_len || !workspace || B < 1 || T < 1) return bad(CFB_ERR_INVALID_ARG, ": null pointer or empty batch");
+  if (feats_dtype != CFB_F32 && feats_dtype != CFB_BF16) return bad(CFB_ERR_INVALID_ARG, ": feats must be f32 or bf16");
+  if (out_dtype != CFB_F32 && out_dtype != CFB_BF16) return bad(CFB_ERR_INVALID_ARG, ": encoded must be f32 or bf16");
+  return CFB_OK;
+}
+
+// One part of a batch on stream st, in the workspace ws laid out by pl: a contiguous range of B utterances (the whole
+// batch, or one half of it), or with pk a group of the B utterances in the packed layout (every utterance in its own slot
+// of token rows, no padding; cfb_forward_packed has computed encoded_len and cleared the result).
+int forward_range(cfb_handle* h, Enqueue& q, cudaStream_t st, const Plan& pl, const PackedShape* pk, bool fused_tail,
+                  const void* feats, int feats_dtype, const int64_t* lengths, int B, int T, void* encoded, int out_dtype,
+                  int32_t* encoded_len, uint8_t* ws) {
   const int Bk = pk ? 1 : B;  // batch extent the kernels see: a packed batch is one long sequence
-  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
   const bool v = h->validate;
   const bool abf = !v;  // activations / matrices in bf16
   const int d = h->d, C = h->C, F2 = h->F2, dff = h->dff, H = h->H, Dp = h->Dp, L = h->L;
   const int N = pl.N, T2 = pl.T2;
   PackedTables tb;
-  if (pk) tb = carve_tables(reinterpret_cast<uint8_t*>(workspace) + pl.tables, pk->count, pk->n_rows);
-  std::string err;
-  int launches = 0;
-  float* raw = v ? reinterpret_cast<float*>(ws + pl.raw) : nullptr;
+  if (pk) tb = carve_tables(ws + pl.tables.off, pk->count, pk->n_rows);
+  float* raw = v ? reinterpret_cast<float*>(ws + pl.raw.off) : nullptr;
 
-  // profiling: tick(label) before a launch group, tock() after it (CUDA events on the forward's stream)
-  size_t prof_e0 = 0;
-  const char* prof_label = nullptr;
-  // NVTX: one range per launch group, named like the profile report's labels (nsys / ncu --nvtx group kernels by them)
-  // Under stream capture the brackets become event-record NODES of the graph (cudaEventRecordExternal): every replay
-  // re-records them on the GPU's own timeline, so the intervals hold the kernel and the node-to-node launch latency the
-  // replayed step really pays, but none of the host's enqueue cost (eager brackets around a 5 us kernel measure mostly
-  // how fast the host enqueues: the GPU runs ahead of it).
-  unsigned int ev_flags = cudaEventRecordDefault;
-  if (h->profiling) {
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusActive) ev_flags = cudaEventRecordExternal;
-  }
-  auto tick = [&](const char* label) {
-    nvtxRangePushA(label);
-    if (!h->profiling) return;
-    if (h->ev_used + 2 > h->ev_pool.size()) {
-      prof_label = nullptr;
-      return;
-    }
-    prof_label = label;
-    prof_e0 = h->ev_used++;
-    cudaEventRecordWithFlags(h->ev_pool[prof_e0], st, ev_flags);
-  };
-  auto tock = [&]() {
-    nvtxRangePop();
-    if (!h->profiling || !prof_label) return;
-    const size_t e1 = h->ev_used++;
-    cudaEventRecordWithFlags(h->ev_pool[e1], st, ev_flags);
-    h->recs.push_back({prof_label, prof_e0, e1});
-    prof_label = nullptr;
-  };
-
-#define CFB_TRY(expr, what)                                                                        \
-  do {                                                                                             \
-    tick(what);                                                                                    \
-    int rc_ = (expr);                                                                              \
-    tock();                                                                                        \
-    if (rc_ != 0) {                                                                                \
-      return fail(h, CFB_ERR_CUDA, std::string("cfb_forward: ") + what + " failed: " +             \
-                                       (err.empty() ? cudaGetErrorString((cudaError_t)rc_) : err)); \
-    }                                                                                              \
-  } while (0)
-
-  auto gemm = [&](const void* A, long long lda, const Slot& W, long long ldw, int M, int Nn, int K, int epi,
-                  bool out_bf16, EpiParams ep, const char* what) -> int {
+  // one launch on the tensor cores, two on the fp32 validation path
+  auto gemm = [&](const void* A, long long lda, const Slot& W, long long ldw, int M, int Nn, int K, int epi, bool out_bf16,
+                  EpiParams ep, const char* label) {
     GemmDesc g;
     g.A = A;
     g.lda = lda;
@@ -756,94 +816,56 @@ static int forward_range(cfb_handle* h, const void* feats, int feats_dtype, cons
     g.epi = epi;
     g.out_bf16 = out_bf16;
     g.ep = ep;
-    int rc;
-    if (v) {
-      rc = launch_gemm_simt(g, raw, st, &err);
-      launches += 2;
-    } else {
-      rc = launch_gemm_tc(g, st, &err);
-      launches += 1;
-    }
-    if (rc != 0 && err.empty()) err = what;
-    return rc;
+    return q(st, label, v ? 2 : 1, [&] { return v ? launch_gemm_simt(g, raw, st, &q.err) : launch_gemm_tc(g, st, &q.err); });
   };
 
-  // conv-module tail as one kernel (conv_tail.cu) whenever the shape allows it; CFB_FUSED_TAIL=0 keeps the two launches
-  const char* tail_var = getenv("CFB_FUSED_TAIL");  // 0 = never, 2 = whenever the shape allows, unset = heuristic
-  const bool tail_env = !(tail_var != nullptr && atoi(tail_var) == 0);
-  // One CTA per 128 frames of a sequence: worth it when the CTAs of the whole batch (both micro-batch halves run
-  // concurrently) fill most of the machine; a CTA takes ~29 us however few there are (measured r02f: 128 CTAs 29 us
-  // vs 39 us for the two kernels, 59 CTAs 29 us vs 25 us).
-  bool fused_tail = tail_env && !v && dw_pw_supported(d);
-  if (fused_tail && !(tail_var != nullptr && atoi(tail_var) == 2)) {
-    int sms = 0;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    if (sms <= 0) sms = 148;
-    const long long ctas = static_cast<long long>(pk ? 1 : B_total) * ((T2 + 127) / 128);
-    const long long waves = (ctas + sms - 1) / sms;
-    fused_tail = ctas * 100 >= waves * sms * 65;
-  }
-
-  // calibration of the brackets themselves: two event records with nothing between them (reported under this label; a
-  // bracket around a kernel holds the same fixed cost on top of the kernel's launch latency and run time)
-  if (h->profiling) {
-    tick("(empty bracket)");
-    tock();
-  }
   // ---- lengths (subsampling.py:164-171)
-  if (!pk || pk->prologue) {
-    CFB_TRY(launch_lengths(reinterpret_cast<const long long*>(lengths), encoded_len, B, T, 2, st), "lengths");
-    ++launches;
-  }
   if (pk) {
-    CFB_TRY(launch_packed_plan(reinterpret_cast<const long long*>(lengths), pk->count, pk->first, pk->step, T, pk->t2_max,
-                               pk->n_rows, pk->n_tiles, tb, st),
-            "packed layout tables");
-    ++launches;
+    q(st, "packed layout tables", 1, [&] {
+      return launch_packed_plan(reinterpret_cast<const long long*>(lengths), pk->count, pk->first, pk->step, T, pk->t2_max,
+                                pk->n_rows, pk->n_tiles, tb, st);
+    });
+  } else {
+    q(st, "lengths", 1, [&] { return launch_lengths(reinterpret_cast<const long long*>(lengths), encoded_len, B, T, 2, st); });
   }
   // ---- subsampling: conv 1->C, conv C->C, linear (subsampling.py:172-175)
   // bf16 path: patch gather + tcgen05 GEMM (the same form dense and packed, so the two stay bit-identical); the CUDA-core
   // kernel below serves the fp32 validation path
   if (pk || !v) {
-    if (pk) {
-      CFB_TRY(launch_conv0_im2col_packed(feats, feats_dtype == CFB_BF16, reinterpret_cast<const long long*>(lengths),
-                                         ws + pl.a0, pk->first, pk->step, h->F0, T, conv_out(T), h->F1, h->Fh, pk->n_rows, tb,
-                                         st),
-              "subsample conv 0 (gather)");
-    } else {
-      CFB_TRY(launch_conv0_im2col(feats, feats_dtype == CFB_BF16, ws + pl.a0, B, h->F0, T, pl.T1, h->F1, pl.Th, h->Fh, st),
-              "subsample conv 0 (gather)");
-    }
-    ++launches;
+    q(st, "subsample conv 0 (gather)", 1, [&] {
+      return pk ? launch_conv0_im2col_packed(feats, feats_dtype == CFB_BF16, reinterpret_cast<const long long*>(lengths),
+                                             ws + pl.a0.off, pk->first, pk->step, h->F0, T, conv_out(T), h->F1, h->Fh,
+                                             pk->n_rows, tb, st)
+                : launch_conv0_im2col(feats, feats_dtype == CFB_BF16, ws + pl.a0.off, B, h->F0, T, pl.T1, h->F1, pl.Th,
+                                      h->Fh, st);
+    });
     EpiParams ep;
-    ep.out = ws + pl.y1;
+    ep.out = ws + pl.y1.off;
     ep.ldo = C;
-    CFB_TRY(gemm(ws + pl.a0, kConv0Cols, h->sub_w1g, kConv0Cols, Bk * 4 * pl.Th * h->Fh, C, kConv0Cols, EPI_RELU, true, ep,
-                 "subsample conv 0"),
-            "subsample conv 0");
+    gemm(ws + pl.a0.off, kConv0Cols, h->sub_w1g, kConv0Cols, Bk * 4 * pl.Th * h->Fh, C, kConv0Cols, EPI_RELU, true, ep,
+         "subsample conv 0");
   } else {
-  CFB_TRY(launch_subsample_first(feats, feats_dtype == CFB_BF16, h->at<float>(h->sub_w1), h->at<float>(h->sub_b1),
-                                 ws + pl.y1, abf, B, h->F0, T, C, pl.T1, h->F1, pl.Th, h->Fh, st),
-          "subsample conv 0");
-  ++launches;
+    q(st, "subsample conv 0", 1, [&] {
+      return launch_subsample_first(feats, feats_dtype == CFB_BF16, h->at<float>(h->sub_w1), h->at<float>(h->sub_b1),
+                                    ws + pl.y1.off, abf, B, h->F0, T, C, pl.T1, h->F1, pl.Th, h->Fh, st);
+    });
   }
   if (v) {
-    CFB_TRY(launch_im2col(reinterpret_cast<const float*>(ws + pl.y1), reinterpret_cast<float*>(ws + pl.cols), B, C,
-                          pl.Th, h->Fh, T2, F2, st),
-            "im2col");
-    ++launches;
+    q(st, "im2col", 1, [&] {
+      return launch_im2col(reinterpret_cast<const float*>(ws + pl.y1.off), reinterpret_cast<float*>(ws + pl.cols.off), B, C,
+                           pl.Th, h->Fh, T2, F2, st);
+    });
     EpiParams ep;
     ep.bias = h->at<float>(h->sub_b2);
-    ep.out = ws + pl.y2;
+    ep.out = ws + pl.y2.off;
     ep.ldo = C;
-    CFB_TRY(gemm(ws + pl.cols, 9LL * C, h->sub_w2, 9LL * C, N * F2, C, 9 * C, EPI_RELU, false, ep, "subsample conv 2"),
-            "subsample conv 2");
+    gemm(ws + pl.cols.off, 9LL * C, h->sub_w2, 9LL * C, N * F2, C, 9 * C, EPI_RELU, false, ep, "subsample conv 2");
   } else {
     ConvDesc cd;
-    cd.y_in = ws + pl.y1;
+    cd.y_in = ws + pl.y1.off;
     cd.W = h->arena + h->sub_w2.off;
     cd.bias = h->at<float>(h->sub_b2);
-    cd.y_out = ws + pl.y2;
+    cd.y_out = ws + pl.y2.off;
     cd.B = Bk;
     cd.C_in = C;
     cd.C_out = C;
@@ -851,60 +873,58 @@ static int forward_range(cfb_handle* h, const void* feats, int feats_dtype, cons
     cd.Fh = h->Fh;
     cd.To = T2;
     cd.Fo = F2;
-    CFB_TRY(launch_conv_tc(cd, st, &err), "subsample conv 2");
-    ++launches;
+    q(st, "subsample conv 2", 1, [&] { return launch_conv_tc(cd, st, &q.err); });
   }
-  float* x = reinterpret_cast<float*>(ws + pl.x);
+  float* x = reinterpret_cast<float*>(ws + pl.x.off);
   {
     EpiParams ep;
     ep.bias = h->at<float>(h->sub_b3);
     ep.out = x;
     ep.ldo = d;
-    CFB_TRY(gemm(ws + pl.y2, static_cast<long long>(F2) * C, h->sub_w3, static_cast<long long>(F2) * C, N, d, F2 * C,
-                 EPI_LINEAR, false, ep, "pre_encode.out"),
-            "pre_encode.out");
+    gemm(ws + pl.y2.off, static_cast<long long>(F2) * C, h->sub_w3, static_cast<long long>(F2) * C, N, d, F2 * C, EPI_LINEAR,
+         false, ep, "pre_encode.out");
   }
   // ---- relative positional table and its per-layer projections (multi_head_attention.py:186-188, 296-316)
   const int T2pos = pk ? pk->t2_max : T2;  // extent of the relative-position table
-  CFB_TRY(launch_pos_table(ws + pl.pe, abf, h->at<float>(h->div_term), T2pos, d, st), "pos table");
-  ++launches;
+  q(st, "pos table", 1, [&] { return launch_pos_table(ws + pl.pe.off, abf, h->at<float>(h->div_term), T2pos, d, st); });
   {
     EpiParams ep;
-    ep.out = ws + pl.pos;
+    ep.out = ws + pl.pos.off;
     ep.ldo = static_cast<long long>(L) * Dp;
-    CFB_TRY(gemm(ws + pl.pe, d, h->w_pos, d, pl.P, L * Dp, d, EPI_LINEAR, abf, ep, "linear_pos"), "linear_pos");
+    gemm(ws + pl.pe.off, d, h->w_pos, d, pl.P, L * Dp, d, EPI_LINEAR, abf, ep, "linear_pos");
   }
   if (abf) {
     // the attention kernels compute the position term from fp16 operands into an fp16 accumulator (attention_tc.cu): the
     // projections of all layers are converted once, in place
-    CFB_TRY(launch_bf16_to_f16(ws + pl.pos, static_cast<long long>(L) * Dp, ws + pl.pos, pl.P, L * Dp, st), "linear_pos -> fp16");
-    ++launches;
+    q(st, "linear_pos -> fp16", 1, [&] {
+      return launch_bf16_to_f16(ws + pl.pos.off, static_cast<long long>(L) * Dp, ws + pl.pos.off, pl.P, L * Dp, st);
+    });
   }
 
   const int32_t* lens = encoded_len;
-  void* a = ws + pl.a;
+  void* a = ws + pl.a.off;
   for (int l = 0; l < L; ++l) {
     const LayerW& lw = h->layers[l];
     // -- feed forward 1 (conformer_modules.py:98-101)
     for (int f = 0; f < 2; ++f) {
       if (f == 1) {
         // -- self attention (conformer_modules.py:103-110)
-        CFB_TRY(launch_layernorm(x, h->at<float>(lw.ln_g[1]), h->at<float>(lw.ln_b[1]), a, abf, N, d, nullptr, 1, st),
-                "norm_self_att");
-        ++launches;
+        q(st, "norm_self_att", 1, [&] {
+          return launch_layernorm(x, h->at<float>(lw.ln_g[1]), h->at<float>(lw.ln_b[1]), a, abf, N, d, nullptr, 1, st);
+        });
         EpiParams ep;
         ep.bias = h->at<float>(lw.b_qkv);
         ep.bias2 = h->at<float>(lw.b_qv);
-        ep.out = ws + pl.qkv;
+        ep.out = ws + pl.qkv.off;
         ep.ldo = 4LL * Dp;
         ep.qkv_dp = Dp;
-        CFB_TRY(gemm(a, d, lw.w_qkv, d, N, 3 * Dp, d, EPI_QKV, abf, ep, "qkv projection"), "qkv projection");
+        gemm(a, d, lw.w_qkv, d, N, 3 * Dp, d, EPI_QKV, abf, ep, "qkv projection");
         AttnDesc ad;
-        ad.qkv = ws + pl.qkv;
-        ad.pos = ws + pl.pos + static_cast<size_t>(l) * Dp * h->esz();
+        ad.qkv = ws + pl.qkv.off;
+        ad.pos = ws + pl.pos.off + static_cast<size_t>(l) * Dp * h->esz();
         ad.ld_pos = static_cast<long long>(L) * Dp;
         ad.pos_f16 = abf;
-        ad.ctx = ws + pl.ctx;
+        ad.ctx = ws + pl.ctx.off;
         ad.lens = lens;
         ad.B = B;
         ad.T = T2pos;
@@ -916,21 +936,20 @@ static int forward_range(cfb_handle* h, const void* feats, int feats_dtype, cons
           ad.n_tiles = pk->n_tiles;
           ad.rows = N;
         }
-        CFB_TRY(v ? launch_attn_simt(ad, st, &err) : launch_attn_tc(ad, st, &err), "rel-pos attention");
-        ++launches;
+        q(st, "rel-pos attention", 1, [&] { return v ? launch_attn_simt(ad, st, &q.err) : launch_attn_tc(ad, st, &q.err); });
         EpiParams eo;
         eo.bias = h->at<float>(lw.b_out);
         eo.out = x;
         eo.ldo = d;
         eo.alpha = 1.f;
-        CFB_TRY(gemm(ws + pl.ctx, Dp, lw.w_out, Dp, N, d, Dp, EPI_RESID, false, eo, "linear_out"), "linear_out");
+        gemm(ws + pl.ctx.off, Dp, lw.w_out, Dp, N, d, Dp, EPI_RESID, false, eo, "linear_out");
         // -- convolution module (conformer_modules.py:112-114, 160-180)
-        CFB_TRY(launch_layernorm(x, h->at<float>(lw.ln_g[2]), h->at<float>(lw.ln_b[2]), a, abf, N, d, nullptr, 1, st),
-                "norm_conv");
-        ++launches;
+        q(st, "norm_conv", 1, [&] {
+          return launch_layernorm(x, h->at<float>(lw.ln_g[2]), h->at<float>(lw.ln_b[2]), a, abf, N, d, nullptr, 1, st);
+        });
         EpiParams eg;
         eg.bias = h->at<float>(lw.b_pw1);
-        eg.out = ws + pl.g;
+        eg.out = ws + pl.g.off;
         eg.ldo = d;
         if (pk) {
           eg.row_t = tb.row_t;  // zero at the gap rows: the depth-wise halo of a slot must not see its neighbours
@@ -938,11 +957,11 @@ static int forward_range(cfb_handle* h, const void* feats, int feats_dtype, cons
           eg.lens = lens;
           eg.frames_per_seq = T2;
         }
-        CFB_TRY(gemm(a, d, lw.w_pw1, d, N, 2 * d, d, EPI_GLU, abf, eg, "pointwise_conv1+glu"), "pointwise_conv1+glu");
+        gemm(a, d, lw.w_pw1, d, N, 2 * d, d, EPI_GLU, abf, eg, "pointwise_conv1+glu");
         if (fused_tail) {
           // depthwise + BatchNorm + Swish + pointwise_conv2 + residual in one kernel (conv_tail.cu)
           DwPwDesc dp;
-          dp.g = ws + pl.g;
+          dp.g = ws + pl.g.off;
           dp.taps32 = h->at<float>(lw.dw_taps32);
           dp.W = h->arena + lw.w_pw2.off;
           dp.bias2 = h->at<float>(lw.b_pw2);
@@ -950,68 +969,53 @@ static int forward_range(cfb_handle* h, const void* feats, int feats_dtype, cons
           dp.B = Bk;
           dp.T = T2;
           dp.d = d;
-          CFB_TRY(launch_dw_pw(dp, st, &err), "depthwise+pointwise_conv2");
-          ++launches;
+          q(st, "depthwise+pointwise_conv2", 1, [&] { return launch_dw_pw(dp, st, &q.err); });
         } else {
-        CFB_TRY(launch_depthwise(ws + pl.g, h->at<float>(lw.dw_taps), h->at<float>(lw.dw_bias), ws + pl.c, abf, Bk, T2,
-                                 d, h->ksize, st),
-                "depthwise conv");
-        ++launches;
-        EpiParams e2;
-        e2.bias = h->at<float>(lw.b_pw2);
-        e2.out = x;
-        e2.ldo = d;
-        e2.alpha = 1.f;
-        CFB_TRY(gemm(ws + pl.c, d, lw.w_pw2, d, N, d, d, EPI_RESID, false, e2, "pointwise_conv2"), "pointwise_conv2");
+          q(st, "depthwise conv", 1, [&] {
+            return launch_depthwise(ws + pl.g.off, h->at<float>(lw.dw_taps), h->at<float>(lw.dw_bias), ws + pl.c.off, abf, Bk,
+                                    T2, d, h->ksize, st);
+          });
+          EpiParams e2;
+          e2.bias = h->at<float>(lw.b_pw2);
+          e2.out = x;
+          e2.ldo = d;
+          e2.alpha = 1.f;
+          gemm(ws + pl.c.off, d, lw.w_pw2, d, N, d, d, EPI_RESID, false, e2, "pointwise_conv2");
         }
       }
       const int ln = f == 0 ? 0 : 3;
       if (!(f == 0 && l > 0 && abf)) {  // bf16 path: norm_feed_forward1 of layers > 0 is fused into the previous norm_out
-        CFB_TRY(launch_layernorm(x, h->at<float>(lw.ln_g[ln]), h->at<float>(lw.ln_b[ln]), a, abf, N, d, nullptr, 1, st),
-                "norm_feed_forward");
-        ++launches;
+        q(st, "norm_feed_forward", 1, [&] {
+          return launch_layernorm(x, h->at<float>(lw.ln_g[ln]), h->at<float>(lw.ln_b[ln]), a, abf, N, d, nullptr, 1, st);
+        });
       }
       EpiParams e1;
       e1.bias = h->at<float>(lw.ff_b1[f]);
-      e1.out = ws + pl.hbuf;
+      e1.out = ws + pl.hbuf.off;
       e1.ldo = dff;
-      CFB_TRY(gemm(a, d, lw.ff_w1[f], d, N, dff, d, EPI_SWISH, abf, e1, "linear1+swish"), "linear1+swish");
+      gemm(a, d, lw.ff_w1[f], d, N, dff, d, EPI_SWISH, abf, e1, "linear1+swish");
       EpiParams e2;
       e2.bias = h->at<float>(lw.ff_b2[f]);
       e2.out = x;
       e2.ldo = d;
       e2.alpha = 0.5f;  // fc_factor (conformer_modules.py:57,101,118)
-      CFB_TRY(gemm(ws + pl.hbuf, dff, lw.ff_w2[f], dff, N, d, dff, EPI_RESID, false, e2, "linear2"), "linear2");
+      gemm(ws + pl.hbuf.off, dff, lw.ff_w2[f], dff, N, d, dff, EPI_RESID, false, e2, "linear2");
     }
     // -- norm_out (conformer_modules.py:120); the last one writes the result
-    const bool last = (l == L - 1);
-    if (last && pk) {
-      // the dense (B, T', d) result of the reference API: zeros, then the valid rows of every slot (packed.cu)
-      if (pk->prologue) {
-        const size_t out_bytes = static_cast<size_t>(B) * pk->t2_max * d * (out_dtype == CFB_BF16 ? 2 : 4);
-        if (cudaMemsetAsync(encoded, 0, out_bytes, st) != cudaSuccess)
-          return fail(h, CFB_ERR_CUDA, "cfb_forward_packed: memset failed");
+    const bool last = l == L - 1;
+    const float* g4 = h->at<float>(lw.ln_g[4]);
+    const float* b4 = h->at<float>(lw.ln_b[4]);
+    q(st, "norm_out", 1, [&] {
+      if (last && pk)  // the valid rows of every slot into the dense (B, T', d) result of the reference API (packed.cu)
+        return launch_layernorm_scatter(x, g4, b4, encoded, out_dtype == CFB_BF16, N, d, tb.row_out, st);
+      if (last && !h->has_out_proj) return launch_layernorm(x, g4, b4, encoded, out_dtype == CFB_BF16, N, d, lens, T2, st);
+      if (last) return launch_layernorm(x, g4, b4, a, abf, N, d, nullptr, 1, st);
+      if (abf) {
+        const LayerW& nx = h->layers[l + 1];
+        return launch_layernorm_dual(x, g4, b4, x, h->at<float>(nx.ln_g[0]), h->at<float>(nx.ln_b[0]), a, N, d, st);
       }
-      CFB_TRY(launch_layernorm_scatter(x, h->at<float>(lw.ln_g[4]), h->at<float>(lw.ln_b[4]), encoded, out_dtype == CFB_BF16,
-                                       N, d, tb.row_out, st),
-              "norm_out");
-    } else if (last && !h->has_out_proj) {
-      CFB_TRY(launch_layernorm(x, h->at<float>(lw.ln_g[4]), h->at<float>(lw.ln_b[4]), encoded, out_dtype == CFB_BF16, N,
-                               d, lens, T2, st),
-              "norm_out");
-    } else if (last) {
-      CFB_TRY(launch_layernorm(x, h->at<float>(lw.ln_g[4]), h->at<float>(lw.ln_b[4]), a, abf, N, d, nullptr, 1, st),
-              "norm_out");
-    } else if (abf) {
-      const LayerW& nx = h->layers[l + 1];
-      CFB_TRY(launch_layernorm_dual(x, h->at<float>(lw.ln_g[4]), h->at<float>(lw.ln_b[4]), x, h->at<float>(nx.ln_g[0]),
-                                    h->at<float>(nx.ln_b[0]), a, N, d, st),
-              "norm_out");
-    } else {
-      CFB_TRY(launch_layernorm(x, h->at<float>(lw.ln_g[4]), h->at<float>(lw.ln_b[4]), x, false, N, d, nullptr, 1, st),
-              "norm_out");
-    }
-    ++launches;
+      return launch_layernorm(x, g4, b4, x, false, N, d, nullptr, 1, st);
+    });
   }
   if (h->has_out_proj) {  // conformer_encoder.py:277-278
     EpiParams ep;
@@ -1020,56 +1024,42 @@ static int forward_range(cfb_handle* h, const void* feats, int feats_dtype, cons
     ep.ldo = h->d_out;
     ep.lens = lens;
     ep.frames_per_seq = T2;
-    CFB_TRY(gemm(a, d, h->w_oproj, d, N, h->d_out, d, EPI_LINEAR, out_dtype == CFB_BF16, ep, "out_proj"), "out_proj");
+    gemm(a, d, h->w_oproj, d, N, h->d_out, d, EPI_LINEAR, out_dtype == CFB_BF16, ep, "out_proj");
   }
-#undef CFB_TRY
-  *launches_out += launches;
-  return CFB_OK;
+  return q.rc;
 }
+
+}  // namespace
 
 extern "C" {
 
 int cfb_forward(cfb_handle* h, const void* feats, int feats_dtype, const int64_t* lengths, int B, int T, void* encoded,
                 int out_dtype, int32_t* encoded_len, void* workspace, size_t ws_bytes, cfb_stream stream) {
-  if (!h) return CFB_ERR_INVALID_ARG;
-  if (!h->finalized) return fail(h, CFB_ERR_STATE, "cfb_forward: weights are not finalized");
-  if (!feats || !encoded || !encoded_len || !workspace || B < 1 || T < 1)
-    return fail(h, CFB_ERR_INVALID_ARG, "cfb_forward: null pointer or empty batch");
-  if (feats_dtype != CFB_F32 && feats_dtype != CFB_BF16)
-    return fail(h, CFB_ERR_INVALID_ARG, "cfb_forward: feats must be f32 or bf16");
-  if (out_dtype != CFB_F32 && out_dtype != CFB_BF16)
-    return fail(h, CFB_ERR_INVALID_ARG, "cfb_forward: encoded must be f32 or bf16");
-  if (ws_bytes < workspace_need(h, B, T) || (reinterpret_cast<uintptr_t>(workspace) & 255))
+  if (int rc = check_forward(h, "cfb_forward", feats, feats_dtype, encoded, out_dtype, encoded_len, workspace, B, T)) return rc;
+  if (ws_bytes < dense_workspace(h, B, T) || (reinterpret_cast<uintptr_t>(workspace) & 255))
     return fail(h, CFB_ERR_WORKSPACE, "cfb_forward: workspace too small or not 256-byte aligned");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  int launches = 0;
-  set_pdl_auto(static_cast<long long>(B) * conv_out(conv_out(T)) <= 4096);
-  // Utterances are independent, so a batch can run as two half-batches on two streams (fork / join with events,
-  // capturable): the halves' kernels interleave on the GPU -- one half's memory-bound LayerNorms and kernel tails
-  // overlap the other half's GEMMs instead of leaving the tensor cores idle.  Results are identical to the
-  // single-stream schedule (every row sees the same padded extent T).  Off while per-kernel profiling is on.
-  const int b0 = h->profiling ? 0 : micro_split(h, B);
-  if (b0 == 0) {
-    int rc = forward_range(h, feats, feats_dtype, lengths, B, T, encoded, out_dtype, encoded_len, workspace, st, &launches, B);
-    h->launches = launches;
-    return rc;
-  }
-  const int b1 = B - b0;
   const int t_out = conv_out(conv_out(T));
+  set_pdl_auto(static_cast<long long>(B) * t_out <= 4096);
+  const bool fused_tail = use_fused_tail(h, static_cast<long long>(B) * ((t_out + 127) / 128));
+  Enqueue q(h, st);
+  // Utterances are independent, so a batch can run as two half-batches on two streams (run_parts).  Results are
+  // identical to the single-stream schedule (every row sees the same padded extent T).  Off while per-kernel profiling
+  // is on.
+  const int n = h->profiling ? 1 : dense_parts(h, B);
   const size_t in_es = feats_dtype == CFB_F32 ? 4 : 2, out_es = out_dtype == CFB_F32 ? 4 : 2;
-  const uint8_t* feats1 = reinterpret_cast<const uint8_t*>(feats) + static_cast<size_t>(b0) * h->F0 * T * in_es;
-  uint8_t* enc1 = reinterpret_cast<uint8_t*>(encoded) + static_cast<size_t>(b0) * t_out * h->d_out * out_es;
-  uint8_t* ws1 = reinterpret_cast<uint8_t*>(workspace) + make_plan(h, b0, T).total;
-  if (cudaEventRecord(h->ev_fork, st) != cudaSuccess || cudaStreamWaitEvent(h->aux_stream, h->ev_fork, 0) != cudaSuccess)
-    return fail(h, CFB_ERR_CUDA, "cfb_forward: stream fork failed");
-  int rc = forward_range(h, feats, feats_dtype, lengths, b0, T, encoded, out_dtype, encoded_len, workspace, st, &launches, B);
-  int rc1 = forward_range(h, feats1, feats_dtype, lengths ? lengths + b0 : nullptr, b1, T, enc1, out_dtype, encoded_len + b0,
-                          ws1, h->aux_stream, &launches, B);
-  // always join, even after an error, so a capture in progress is not left with a dangling branch
-  cudaEventRecord(h->ev_join, h->aux_stream);
-  cudaStreamWaitEvent(st, h->ev_join, 0);
-  h->launches = launches;
-  return rc != CFB_OK ? rc : rc1;
+  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
+  return run_parts(h, st, n, [&](int i, cudaStream_t s) {
+    const Range r = dense_part(B, n, i);
+    const Plan pl = make_plan(h, r.count, T);
+    const int rc = forward_range(h, q, s, pl, nullptr, fused_tail,
+                                 reinterpret_cast<const uint8_t*>(feats) + static_cast<size_t>(r.first) * h->F0 * T * in_es,
+                                 feats_dtype, lengths ? lengths + r.first : nullptr, r.count, T,
+                                 reinterpret_cast<uint8_t*>(encoded) + static_cast<size_t>(r.first) * t_out * h->d_out * out_es,
+                                 out_dtype, encoded_len + r.first, ws);
+    ws += pl.total;
+    return rc;
+  });
 }
 
 }  // extern "C"
@@ -1092,84 +1082,47 @@ static int packed_groups(const cfb_handle* h, int B, int n_rows) {
   g = std::min(std::min(g, B), cfb_handle::kMaxGroups);
   return std::max(g, 1);
 }
-static size_t packed_plan_bytes(const cfb_handle* h, int B, int T, const PackedShape& ps) {
-  return make_plan(h, B, T, ps.n_rows, ps.t2_max, ps.count, ps.n_tiles).total;
-}
-static size_t packed_workspace_need(const cfb_handle* h, const int64_t* lengths_host, int B, int T) {
-  size_t need = 0;
-  for (int groups = 1; groups <= std::min(B, cfb_handle::kMaxGroups); ++groups) {
-    size_t sum = 0;
-    for (int g = 0; g < groups; ++g) sum += packed_plan_bytes(h, B, T, packed_shape(lengths_host, B, T, g, groups));
-    need = std::max(need, sum);
-  }
-  return need;
-}
 
 extern "C" {
 
 int cfb_packed_workspace_bytes(const cfb_handle* h, const int64_t* lengths_host, int B, int T, size_t* out) {
   if (!h || !out || B < 1 || T < 1) return fail(h, CFB_ERR_INVALID_ARG, "cfb_packed_workspace_bytes: bad argument");
-  *out = packed_workspace_need(h, lengths_host, B, T);
+  *out = packed_workspace(h, lengths_host, B, T);
   return CFB_OK;
 }
 
 int cfb_forward_packed(cfb_handle* h, const void* feats, int feats_dtype, const int64_t* lengths, const int64_t* lengths_host,
                        int B, int T, void* encoded, int out_dtype, int32_t* encoded_len, void* workspace, size_t ws_bytes,
                        cfb_stream stream) {
-  if (!h) return CFB_ERR_INVALID_ARG;
-  if (!h->finalized) return fail(h, CFB_ERR_STATE, "cfb_forward_packed: weights are not finalized");
-  if (!feats || !encoded || !encoded_len || !workspace || B < 1 || T < 1)
-    return fail(h, CFB_ERR_INVALID_ARG, "cfb_forward_packed: null pointer or empty batch");
+  if (int rc = check_forward(h, "cfb_forward_packed", feats, feats_dtype, encoded, out_dtype, encoded_len, workspace, B, T))
+    return rc;
   if ((lengths == nullptr) != (lengths_host == nullptr))
     return fail(h, CFB_ERR_INVALID_ARG, "cfb_forward_packed: lengths and lengths_host must both be given (or both NULL)");
-  if (feats_dtype != CFB_F32 && feats_dtype != CFB_BF16)
-    return fail(h, CFB_ERR_INVALID_ARG, "cfb_forward_packed: feats must be f32 or bf16");
-  if (out_dtype != CFB_F32 && out_dtype != CFB_BF16)
-    return fail(h, CFB_ERR_INVALID_ARG, "cfb_forward_packed: encoded must be f32 or bf16");
   if (h->validate) return fail(h, CFB_ERR_UNSUPPORTED, "cfb_forward_packed: the fp32 validation path runs dense batches only");
   if (h->has_out_proj) return fail(h, CFB_ERR_UNSUPPORTED, "cfb_forward_packed: out_proj (feat_out != d_model) runs dense batches only");
   if (B > 2048) return fail(h, CFB_ERR_UNSUPPORTED, "cfb_forward_packed: at most 2048 utterances per call");
-  if (ws_bytes < packed_workspace_need(h, lengths_host, B, T) || (reinterpret_cast<uintptr_t>(workspace) & 255))
+  if (ws_bytes < packed_workspace(h, lengths_host, B, T) || (reinterpret_cast<uintptr_t>(workspace) & 255))
     return fail(h, CFB_ERR_WORKSPACE, "cfb_forward_packed: workspace too small or not 256-byte aligned");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  int launches = 0;
   const PackedShape ps = packed_shape(lengths_host, B, T);
   set_pdl_auto(ps.n_rows <= kSmallBatchRows);
-  const int groups = packed_groups(h, B, ps.n_rows);
-  if (groups == 1) {
-    int rc = forward_range(h, feats, feats_dtype, lengths, B, T, encoded, out_dtype, encoded_len, workspace, st, &launches, B, &ps);
-    h->launches = launches;
+  const bool fused_tail = use_fused_tail(h, (ps.n_rows + 127) / 128);
+  const int n = packed_groups(h, B, ps.n_rows);
+  Enqueue q(h, st);
+  // encoded_len and the cleared dense result are needed by every group: enqueue them, then fork
+  if (q(st, "lengths", 1, [&] { return launch_lengths(reinterpret_cast<const long long*>(lengths), encoded_len, B, T, 2, st); }))
+    return q.rc;
+  const size_t out_bytes = static_cast<size_t>(B) * ps.t2_max * h->d * (out_dtype == CFB_BF16 ? 2 : 4);
+  if (cudaMemsetAsync(encoded, 0, out_bytes, st) != cudaSuccess) return fail(h, CFB_ERR_CUDA, "cfb_forward_packed: memset failed");
+  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
+  return run_parts(h, st, n, [&](int g, cudaStream_t s) {
+    const PackedShape gs = packed_shape(lengths_host, B, T, g, n);
+    const Plan pl = make_plan(h, B, T, &gs);
+    const int rc = forward_range(h, q, s, pl, &gs, fused_tail, feats, feats_dtype, lengths, B, T, encoded, out_dtype,
+                                 encoded_len, ws);
+    ws += pl.total;
     return rc;
-  }
-  // encoded_len and the cleared result are needed by every group: enqueue them, then fork
-  if (launch_lengths(reinterpret_cast<const long long*>(lengths), encoded_len, B, T, 2, st) != 0)
-    return fail(h, CFB_ERR_CUDA, "cfb_forward_packed: lengths kernel failed");
-  ++launches;
-  {
-    const size_t out_bytes = static_cast<size_t>(B) * ps.t2_max * h->d * (out_dtype == CFB_BF16 ? 2 : 4);
-    if (cudaMemsetAsync(encoded, 0, out_bytes, st) != cudaSuccess) return fail(h, CFB_ERR_CUDA, "cfb_forward_packed: memset failed");
-  }
-  if (cudaEventRecord(h->ev_fork, st) != cudaSuccess) return fail(h, CFB_ERR_CUDA, "cfb_forward_packed: stream fork failed");
-  for (int g = 1; g < groups; ++g)
-    if (cudaStreamWaitEvent(h->group_stream[g], h->ev_fork, 0) != cudaSuccess)
-      return fail(h, CFB_ERR_CUDA, "cfb_forward_packed: stream fork failed");
-  int rc = CFB_OK;
-  uint8_t* wsg = reinterpret_cast<uint8_t*>(workspace);
-  for (int g = 0; g < groups; ++g) {
-    PackedShape gs = packed_shape(lengths_host, B, T, g, groups);
-    gs.prologue = false;
-    const int r = forward_range(h, feats, feats_dtype, lengths, B, T, encoded, out_dtype, encoded_len, wsg,
-                                g == 0 ? st : h->group_stream[g], &launches, B, &gs);
-    if (rc == CFB_OK) rc = r;
-    wsg += packed_plan_bytes(h, B, T, gs);
-  }
-  // always join, even after an error, so a capture in progress is not left with a dangling branch
-  for (int g = 1; g < groups; ++g) {
-    cudaEventRecord(h->group_join[g], h->group_stream[g]);
-    cudaStreamWaitEvent(st, h->group_join[g], 0);
-  }
-  h->launches = launches;
-  return rc;
+  });
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

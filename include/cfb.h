@@ -125,8 +125,10 @@ CFB_API int cfb_forward_packed(cfb_handle* h, const void* feats, int feats_dtype
                        const int64_t* lengths_host, int B, int T, void* encoded, int out_dtype, int32_t* encoded_len,
                        void* workspace, size_t ws_bytes, cfb_stream stream);
 
-/* Where an intermediate lives inside the workspace of a (B, T) forward (tests / debugging): name is one of
- * "y1" "y2" "x" "a" "h" "qkv" "ctx" "g" "c" "pe" "pos".  Offsets are bytes from the workspace base. */
+/* Where an intermediate lives inside the workspace of a (B, T) cfb_forward (tests / debugging): name is one of
+ * "y1" "y2" "x" "a" "h" "qkv" "ctx" "g" "c" "pe" "pos".  Offsets are bytes from the workspace base.  A bf16 batch of
+ * B >= 8 runs as two half-batches, each with a workspace layout of its own, so for it the call returns
+ * CFB_ERR_INVALID_ARG: ask for B <= 7, or use CFB_PREC_FP32_VALIDATE (never split). */
 CFB_API int cfb_debug_buffer(const cfb_handle* h, int B, int T, const char* name, size_t* offset, size_t* bytes);
 
 /* Per-kernel timing (bench.py's roofline): when on, cfb_forward brackets every launch with CUDA events on the

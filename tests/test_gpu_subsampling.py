@@ -4,7 +4,7 @@ is the device's own input to that stage, so every stage is judged by its own rou
 Stages: the first strided conv (y1), the implicit-GEMM second conv (y2), the sinusoid table (pe), the per-layer
 linear_pos projections in their head packing (pos, fp16 on the bf16 path), the attention of the last layer (ctx) and
 the final norm_out (encoded).  Buffers are read with ConformerEncoder.debug_buffer after a dense forward with B <= 7
-(from B = 8 on, cfb_forward splits the batch into two half-batch plans and the debug offsets describe neither).
+(from B = 8 on, cfb_forward splits a bf16 batch into two half-batch plans and cfb_debug_buffer refuses it).
 
 Tolerances are bounds, not measurements: u = 2^-24 is the fp32 unit roundoff, S the same sum taken over magnitudes
 (so the fp32 accumulation of n terms is off by at most n * u * S), and a rounded output may move by one ulp of its

@@ -135,9 +135,12 @@ bool gemm_tc2_supported(const GemmDesc& g);
 int launch_gemm_tc2(const GemmDesc& g, cudaStream_t st, std::string* err);
 int launch_conv_tc(const ConvDesc& c, cudaStream_t st, std::string* err);
 int launch_gemm_simt(const GemmDesc& g, float* scratch, cudaStream_t st, std::string* err);
+// tensor-core attention: dkp 64 -> attention_tc.cu / attention_tcp.cu, dkp 128 -> attention_tc128.cu
 int launch_attn_tc(const AttnDesc& a, cudaStream_t st, std::string* err);
 // persistent form (one CTA per SM walks over the (query tile, head, sequence) items; attention_tcp.cu)
 int launch_attn_tcp(const AttnDesc& a, cudaStream_t st, std::string* err);
+// heads 64 < dk <= 128, padded to 128 columns (attention_tc128.cu); per-item form only
+int launch_attn_tc128(const AttnDesc& a, cudaStream_t st, std::string* err);
 int launch_attn_simt(const AttnDesc& a, cudaStream_t st, std::string* err);
 // fp16 view of the positional projections for the tensor-core attention kernels (attention_tc.cu)
 const void* attn_pos_f16(const AttnDesc& a, int Dp, cudaStream_t st);

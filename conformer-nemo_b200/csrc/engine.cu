@@ -294,7 +294,7 @@ int cfb_create(const cfb_config* cfg, int device, cfb_handle** out) {
     return bad(CFB_ERR_UNSUPPORTED, "only subsampling_factor=4 (two strided convolutions) is supported");
   if (cfg->d_model % 16) return bad(CFB_ERR_UNSUPPORTED, "d_model must be a multiple of 16");
   if (cfg->d_model > 1024) return bad(CFB_ERR_UNSUPPORTED, "d_model > 1024 is not supported");
-  if (cfg->d_model / cfg->n_heads > 64) return bad(CFB_ERR_UNSUPPORTED, "head dimension > 64 is not supported");
+  if (cfg->d_model / cfg->n_heads > 128) return bad(CFB_ERR_UNSUPPORTED, "head dimension > 128 is not supported");
   if ((cfg->d_model / cfg->n_heads) % 2) return bad(CFB_ERR_UNSUPPORTED, "head dimension must be even");
   if (cfg->conv_kernel_size < 1 || cfg->conv_kernel_size > 31 || cfg->conv_kernel_size % 2 == 0)
     return bad(CFB_ERR_UNSUPPORTED, "conv_kernel_size must be odd and <= 31");
@@ -323,7 +323,7 @@ int cfb_create(const cfb_config* cfg, int device, cfb_handle** out) {
   h->dff = cfg->d_model * cfg->ff_expansion_factor;
   h->H = cfg->n_heads;
   h->dk = h->d / h->H;
-  h->dkp = 64;
+  h->dkp = h->dk <= 64 ? 64 : 128;  // every head padded to the width of its attention kernel (attention_tc.cu / _tc128.cu)
   h->Dp = h->H * h->dkp;
   h->L = cfg->n_layers;
   h->ksize = cfg->conv_kernel_size;
@@ -1239,6 +1239,10 @@ int cfb_op_rel_attention(int use_tc, const void* qkv, const void* pos, int64_t l
   a.H = H;
   a.dk = dk;
   a.dkp = dkp;
+  if (use_tc && ((dkp != 64 && dkp != 128) || dk < 1 || dk > dkp)) {
+    op_fail(-1, "rel_attention: the tensor-core path takes dkp 64 or 128 and 1 <= dk <= dkp");
+    return CFB_ERR_INVALID_ARG;
+  }
   std::string err;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   int rc = use_tc ? launch_attn_tc(a, st, &err) : launch_attn_simt(a, st, &err);

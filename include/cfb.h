@@ -61,7 +61,8 @@ typedef struct cfb_config {
   int32_t subsampling_factor;        /* power of two >= 2; 'striding' is the only supported scheme             */
   int32_t subsampling_conv_channels; /* -1 = d_model                                                           */
   int32_t ff_expansion_factor;
-  int32_t n_heads;
+  int32_t n_heads;                   /* head dimension d_model / n_heads even and <= 128 (heads <= 64 wide are   */
+                                     /* padded to 64 columns, wider ones to 128)                               */
   int32_t conv_kernel_size;          /* odd, <= 31 + ... (depth-wise taps)                                     */
   int32_t xscaling;                  /* 1: multiply pre_encode output by sqrt(d_model) (multi_head_attention.py:305) */
   int32_t precision;                 /* cfb_precision                                                          */
@@ -205,7 +206,9 @@ CFB_API int cfb_op_logmel(const float* audio, const int64_t* lengths, int B, int
  *   pos  (2T-1 rows, ld_pos): linear_pos(pos_emb) for this layer, same head packing, row k <-> relative position T-1-k
  *   ctx  (B*T, Dp): softmax((q+u)k^T + rel_shift((q+v)p^T)) / sqrt(dk)) v, keys >= lens[b] excluded, query rows
  *        >= lens[b] written as zeros.
- * use_tensor_cores != 0: bf16 in/out, fused flash-style tcgen05 kernel (no T x T matrix in HBM); == 0: fp32 CUDA-core kernel. */
+ * use_tensor_cores != 0: bf16 in/out, fused flash-style tcgen05 kernel (no T x T matrix in HBM) for dkp 64 or 128 with
+ *   1 <= dk <= dkp (pad columns dk..dkp-1 of q, k, v and pos must be zero), anything else returns CFB_ERR_INVALID_ARG;
+ *   == 0: fp32 CUDA-core kernel (any dkp). */
 CFB_API int cfb_op_rel_attention(int use_tensor_cores, const void* qkv, const void* pos, int64_t ld_pos, void* ctx,
                          const int32_t* lens, int B, int T, int H, int dk, int dkp, cfb_stream stream);
 

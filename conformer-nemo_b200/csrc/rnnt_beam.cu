@@ -51,7 +51,7 @@ struct BeamParams {
   const float *embed, *w_ih, *w_hh, *b_ih, *b_hh, *w_pred, *b_pred, *w_out, *b_out;
   const float* encp;         // (B*T, J) = joint.enc(encoded)
   const int32_t* lens;
-  unsigned int* counter;     // grid barrier + phase clocks
+  unsigned int* counter;     // grid barrier
   int* work;                 // [kMaxB][kWork]
   float* logits;             // [B][V1]
   int4* nodes;               // [B][max_nodes] (token, parent, frame, state slot)
@@ -162,21 +162,7 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_beam_kernel(const BeamParams
   __shared__ int c_t, c_len, c_sym, c_nh, c_nk, c_nodes, c_states, c_pops, c_cur, c_done, c_pops_total, c_pops_max, c_why;
   __shared__ double c_score;
 
-  for (int i = tid; i < nu * 4 * (K2 / 4); i += kThreads) {
-    const int k4 = i % (K2 / 4), r = i / (K2 / 4), gate = r & 3, ul = r >> 2;
-    const int row = gate * H + u_lo + ul;
-    const float* src = k4 < H / 4 ? p.w_ih + static_cast<size_t>(row) * H + k4 * 4
-                                  : p.w_hh + static_cast<size_t>(row) * H + (k4 - H / 4) * 4;
-    reinterpret_cast<float4*>(s_wl)[i] = __ldg(reinterpret_cast<const float4*>(src));
-  }
-  for (int i = tid; i < nu * 4; i += kThreads) {
-    const int row = (i & 3) * H + u_lo + (i >> 2);
-    s_bl[i] = p.b_ih[row] + p.b_hh[row];
-  }
-  for (int i = tid; i < np * (H / 4); i += kThreads)
-    reinterpret_cast<float4*>(s_wp)[i] = __ldg(reinterpret_cast<const float4*>(p.w_pred + static_cast<size_t>(p_lo) * H) + i);
-  for (int i = tid; i < nj * (J / 4); i += kThreads)
-    reinterpret_cast<float4*>(s_wj)[i] = __ldg(reinterpret_cast<const float4*>(p.w_out + static_cast<size_t>(j_lo) * J) + i);
+  load_row_weights(p, u_lo, nu, p_lo, np, j_lo, nj, s_wl, s_bl, s_wp, s_wj);
 
   const int b_own = cta < B ? cta : -1;
   int4* nodes = b_own >= 0 ? p.nodes + static_cast<size_t>(b_own) * p.max_nodes : nullptr;
@@ -334,14 +320,6 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_beam_kernel(const BeamParams
   unsigned int bar_target = 0;
   grid_sync(p.counter, bar_target);
 
-  unsigned long long* timers = reinterpret_cast<unsigned long long*>(p.counter + 16);
-  long long tk = clock64();
-#define BEAM_TICK(slot)                                        \
-  if (cta == 0 && tid == 0) {                                  \
-    const long long now = clock64();                           \
-    timers[slot] += static_cast<unsigned long long>(now - tk); \
-    tk = now;                                                  \
-  }
   for (;;) {
     // ---- the work records of this iteration (identical in every CTA) --------------------------------------------------
     for (int i = tid; i < B * kWork; i += kThreads) s_wk[i / kWork][i % kWork] = __ldcg(p.work + i);
@@ -358,8 +336,6 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_beam_kernel(const BeamParams
     __syncthreads();
     const int n_active = s_na, n_need = s_nn;
     if (n_active == 0) break;
-    if (cta == 0 && tid == 0) timers[6] += 1;  // lock-step iterations
-    BEAM_TICK(7)
 
     if (n_need > 0) {
       // ---- A: LSTM cell of the new nodes, my hidden units ----------------------------------------------------------------
@@ -396,9 +372,7 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_beam_kernel(const BeamParams
         }
         __syncthreads();
       }
-      BEAM_TICK(0)
       grid_sync(p.counter, bar_target);
-      BEAM_TICK(4)
       // ---- B: joint.pred of the new nodes, my rows ----------------------------------------------------------------------
       const int tile_p = min(kMaxB, p.stage_floats / H);
       for (int s0 = 0; np > 0 && s0 < n_need; s0 += tile_p) {
@@ -417,9 +391,7 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_beam_kernel(const BeamParams
         }
         __syncthreads();
       }
-      BEAM_TICK(1)
       grid_sync(p.counter, bar_target);
-      BEAM_TICK(4)
     }
 
     // ---- C: joint logits of my output rows for every active utterance at (frame, popped node) -----------------------------
@@ -442,9 +414,7 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_beam_kernel(const BeamParams
       }
       __syncthreads();
     }
-    BEAM_TICK(2)
     grid_sync(p.counter, bar_target);
-    BEAM_TICK(4)
 
     // ---- D: control of the owned utterance ------------------------------------------------------------------------------
     if (b_own >= 0 && s_wk[b_own][W_ACTIVE]) {
@@ -581,15 +551,13 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_beam_kernel(const BeamParams
         }
       }
     }
-    BEAM_TICK(3)
     grid_sync(p.counter, bar_target);
-    BEAM_TICK(4)
   }
-#undef BEAM_TICK
 }
 
 struct BeamScratch {
-  size_t sync_off, sync_bytes, work_off, logits_off, nodes_off, depth_off, states_off, encp_off, a_off, w_off, total;
+  size_t sync_off, sync_bytes, work_off, logits_off, nodes_off, depth_off, states_off;
+  RnntEncScratch enc;
 };
 BeamScratch beam_scratch_layout(int E, int H, int J, int V1, int B, int T, const cfb_rnnt_beam_caps& c) {
   BeamScratch s;
@@ -608,13 +576,7 @@ BeamScratch beam_scratch_layout(int E, int H, int J, int V1, int B, int T, const
   off += align256(sizeof(int) * Bc * c.max_nodes);
   s.states_off = off;
   off += align256(sizeof(float) * Bc * c.max_states * (2 * static_cast<size_t>(H) + J));
-  s.encp_off = off;
-  off += align256(sizeof(float) * static_cast<size_t>(B) * T * J);
-  s.a_off = off;
-  off += align256(sizeof(bf16) * static_cast<size_t>(B) * T * 3 * E);
-  s.w_off = off;
-  off += align256(sizeof(bf16) * static_cast<size_t>(J) * 3 * E);
-  s.total = off;
+  s.enc = rnnt_enc_scratch(off, E, J, B, T);
   return s;
 }
 
@@ -633,7 +595,7 @@ size_t cfb_rnnt_beam_scratch_bytes(int enc_hidden, int pred_hidden, int joint_hi
                                    const cfb_rnnt_beam_caps* caps) {
   if (enc_hidden < 1 || pred_hidden < 1 || joint_hidden < 1 || num_classes_with_blank < 2 || B < 1 || T < 1 || !caps_valid(caps))
     return 0;
-  return beam_scratch_layout(enc_hidden, pred_hidden, joint_hidden, num_classes_with_blank, B, T, *caps).total;
+  return beam_scratch_layout(enc_hidden, pred_hidden, joint_hidden, num_classes_with_blank, B, T, *caps).enc.end;
 }
 
 int cfb_op_rnnt_beam(const cfb_rnnt_weights* w, const void* encoded, int x_dtype, const int32_t* encoded_len, int B, int T,
@@ -643,27 +605,18 @@ int cfb_op_rnnt_beam(const cfb_rnnt_weights* w, const void* encoded, int x_dtype
   if (!w || !encoded || !encoded_len || !n_hyps || !lengths || !tokens || !timesteps || !scores || !h_out || !c_out || !stats ||
       !flags || !scratch || !caps_valid(caps))
     return CFB_ERR_INVALID_ARG;
+  if (B < 1 || T < 1 || beam_size < 1 || !(temperature > 0.f) || !rnnt_weights_valid(*w, x_dtype)) return CFB_ERR_INVALID_ARG;
   const int E = w->enc_hidden, H = w->pred_hidden, J = w->joint_hidden, V1 = w->num_classes_with_blank;
-  if (B < 1 || T < 1 || E < 8 || (E % 8) || H < 4 || (H % 4) || J < 4 || (J % 4) || V1 < 2 || beam_size < 1 || !(temperature > 0.f))
-    return CFB_ERR_INVALID_ARG;
-  if (w->activation < 0 || w->activation > 2 || (x_dtype != CFB_F32 && x_dtype != CFB_BF16)) return CFB_ERR_INVALID_ARG;
-  if (!w->embed || !w->w_ih || !w->w_hh || !w->b_ih || !w->b_hh || !w->w_pred || !w->b_pred || !w->w_enc || !w->b_enc || !w->w_out ||
-      !w->b_out)
-    return CFB_ERR_INVALID_ARG;
   const int V = V1 - 1;
   const int beam = beam_size < V1 ? beam_size : V1, beam_k = beam < V ? beam : V;  // default_beam_search's widths
   if (beam_k > kMaxBeamK || caps->max_hyps > kMaxHyps) return CFB_ERR_UNSUPPORTED;
   const BeamScratch lay = beam_scratch_layout(E, H, J, V1, B, T, *caps);
-  if (scratch_bytes < lay.total || (reinterpret_cast<uintptr_t>(scratch) & 255)) return CFB_ERR_WORKSPACE;
+  if (scratch_bytes < lay.enc.end || (reinterpret_cast<uintptr_t>(scratch) & 255)) return CFB_ERR_WORKSPACE;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   uint8_t* ws = reinterpret_cast<uint8_t*>(scratch);
 
-  int dev = 0, sms = 0, max_smem = 0, coop = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return CFB_ERR_CUDA;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-  cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
-  if (!coop || sms < 1) return CFB_ERR_UNSUPPORTED;
+  int sms = 0, max_smem = 0;
+  if (int rc = rnnt_device_query(&sms, &max_smem)) return rc;
   cudaFuncAttributes fa;
   if (cudaFuncGetAttributes(&fa, rnnt_beam_kernel) != cudaSuccess) return CFB_ERR_CUDA;
   // shared memory: my weight rows + the owned utterance's two hypothesis lists + as much staging as is useful and fits
@@ -686,34 +639,9 @@ int cfb_op_rnnt_beam(const cfb_rnnt_weights* w, const void* encoded, int x_dtype
   if (cudaFuncSetAttribute(rnnt_beam_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)) != cudaSuccess)
     return CFB_ERR_CUDA;
 
-  // joint.enc over every frame: encp = encoded W_enc^T + b_enc on the tensor cores with split operands
-  const bool xf32 = x_dtype == CFB_F32;
-  const long long M = static_cast<long long>(B) * T;
-  bf16* a_split = reinterpret_cast<bf16*>(ws + lay.a_off);
-  bf16* w_split = reinterpret_cast<bf16*>(ws + lay.w_off);
-  float* encp = reinterpret_cast<float*>(ws + lay.encp_off);
-  {
-    const long long n = M * E;
-    const int blocks = static_cast<int>((n + 255) / 256 < 148 * 16 ? (n + 255) / 256 : 148 * 16);
-    split_bf16_kernel<<<blocks, 256, 0, st>>>(encoded, a_split, M, E, xf32 ? 0 : 2);
-    split_bf16_kernel<<<(J * E + 255) / 256, 256, 0, st>>>(w->w_enc, w_split, J, E, 1);
-    GemmDesc g;
-    g.A = a_split;
-    g.lda = xf32 ? 3 * E : 2 * E;
-    g.W = w_split;
-    g.ldw = 3 * E;
-    g.M = static_cast<int>(M);
-    g.N = J;
-    g.K = xf32 ? 3 * E : 2 * E;
-    g.epi = EPI_LINEAR;
-    g.out_bf16 = false;
-    g.ep.bias = w->b_enc;
-    g.ep.out = encp;
-    g.ep.ldo = J;
-    std::string err;
-    if (launch_gemm_tc(g, st, &err) != 0) return CFB_ERR_CUDA;
-  }
+  if (int rc = rnnt_joint_enc(*w, encoded, x_dtype, B, T, ws, lay.enc, st)) return rc;
 
+  const float* encp = reinterpret_cast<const float*>(ws + lay.enc.encp_off);
   const int X = caps->max_expansions;
   for (int b0 = 0; b0 < B; b0 += Bl) {
     const int Bc = B - b0 < Bl ? B - b0 : Bl;

@@ -1,8 +1,10 @@
 // Helpers shared by the transducer decode kernels (rnnt_greedy.cu, rnnt_beam.cu): the fence-free grid barrier of a
 // cooperative launch, small dot-product / activation helpers, the packed (value, index) arg-max key, the row partition
-// over CTAs and the split-operand conversion that feeds joint.enc to the tcgen05 GEMM.
+// over CTAs and the load of a CTA's rows into shared memory, and the host side both entry points share: weight
+// validation, the device query and the joint.enc projection (defined in rnnt_greedy.cu).
 #pragma once
 
+#include "../../include/cfb.h"
 #include "common.cuh"
 
 namespace cfb {
@@ -69,33 +71,63 @@ __device__ __forceinline__ void row_range(int n, int c, int g, int* lo, int* hi)
   *hi = static_cast<int>(static_cast<long long>(n) * (c + 1) / g);
 }
 
-// fp32 (rows, K) -> bf16 (rows, 3K) [hi | hi | lo]   (mode 0, activations)
-//                -> bf16 (rows, 3K) [hi | lo | hi]   (mode 1, weights)
-// bf16 input (mode 2): (rows, K) -> (rows, 2K) [x | x]
-__global__ void __launch_bounds__(256) split_bf16_kernel(const void* __restrict__ x, bf16* __restrict__ y, long long rows, int K,
-                                                         int mode) {
-  const long long n = rows * K;
-  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
-       i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const long long r = i / K;
-    const int k = static_cast<int>(i % K);
-    if (mode == 2) {
-      const bf16 v = reinterpret_cast<const bf16*>(x)[i];
-      y[r * 2 * K + k] = v;
-      y[r * 2 * K + K + k] = v;
-    } else {
-      const float v = reinterpret_cast<const float*>(x)[i];
-      const bf16 hi = __float2bfloat16_rn(v);
-      const bf16 lo = __float2bfloat16_rn(v - __bfloat162float(hi));
-      bf16* o = y + r * 3 * K;
-      o[k] = hi;
-      o[K + k] = mode == 0 ? hi : lo;
-      o[2 * K + k] = mode == 0 ? lo : hi;
-    }
+// The rows of the row partition a CTA keeps in shared memory for the whole decode (P: the kernel's parameters):
+//   s_wl [nu][4][2H]  the LSTM rows of hidden units [u_lo, u_lo + nu), gate-major per unit: [w_ih row | w_hh row],
+//   s_bl [nu][4]      their b_ih + b_hh,
+//   s_wp [np][H]      joint.pred rows [p_lo, p_lo + np),
+//   s_wj [nj][J]      output-layer rows [j_lo, j_lo + nj).
+template <class P>
+__device__ __forceinline__ void load_row_weights(const P& p, int u_lo, int nu, int p_lo, int np, int j_lo, int nj, float* s_wl,
+                                                 float* s_bl, float* s_wp, float* s_wj) {
+  const int H = p.H, J = p.J, tid = threadIdx.x, nt = blockDim.x;
+  for (int i = tid; i < nu * 4 * (2 * H / 4); i += nt) {
+    const int k4 = i % (2 * H / 4), r = i / (2 * H / 4), gate = r & 3, ul = r >> 2;
+    const int row = gate * H + u_lo + ul;
+    const float* src = k4 < H / 4 ? p.w_ih + static_cast<size_t>(row) * H + k4 * 4
+                                  : p.w_hh + static_cast<size_t>(row) * H + (k4 - H / 4) * 4;
+    reinterpret_cast<float4*>(s_wl)[i] = __ldg(reinterpret_cast<const float4*>(src));
   }
+  for (int i = tid; i < nu * 4; i += nt) {
+    const int row = (i & 3) * H + u_lo + (i >> 2);
+    s_bl[i] = p.b_ih[row] + p.b_hh[row];
+  }
+  for (int i = tid; i < np * (H / 4); i += nt)
+    reinterpret_cast<float4*>(s_wp)[i] = __ldg(reinterpret_cast<const float4*>(p.w_pred + static_cast<size_t>(p_lo) * H) + i);
+  for (int i = tid; i < nj * (J / 4); i += nt)
+    reinterpret_cast<float4*>(s_wj)[i] = __ldg(reinterpret_cast<const float4*>(p.w_out + static_cast<size_t>(j_lo) * J) + i);
 }
 
 inline size_t align256(size_t v) { return (v + 255) / 256 * 256; }
 
 }  // namespace
+
+// ---- host side of cfb_op_rnnt_greedy / cfb_op_rnnt_beam ------------------------------------------------------------------
+
+// The sizes, activation, pointers and encoder-output dtype both decoders accept.
+bool rnnt_weights_valid(const cfb_rnnt_weights& w, int x_dtype);
+
+// SMs and opt-in shared memory per block of the current device: CFB_ERR_CUDA, CFB_ERR_UNSUPPORTED without cooperative launch.
+int rnnt_device_query(int* sms, int* max_smem);
+
+// The joint.enc buffers at the end of both scratch layouts, from `off` on: encp (B*T, J) fp32 = joint.enc(encoded) and
+// the split operands of its GEMM, a (B*T, 3E) and w (J, 3E) bf16.
+struct RnntEncScratch {
+  size_t encp_off, a_off, w_off, end;
+};
+inline RnntEncScratch rnnt_enc_scratch(size_t off, int E, int J, int B, int T) {
+  RnntEncScratch s;
+  s.encp_off = off;
+  off += align256(sizeof(float) * static_cast<size_t>(B) * T * J);
+  s.a_off = off;
+  off += align256(sizeof(bf16) * static_cast<size_t>(B) * T * 3 * E);
+  s.w_off = off;
+  off += align256(sizeof(bf16) * static_cast<size_t>(J) * 3 * E);
+  s.end = off;
+  return s;
+}
+
+// Enqueues encp = encoded W_enc^T + b_enc over every frame into the scratch at `ws` (0 or CFB_ERR_CUDA).
+int rnnt_joint_enc(const cfb_rnnt_weights& w, const void* encoded, int x_dtype, int B, int T, uint8_t* ws, const RnntEncScratch& s,
+                   cudaStream_t st);
+
 }  // namespace cfb

@@ -44,7 +44,7 @@ struct RnntParams {
   float* hbuf;   // [2][B][H]
   float* predp;  // [B][J]
   unsigned long long* slots;  // [3][2][kMaxB]
-  unsigned int* counter;
+  unsigned int* counter;      // grid barrier
   // outputs
   int32_t *tokens, *timesteps, *n_tokens, *flags;
   float *scores, *h_out, *c_out;
@@ -152,12 +152,117 @@ __device__ int build_list(const int* flag, int B, int* list, int* s_tmp) {
   return total;
 }
 
+// Per-utterance control of a launch, replicated in every CTA and advanced identically from the one exchanged datum (the
+// combined arg-max keys in p.slots): frame, symbols emitted at it, last label, which half of hbuf / s_c holds the pending
+// prediction-network state, tokens emitted, length, score (CTA 0's copy is written out), active and emitted flags and
+// their ascending lists.  Both greedy kernels run exactly this decode rule.
+struct GreedyControl {
+  double score[kMaxB];
+  int t[kMaxB], sym[kMaxB], last[kMaxB], par[kMaxB], ntok[kMaxB], len[kMaxB];
+  int active[kMaxB], emit[kMaxB], alist[kMaxB], elist[kMaxB];
+  int tmp[kWarps];
+
+  // Every utterance starts at frame 0 with the SOS step pending (joint.pred of its first prediction-network output).
+  __device__ void init(const RnntParams& p) {
+    const int tid = threadIdx.x;
+    if (tid < kMaxB) {
+      const int n = tid < p.B ? min(max(p.lens[tid], 0), p.T) : 0;
+      len[tid] = n;
+      t[tid] = 0;
+      sym[tid] = 0;
+      last[tid] = p.V1 - 1;
+      par[tid] = 0;
+      ntok[tid] = 0;
+      score[tid] = 0.0;
+      active[tid] = n > 0;
+      emit[tid] = tid < p.B;
+    }
+    __syncthreads();
+  }
+
+  __device__ void build_lists(int B, int* n_emit, int* n_active) {
+    *n_emit = build_list(emit, B, elist, tmp);
+    *n_active = build_list(active, B, alist, tmp);
+  }
+
+  // Consumes the keys of lock-step iteration `it` (frame t and, only after a blank, the speculatively evaluated t + 1),
+  // appends the emitted token (CTA 0), clears the slots of iteration it + 2 (the three sets rotate: every CTA finished
+  // reading them in iteration it - 1) and rebuilds the lists.
+  __device__ void update(const RnntParams& p, unsigned int it, int* n_emit, int* n_active) {
+    const int tid = threadIdx.x, cta = blockIdx.x, blank = p.V1 - 1;
+    if (tid < kMaxB) {
+      int e = 0;
+      if (tid < p.B && active[tid]) {
+        int tt = t[tid], sy = sym[tid];
+        const int n_len = len[tid];
+        for (int f = 0; f < 2; ++f) {
+          float v;
+          int k;
+          unpack_key(__ldcg(&p.slots[((it % 3) * 2 + f) * kMaxB + tid]), &v, &k);
+          if (k == blank) {
+            ++tt;
+            sy = 0;
+            if (tt >= n_len) break;
+            continue;
+          }
+          e = 1;
+          const int n = ntok[tid];
+          if (cta == 0) {
+            if (n < p.max_tokens) {
+              p.tokens[static_cast<size_t>(tid) * p.max_tokens + n] = k;
+              p.timesteps[static_cast<size_t>(tid) * p.max_tokens + n] = tt;
+            } else {
+              atomicOr(p.flags, 1);
+            }
+            score[tid] += static_cast<double>(v);
+          }
+          ntok[tid] = n + 1;
+          last[tid] = k;
+          if (++sy >= (p.max_symbols > 0 ? p.max_symbols : kHardSymbolLimit)) {
+            if (p.max_symbols <= 0 && cta == 0) atomicOr(p.flags, 2);  // runaway emission: the reference would not return
+            ++tt;
+            sy = 0;
+          }
+          break;  // the prediction network must advance before the next joint evaluation
+        }
+        t[tid] = tt;
+        sym[tid] = sy;
+        active[tid] = tt < n_len;
+      }
+      emit[tid] = e;
+      if (cta == 0) {
+        p.slots[(((it + 2) % 3) * 2 + 0) * kMaxB + tid] = 0ull;
+        p.slots[(((it + 2) % 3) * 2 + 1) * kMaxB + tid] = 0ull;
+      }
+    }
+    __syncthreads();
+    build_lists(p.B, n_emit, n_active);
+  }
+
+  // Results: the committed state is the half the pending one does not occupy.  This CTA's cell states are those of units
+  // [u0, u0 + nu) in s_c [2][B][cstride].
+  __device__ void write_results(const RnntParams& p, const float* s_c, int cstride, int u0, int nu) {
+    const int tid = threadIdx.x, cta = blockIdx.x, B = p.B, H = p.H;
+    for (int i = tid; i < nu * B; i += kThreads) {
+      const int u = i % nu, b = i / nu;
+      p.c_out[static_cast<size_t>(b) * H + u0 + u] = s_c[((par[b] ^ 1) * B + b) * cstride + u];
+    }
+    for (int i = cta * kThreads + tid; i < B * H; i += gridDim.x * kThreads) {
+      const int b = i / H, u = i % H;
+      p.h_out[i] = __ldcg(p.hbuf + (static_cast<size_t>(par[b] ^ 1) * B + b) * H + u);
+    }
+    if (cta == 0 && tid < B) {
+      p.n_tokens[tid] = ntok[tid];
+      p.scores[tid] = static_cast<float>(score[tid]);
+    }
+  }
+};
+
 __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntParams p) {
   extern __shared__ __align__(16) float smem[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int G = gridDim.x, cta = blockIdx.x;
   const int H = p.H, J = p.J, V1 = p.V1, B = p.B, K2 = 2 * p.H;
-  const int blank = V1 - 1;
 
   int u_lo, u_hi, p_lo, p_hi, j_lo, j_hi;
   row_range(H, cta, G, &u_lo, &u_hi);
@@ -173,44 +278,11 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
   float* s_c = s_bl + p.umax * 4;                             // [2][B][umax] cell state of my units
   float4* s_stage = reinterpret_cast<float4*>(s_c + ((static_cast<size_t>(2) * B * p.umax + 3) / 4) * 4);  // p.stage_floats
   const int J4 = J / 4, H4 = H / 4, K24 = K2 / 4;
-  // utterances staged at a time: joint tasks take groups of 4, the LSTM / pred tasks pairs
-  const int tile_j = min(kMaxTile, p.stage_floats / J) & ~3, tile_l = min(kMaxTile, p.stage_floats / K2) & ~1,
-            tile_p = min(kMaxTile, p.stage_floats / H) & ~1;
   __shared__ unsigned long long s_best[2 * kMaxB];  // [frame 0 | frame 1][utterance]
-  __shared__ double s_score[kMaxB];
-  __shared__ int s_t[kMaxB], s_sym[kMaxB], s_last[kMaxB], s_par[kMaxB], s_ntok[kMaxB], s_len[kMaxB];
-  __shared__ int s_active[kMaxB], s_emit[kMaxB], s_alist[kMaxB], s_elist[kMaxB];
-  __shared__ int s_tmp[kWarps];
+  __shared__ GreedyControl ctl;
 
-  // ---- load my weight rows (once) ----------------------------------------------------------------------------------
-  for (int i = tid; i < nu * 4 * (K2 / 4); i += kThreads) {
-    const int k4 = i % (K2 / 4), r = i / (K2 / 4), gate = r & 3, ul = r >> 2;
-    const int row = gate * H + u_lo + ul;
-    const float* src = k4 < H / 4 ? p.w_ih + static_cast<size_t>(row) * H + k4 * 4
-                                  : p.w_hh + static_cast<size_t>(row) * H + (k4 - H / 4) * 4;
-    reinterpret_cast<float4*>(s_wl)[i] = __ldg(reinterpret_cast<const float4*>(src));
-  }
-  for (int i = tid; i < nu * 4; i += kThreads) {
-    const int row = (i & 3) * H + u_lo + (i >> 2);
-    s_bl[i] = p.b_ih[row] + p.b_hh[row];
-  }
-  for (int i = tid; i < np * (H / 4); i += kThreads)
-    reinterpret_cast<float4*>(s_wp)[i] = __ldg(reinterpret_cast<const float4*>(p.w_pred + static_cast<size_t>(p_lo) * H) + i);
-  for (int i = tid; i < nj * (J / 4); i += kThreads)
-    reinterpret_cast<float4*>(s_wj)[i] = __ldg(reinterpret_cast<const float4*>(p.w_out + static_cast<size_t>(j_lo) * J) + i);
-  if (tid < kMaxB) {
-    const int len = tid < B ? min(max(p.lens[tid], 0), p.T) : 0;
-    s_len[tid] = len;
-    s_t[tid] = 0;
-    s_sym[tid] = 0;
-    s_last[tid] = blank;
-    s_par[tid] = 0;
-    s_ntok[tid] = 0;
-    s_score[tid] = 0.0;
-    s_active[tid] = len > 0;
-    s_emit[tid] = tid < B;  // the SOS step: every utterance needs joint.pred of its first prediction-network output
-  }
-  __syncthreads();
+  load_row_weights(p, u_lo, nu, p_lo, np, j_lo, nj, s_wl, s_bl, s_wp, s_wj);
+  ctl.init(p);
 
   // ---- SOS: pending = LSTM(x = 0, h = 0, c = 0) = f(bias) for every utterance; committed state = 0 (hbuf[1] is zeroed) --
   for (int i = tid; i < nu * B; i += kThreads) {
@@ -223,31 +295,22 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
     p.hbuf[(static_cast<size_t>(0) * B + b) * H + u_lo + ul] = h1;
   }
   unsigned int bar_target = 0;
-  int n_emit = build_list(s_emit, B, s_elist, s_tmp);
-  int n_active = build_list(s_active, B, s_alist, s_tmp);
+  int n_emit, n_active;
+  ctl.build_lists(B, &n_emit, &n_active);
   grid_sync(p.counter, bar_target);
 
   bool first = true;
-  // phase clocks of CTA 0 (cycles; bytes 64..191 of the sync header): joint, barrier, control, lstm, barrier, pred, barrier
-  unsigned long long* timers = reinterpret_cast<unsigned long long*>(p.counter + 16);
-  long long tk = clock64();
-#define RNNT_TICK(slot)                                   \
-  if (cta == 0 && tid == 0) {                             \
-    const long long now = clock64();                      \
-    timers[slot] += static_cast<unsigned long long>(now - tk); \
-    tk = now;                                             \
-  }
   for (unsigned int it = 0;; ++it) {
     if (!first) {
       // ---- joint: logits of my rows for every active utterance at its frame, arg-max ----------------------------------
-      RNNT_TICK(7)
-      if (cta == 0 && tid == 0) timers[10] += 1;  // lock-step iterations
       // Two frames per utterance are evaluated with the same prediction-network output: if the first is blank (the common
       // case) the second is already the answer for the next frame, so a lock-step iteration consumes up to two frames.
       if (tid < 2 * kMaxB) s_best[tid] = 0ull;
       __syncthreads();
       const int nchunks = (nj + 7) >> 3;
-      const int tile_s = tile_j >> 1;  // utterances per tile (two staged vectors each)
+      // utterances staged at a time (the tile sizes are recomputed in each phase rather than kept live across the loop):
+      // the joint tasks take groups of 4 staged vectors, two per utterance; the LSTM / pred tasks take pairs
+      const int tile_s = (min(kMaxTile, p.stage_floats / J) & ~3) >> 1;
       for (int s0 = 0; nj > 0 && s0 < n_active; s0 += tile_s) {
         const int ns = min(tile_s, n_active - s0), total = ns * J4;
         // stage z_f = act(enc_proj[b, t_b + f] + pred_proj[b]), f = 0, 1: all loads of a round are issued before the first use
@@ -257,7 +320,7 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
           for (int u = 0; u < kJointRound; ++u) {
             const int idx = base + u * kThreads + tid;
             if (idx < total) {
-              const int bb = s_alist[s0 + idx / J4], k4 = idx % J4, t0 = s_t[bb], t1 = min(t0 + 1, s_len[bb] - 1);
+              const int bb = ctl.alist[s0 + idx / J4], k4 = idx % J4, t0 = ctl.t[bb], t1 = min(t0 + 1, ctl.len[bb] - 1);
               e0[u] = __ldg(reinterpret_cast<const float4*>(p.encp + (static_cast<size_t>(bb) * p.T + t0) * J) + k4);
               e1[u] = __ldg(reinterpret_cast<const float4*>(p.encp + (static_cast<size_t>(bb) * p.T + t1) * J) + k4);
               q[u] = ldcg4(p.predp + static_cast<size_t>(bb) * J + k4 * 4);
@@ -279,7 +342,6 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
           }
         }
         __syncthreads();
-        RNNT_TICK(8)
         const int nv = 2 * ns, ngroups = (nv + 3) >> 2;  // staged vector v = 2 * utterance + frame
         for (int task = warp; task < ngroups * nchunks; task += kWarps) {
           const int grp = task % ngroups, ch = task / ngroups, r0 = ch * 8;
@@ -298,73 +360,23 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
             const unsigned long long other = __shfl_xor_sync(0xffffffffu, key, o);
             key = other > key ? other : key;
           }
-          if (lane < 4 && v < nv) atomicMax(&s_best[(v & 1) * kMaxB + s_alist[s0 + (v >> 1)]], key);
+          if (lane < 4 && v < nv) atomicMax(&s_best[(v & 1) * kMaxB + ctl.alist[s0 + (v >> 1)]], key);
         }
         __syncthreads();
-        RNNT_TICK(9)
       }
       __syncthreads();
       if (nj > 0 && tid < 2 * n_active) {
-        const int b = s_alist[tid >> 1], f = tid & 1;
+        const int b = ctl.alist[tid >> 1], f = tid & 1;
         atomicMax(&p.slots[((it % 3) * 2 + f) * kMaxB + b], s_best[f * kMaxB + b]);
       }
-      RNNT_TICK(0)
       grid_sync(p.counter, bar_target);
-      RNNT_TICK(1)
 
       // ---- control update (replicated in every CTA) ---------------------------------------------------------------------
-      if (tid < kMaxB) {
-        int emit = 0;
-        if (tid < B && s_active[tid]) {
-          int t = s_t[tid], sym = s_sym[tid];
-          const int len = s_len[tid];
-          for (int f = 0; f < 2; ++f) {  // frame t, then (only after a blank) the speculatively evaluated frame t + 1
-            float v;
-            int k;
-            unpack_key(__ldcg(&p.slots[((it % 3) * 2 + f) * kMaxB + tid]), &v, &k);
-            if (k == blank) {
-              ++t;
-              sym = 0;
-              if (t >= len) break;
-              continue;
-            }
-            emit = 1;
-            const int n = s_ntok[tid];
-            if (cta == 0) {
-              if (n < p.max_tokens) {
-                p.tokens[static_cast<size_t>(tid) * p.max_tokens + n] = k;
-                p.timesteps[static_cast<size_t>(tid) * p.max_tokens + n] = t;
-              } else {
-                atomicOr(p.flags, 1);
-              }
-              s_score[tid] += static_cast<double>(v);
-            }
-            s_ntok[tid] = n + 1;
-            s_last[tid] = k;
-            if (++sym >= (p.max_symbols > 0 ? p.max_symbols : kHardSymbolLimit)) {
-              if (p.max_symbols <= 0 && cta == 0) atomicOr(p.flags, 2);  // runaway emission: the reference would not return
-              ++t;
-              sym = 0;
-            }
-            break;  // the prediction network must advance before the next joint evaluation
-          }
-          s_t[tid] = t;
-          s_sym[tid] = sym;
-          s_active[tid] = t < len;
-        }
-        s_emit[tid] = emit;
-        if (cta == 0) {
-          p.slots[(((it + 2) % 3) * 2 + 0) * kMaxB + tid] = 0ull;
-          p.slots[(((it + 2) % 3) * 2 + 1) * kMaxB + tid] = 0ull;
-        }
-      }
-      __syncthreads();
-      n_emit = build_list(s_emit, B, s_elist, s_tmp);
-      n_active = build_list(s_active, B, s_alist, s_tmp);
-      RNNT_TICK(2)
+      ctl.update(p, it, &n_emit, &n_active);
 
       // ---- LSTM cell for the utterances that emitted: commit the pending state, compute the next one -----------------------
       if (n_emit > 0) {
+        const int tile_l = min(kMaxTile, p.stage_floats / K2) & ~1;
         for (int s0 = 0; nu > 0 && s0 < n_emit; s0 += tile_l) {
           const int ns = min(tile_l, n_emit - s0), total = ns * K24;
           // stage [embed(last label) | h] of the utterances of this tile
@@ -374,9 +386,9 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
             for (int u = 0; u < kStageRound; ++u) {
               const int idx = base + u * kThreads + tid;
               if (idx < total) {
-                const int bb = s_elist[s0 + idx / K24], k4 = idx % K24;
-                v[u] = k4 < H4 ? __ldg(reinterpret_cast<const float4*>(p.embed + static_cast<size_t>(s_last[bb]) * H) + k4)
-                               : ldcg4(p.hbuf + (static_cast<size_t>(s_par[bb]) * B + bb) * H + (k4 - H4) * 4);
+                const int bb = ctl.elist[s0 + idx / K24], k4 = idx % K24;
+                v[u] = k4 < H4 ? __ldg(reinterpret_cast<const float4*>(p.embed + static_cast<size_t>(ctl.last[bb]) * H) + k4)
+                               : ldcg4(p.hbuf + (static_cast<size_t>(ctl.par[bb]) * B + bb) * H + (k4 - H4) * 4);
               }
             }
 #pragma unroll
@@ -386,7 +398,6 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
             }
           }
           __syncthreads();
-          RNNT_TICK(11)
           const int ngr = (ns + 3) >> 2;  // tasks = (hidden unit: its 4 gate rows) x (group of 4 utterances)
           for (int task = warp; task < ngr * nu; task += kWarps) {
             const int grp = task % ngr, ul = task / ngr;
@@ -402,8 +413,8 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
             const float gi = __shfl_sync(0xffffffffu, total, u) + bl[0], gf = __shfl_sync(0xffffffffu, total, 4 + u) + bl[1];
             const float gg = __shfl_sync(0xffffffffu, total, 8 + u) + bl[2], go = __shfl_sync(0xffffffffu, total, 12 + u) + bl[3];
             if (lane < 4 && 4 * grp + u < ns) {
-              const int b = s_elist[s0 + 4 * grp + u];
-              const int par = s_par[b];
+              const int b = ctl.elist[s0 + 4 * grp + u];
+              const int par = ctl.par[b];
               const float c_old = s_c[(par * B + b) * p.umax + ul];
               const float c_new = sigmoidf_(gf) * c_old + sigmoidf_(gi) * tanhf(gg);
               const float h_new = sigmoidf_(go) * tanhf(c_new);
@@ -414,10 +425,8 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
           __syncthreads();
         }
         __syncthreads();
-        if (tid < n_emit) s_par[s_elist[tid]] ^= 1;
-        RNNT_TICK(3)
+        if (tid < n_emit) ctl.par[ctl.elist[tid]] ^= 1;
         grid_sync(p.counter, bar_target);
-        RNNT_TICK(4)
       }
       if (n_active == 0) break;
     }
@@ -426,6 +435,7 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
     // ---- joint.pred of the new prediction-network outputs -------------------------------------------------------------------
     if (n_emit > 0) {
       const int nchunks = (np + 3) >> 2;
+      const int tile_p = min(kMaxTile, p.stage_floats / H) & ~1;
       for (int s0 = 0; np > 0 && s0 < n_emit; s0 += tile_p) {
         const int ns = min(tile_p, n_emit - s0), total = ns * H4;
         for (int base = 0; base < total; base += kThreads * kStageRound) {
@@ -434,8 +444,8 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
           for (int u = 0; u < kStageRound; ++u) {
             const int idx = base + u * kThreads + tid;
             if (idx < total) {
-              const int bb = s_elist[s0 + idx / H4];
-              v[u] = ldcg4(p.hbuf + (static_cast<size_t>(s_par[bb]) * B + bb) * H + (idx % H4) * 4);
+              const int bb = ctl.elist[s0 + idx / H4];
+              v[u] = ldcg4(p.hbuf + (static_cast<size_t>(ctl.par[bb]) * B + bb) * H + (idx % H4) * 4);
             }
           }
 #pragma unroll
@@ -445,14 +455,13 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
           }
         }
         __syncthreads();
-        RNNT_TICK(12)
         const int npe = (ns + 1) >> 1;
         for (int task = warp; task < npe * nchunks; task += kWarps) {
           const int pr = task % npe, ch = task / npe, r0 = ch * 4;
           const int i0 = 2 * pr, i1 = (2 * pr + 1 < ns) ? 2 * pr + 1 : i0;
           float acc[4][2] = {};
           tile_dot(reinterpret_cast<const float4*>(s_wp) + r0 * H4, H4, np - r0, s_stage + i0 * H4, s_stage + i1 * H4, H4, lane, acc);
-          const int b0 = s_elist[s0 + i0], b1 = s_elist[s0 + i1];
+          const int b0 = ctl.elist[s0 + i0], b1 = ctl.elist[s0 + i1];
 #pragma unroll
           for (int r = 0; r < 4; ++r) {
             if (r0 + r < np) {
@@ -465,26 +474,12 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_kernel(const RnntPara
         }
         __syncthreads();
       }
-      RNNT_TICK(5)
       grid_sync(p.counter, bar_target);
-      RNNT_TICK(6)
     }
     if (n_active == 0) break;
   }
 
-  // ---- results: committed state = the buffer the pending one does not occupy ------------------------------------------------
-  for (int i = tid; i < nu * B; i += kThreads) {
-    const int ul = i % nu, b = i / nu;
-    p.c_out[static_cast<size_t>(b) * H + u_lo + ul] = s_c[((s_par[b] ^ 1) * B + b) * p.umax + ul];
-  }
-  for (int i = cta * kThreads + tid; i < B * H; i += G * kThreads) {
-    const int b = i / H, u = i % H;
-    p.h_out[i] = __ldcg(p.hbuf + (static_cast<size_t>(s_par[b] ^ 1) * B + b) * H + u);
-  }
-  if (cta == 0 && tid < B) {
-    p.n_tokens[tid] = s_ntok[tid];
-    p.scores[tid] = static_cast<float>(s_score[tid]);
-  }
+  ctl.write_results(p, s_c, p.umax, u_lo, nu);
 }
 
 // ======================================================================================================================
@@ -529,7 +524,6 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int G = gridDim.x, cta = blockIdx.x, NQ = G / kC, q = cta / kC, r = cta % kC;
   const int H = p.H, J = p.J, V1 = p.V1, B = p.B;
-  const int blank = V1 - 1;
   const int Lq = H / 2, Hq = H / 4, Jq = J / 4;          // K slices (floats): LSTM [x | h], joint.pred, output layer
   const int Lq4 = Lq / 4, Hq4 = Hq / 4, Jq4 = Jq / 4;
 
@@ -557,10 +551,7 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
   const int tile_s = min(kTileV / 2, p.stage_floats / (2 * Jq)) & ~1;   // utterances per joint tile (two vectors each)
   const int tile_l = min(kTileL, p.stage_floats / Lq) & ~3, tile_p = min(kTileP, p.stage_floats / Hq) & ~3;
   __shared__ unsigned long long s_best[2 * kMaxB];
-  __shared__ double s_score[kMaxB];
-  __shared__ int s_t[kMaxB], s_sym[kMaxB], s_last[kMaxB], s_par[kMaxB], s_ntok[kMaxB], s_len[kMaxB];
-  __shared__ int s_active[kMaxB], s_emit[kMaxB], s_alist[kMaxB], s_elist[kMaxB];
-  __shared__ int s_tmp[kWarps];
+  __shared__ GreedyControl ctl;
 
   // ---- my K-quarter of the cluster's weight rows (once) --------------------------------------------------------------------
   for (int i = tid; i < nuq * 4 * Lq4; i += kThreads) {
@@ -580,19 +571,7 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
     const int row = (i & 3) * H + uq_lo + mu_lo + (i >> 2);
     s_bl[i] = p.b_ih[row] + p.b_hh[row];
   }
-  if (tid < kMaxB) {
-    const int len = tid < B ? min(max(p.lens[tid], 0), p.T) : 0;
-    s_len[tid] = len;
-    s_t[tid] = 0;
-    s_sym[tid] = 0;
-    s_last[tid] = blank;
-    s_par[tid] = 0;
-    s_ntok[tid] = 0;
-    s_score[tid] = 0.0;
-    s_active[tid] = len > 0;
-    s_emit[tid] = tid < B;
-  }
-  __syncthreads();
+  ctl.init(p);
   // SOS: pending = LSTM(0; 0, 0) = f(bias) for the units this rank finalises; committed state = 0 (hbuf[1] is zeroed)
   for (int i = tid; i < nmu * B; i += kThreads) {
     const int m = i % nmu, b = i / nmu;
@@ -605,18 +584,14 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
   }
   unsigned int bar_target = 0;
   int jbuf = 0, lbuf = 0, pbuf = 0;
-  int n_emit = build_list(s_emit, B, s_elist, s_tmp);
-  int n_active = build_list(s_active, B, s_alist, s_tmp);
+  int n_emit, n_active;
+  ctl.build_lists(B, &n_emit, &n_active);
   cluster_sync_all();  // every CTA of the cluster is running before the first remote shared-memory store
   grid_sync(p.counter, bar_target);
 
   bool first = true;
-  unsigned long long* timers = reinterpret_cast<unsigned long long*>(p.counter + 16);
-  long long tk = clock64();
   for (unsigned int it = 0;; ++it) {
     if (!first) {
-      RNNT_TICK(7)
-      if (cta == 0 && tid == 0) timers[10] += 1;
       // ---- joint at frames t and t + 1 of every active utterance ----------------------------------------------------------------
       if (tid < 2 * kMaxB) s_best[tid] = 0ull;
       __syncthreads();
@@ -628,7 +603,7 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
           for (int u = 0; u < kJointRound; ++u) {
             const int idx = base + u * kThreads + tid;
             if (idx < total) {
-              const int bb = s_alist[s0 + idx / Jq4], k4 = idx % Jq4, t0 = s_t[bb], t1 = min(t0 + 1, s_len[bb] - 1);
+              const int bb = ctl.alist[s0 + idx / Jq4], k4 = idx % Jq4, t0 = ctl.t[bb], t1 = min(t0 + 1, ctl.len[bb] - 1);
               e0[u] = __ldg(reinterpret_cast<const float4*>(p.encp + (static_cast<size_t>(bb) * p.T + t0) * J + r * Jq) + k4);
               e1[u] = __ldg(reinterpret_cast<const float4*>(p.encp + (static_cast<size_t>(bb) * p.T + t1) * J + r * Jq) + k4);
               qq[u] = ldcg4(p.predp + static_cast<size_t>(bb) * J + r * Jq + k4 * 4);
@@ -650,7 +625,6 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
           }
         }
         __syncthreads();
-        RNNT_TICK(8)
         const int nv = 2 * ns, ngroups = (nv + 3) >> 2;
         float* pj = s_pj + jbuf * (kC * 8 * kTileV);
         for (int task = warp; task < ngroups * nchunks; task += kWarps) {
@@ -671,71 +645,20 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
             const float* src = pj + row * kTileV + v;
             const float sum = ((src[0] + src[8 * kTileV]) + src[2 * 8 * kTileV]) + src[3 * 8 * kTileV];
             const int out_row = jq_lo + r * 8 + row;
-            atomicMax(&s_best[(v & 1) * kMaxB + s_alist[s0 + (v >> 1)]], pack_key(sum + __ldg(p.b_out + out_row), out_row));
+            atomicMax(&s_best[(v & 1) * kMaxB + ctl.alist[s0 + (v >> 1)]], pack_key(sum + __ldg(p.b_out + out_row), out_row));
           }
         }
         jbuf ^= 1;
         __syncthreads();
-        RNNT_TICK(9)
       }
       if (r < nchunks && tid < 2 * n_active) {
-        const int b = s_alist[tid >> 1], f = tid & 1;
+        const int b = ctl.alist[tid >> 1], f = tid & 1;
         atomicMax(&p.slots[((it % 3) * 2 + f) * kMaxB + b], s_best[f * kMaxB + b]);
       }
-      RNNT_TICK(0)
       grid_sync(p.counter, bar_target);
-      RNNT_TICK(1)
 
-      // ---- control update (replicated in every CTA) ---------------------------------------------------------------------------
-      if (tid < kMaxB) {
-        int emit = 0;
-        if (tid < B && s_active[tid]) {
-          int t = s_t[tid], sym = s_sym[tid];
-          const int len = s_len[tid];
-          for (int f = 0; f < 2; ++f) {
-            float v;
-            int k;
-            unpack_key(__ldcg(&p.slots[((it % 3) * 2 + f) * kMaxB + tid]), &v, &k);
-            if (k == blank) {
-              ++t;
-              sym = 0;
-              if (t >= len) break;
-              continue;
-            }
-            emit = 1;
-            const int n = s_ntok[tid];
-            if (cta == 0) {
-              if (n < p.max_tokens) {
-                p.tokens[static_cast<size_t>(tid) * p.max_tokens + n] = k;
-                p.timesteps[static_cast<size_t>(tid) * p.max_tokens + n] = t;
-              } else {
-                atomicOr(p.flags, 1);
-              }
-              s_score[tid] += static_cast<double>(v);
-            }
-            s_ntok[tid] = n + 1;
-            s_last[tid] = k;
-            if (++sym >= (p.max_symbols > 0 ? p.max_symbols : kHardSymbolLimit)) {
-              if (p.max_symbols <= 0 && cta == 0) atomicOr(p.flags, 2);
-              ++t;
-              sym = 0;
-            }
-            break;
-          }
-          s_t[tid] = t;
-          s_sym[tid] = sym;
-          s_active[tid] = t < len;
-        }
-        s_emit[tid] = emit;
-        if (cta == 0) {
-          p.slots[(((it + 2) % 3) * 2 + 0) * kMaxB + tid] = 0ull;
-          p.slots[(((it + 2) % 3) * 2 + 1) * kMaxB + tid] = 0ull;
-        }
-      }
-      __syncthreads();
-      n_emit = build_list(s_emit, B, s_elist, s_tmp);
-      n_active = build_list(s_active, B, s_alist, s_tmp);
-      RNNT_TICK(2)
+      // ---- control update (replicated in every CTA) ---------------------------------------------------------------------
+      ctl.update(p, it, &n_emit, &n_active);
 
       // ---- LSTM cell for the utterances that emitted ---------------------------------------------------------------------------
       if (n_emit > 0) {
@@ -747,9 +670,9 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
             for (int u = 0; u < kStageRound; ++u) {
               const int idx = base + u * kThreads + tid;
               if (idx < total) {
-                const int bb = s_elist[s0 + idx / Lq4], k4 = idx % Lq4;
-                v[u] = r < 2 ? __ldg(reinterpret_cast<const float4*>(p.embed + static_cast<size_t>(s_last[bb]) * H + r * Lq) + k4)
-                             : ldcg4(p.hbuf + (static_cast<size_t>(s_par[bb]) * B + bb) * H + (r - 2) * Lq + k4 * 4);
+                const int bb = ctl.elist[s0 + idx / Lq4], k4 = idx % Lq4;
+                v[u] = r < 2 ? __ldg(reinterpret_cast<const float4*>(p.embed + static_cast<size_t>(ctl.last[bb]) * H + r * Lq) + k4)
+                             : ldcg4(p.hbuf + (static_cast<size_t>(ctl.par[bb]) * B + bb) * H + (r - 2) * Lq + k4 * 4);
               }
             }
 #pragma unroll
@@ -785,8 +708,8 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
                 const int st = mumax * 4 * kTileL;
                 g4[gate] = (((src[0] + src[st]) + src[2 * st]) + src[3 * st]) + s_bl[m * 4 + gate];
               }
-              const int b = s_elist[s0 + sidx];
-              const int par = s_par[b];
+              const int b = ctl.elist[s0 + sidx];
+              const int par = ctl.par[b];
               const float c_old = s_c[(par * B + b) * mumax + m];
               const float c_new = sigmoidf_(g4[1]) * c_old + sigmoidf_(g4[0]) * tanhf(g4[2]);
               const float h_new = sigmoidf_(g4[3]) * tanhf(c_new);
@@ -797,10 +720,8 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
           lbuf ^= 1;
           __syncthreads();
         }
-        if (tid < n_emit) s_par[s_elist[tid]] ^= 1;
-        RNNT_TICK(3)
+        if (tid < n_emit) ctl.par[ctl.elist[tid]] ^= 1;
         grid_sync(p.counter, bar_target);
-        RNNT_TICK(4)
       }
       if (n_active == 0) break;
     }
@@ -817,8 +738,8 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
           for (int u = 0; u < kStageRound; ++u) {
             const int idx = base + u * kThreads + tid;
             if (idx < total) {
-              const int bb = s_elist[s0 + idx / Hq4];
-              v[u] = ldcg4(p.hbuf + (static_cast<size_t>(s_par[bb]) * B + bb) * H + r * Hq + (idx % Hq4) * 4);
+              const int bb = ctl.elist[s0 + idx / Hq4];
+              v[u] = ldcg4(p.hbuf + (static_cast<size_t>(ctl.par[bb]) * B + bb) * H + r * Hq + (idx % Hq4) * 4);
             }
           }
 #pragma unroll
@@ -851,57 +772,39 @@ __global__ void __launch_bounds__(kThreads, 1) rnnt_greedy_c4_kernel(const RnntP
           if (sidx < ns) {
             const float* src = pp + m * kTileP + sidx;
             const int st = mpmax * kTileP, row = pq_lo + mp_lo + m;
-            p.predp[static_cast<size_t>(s_elist[s0 + sidx]) * J + row] =
+            p.predp[static_cast<size_t>(ctl.elist[s0 + sidx]) * J + row] =
                 (((src[0] + src[st]) + src[2 * st]) + src[3 * st]) + __ldg(p.b_pred + row);
           }
         }
         pbuf ^= 1;
         __syncthreads();
       }
-      RNNT_TICK(5)
       grid_sync(p.counter, bar_target);
-      RNNT_TICK(6)
     }
     if (n_active == 0) break;
   }
 
-  for (int i = tid; i < nmu * B; i += kThreads) {
-    const int m = i % nmu, b = i / nmu;
-    p.c_out[static_cast<size_t>(b) * H + uq_lo + mu_lo + m] = s_c[((s_par[b] ^ 1) * B + b) * mumax + m];
-  }
-  for (int i = cta * kThreads + tid; i < B * H; i += G * kThreads) {
-    const int b = i / H, u = i % H;
-    p.h_out[i] = __ldcg(p.hbuf + (static_cast<size_t>(s_par[b] ^ 1) * B + b) * H + u);
-  }
-  if (cta == 0 && tid < B) {
-    p.n_tokens[tid] = s_ntok[tid];
-    p.scores[tid] = static_cast<float>(s_score[tid]);
-  }
+  ctl.write_results(p, s_c, mumax, uq_lo + mu_lo, nmu);
   cluster_sync_all();  // no CTA of the cluster exits while a sibling could still address its shared memory
 }
 
 struct RnntScratch {
-  size_t sync_off, sync_bytes, hbuf_off, hbuf_bytes, predp_off, encp_off, a_off, w_off, total;
+  size_t sync_off, sync_bytes, hbuf_off, hbuf_bytes, predp_off;
+  RnntEncScratch enc;
 };
 RnntScratch rnnt_scratch_layout(int E, int H, int J, int B, int T) {
   RnntScratch s;
   const int Bc = B < kMaxB ? B : kMaxB;
   size_t off = 0;
   s.sync_off = off;
-  s.sync_bytes = align256(512 + sizeof(unsigned long long) * 3 * 2 * kMaxB);
+  s.sync_bytes = align256(512 + sizeof(unsigned long long) * 3 * 2 * kMaxB);  // barrier counter | slots from byte 512 on
   off += s.sync_bytes;
   s.hbuf_off = off;
   s.hbuf_bytes = align256(sizeof(float) * 2 * Bc * H);
   off += s.hbuf_bytes;
   s.predp_off = off;
   off += align256(sizeof(float) * Bc * J);
-  s.encp_off = off;
-  off += align256(sizeof(float) * static_cast<size_t>(B) * T * J);
-  s.a_off = off;
-  off += align256(sizeof(bf16) * static_cast<size_t>(B) * T * 3 * E);
-  s.w_off = off;
-  off += align256(sizeof(bf16) * static_cast<size_t>(J) * 3 * E);
-  s.total = off;
+  s.enc = rnnt_enc_scratch(off, E, J, B, T);
   return s;
 }
 
@@ -926,6 +829,25 @@ size_t rnnt_c4_fixed_bytes(int H, int J, int V1, int NQ, int B, int* umax, int* 
                           (static_cast<size_t>(2) * kC * mpmax * kTileP + 3) / 4 * 4);
 }
 
+// Launch configuration of rnnt_greedy_c4_kernel: clusters of kC CTAs and, for the launch itself (not the occupancy
+// query), the cooperative attribute.
+cudaLaunchConfig_t c4_launch_config(int grid, size_t smem, cudaStream_t st, bool cooperative, cudaLaunchAttribute (&attr)[2]) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid);
+  cfg.blockDim = dim3(kThreads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = kC;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  attr[1].id = cudaLaunchAttributeCooperative;
+  attr[1].val.cooperative = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = cooperative ? 2 : 1;
+  return cfg;
+}
+
 // Plans the cluster variant: number of co-resident clusters, shared-memory split.  Returns false when it is not asked for
 // or the device / the sizes rule it out (the row-partitioned kernel is used then).
 bool g_c4_unusable = false;  // set when a cooperative cluster launch was refused once (the other kernel serves from then on)
@@ -944,17 +866,8 @@ bool rnnt_c4_plan(int H, int J, int V1, int Bmax, int max_smem, RnntParams* p, i
   const size_t budget = static_cast<size_t>(max_smem) - fa.sharedSizeBytes;
   if (cudaFuncSetAttribute(rnnt_greedy_c4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(budget)) != cudaSuccess)
     return false;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(kC * 64);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = budget;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = kC;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
+  cudaLaunchAttribute attr[2];
+  const cudaLaunchConfig_t cfg = c4_launch_config(kC * 64, budget, 0, false, attr);
   int nq = 0;
   if (cudaOccupancyMaxActiveClusters(&nq, rnnt_greedy_c4_kernel, &cfg) != cudaSuccess || nq < 8) {
     cudaGetLastError();
@@ -975,7 +888,79 @@ bool rnnt_c4_plan(int H, int J, int V1, int Bmax, int max_smem, RnntParams* p, i
   return true;
 }
 
+// fp32 (rows, K) -> bf16 (rows, 3K) [hi | hi | lo]   (mode 0, activations)
+//                -> bf16 (rows, 3K) [hi | lo | hi]   (mode 1, weights)
+// bf16 input (mode 2): (rows, K) -> (rows, 2K) [x | x]
+__global__ void __launch_bounds__(256) split_bf16_kernel(const void* __restrict__ x, bf16* __restrict__ y, long long rows, int K,
+                                                         int mode) {
+  const long long n = rows * K;
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long r = i / K;
+    const int k = static_cast<int>(i % K);
+    if (mode == 2) {
+      const bf16 v = reinterpret_cast<const bf16*>(x)[i];
+      y[r * 2 * K + k] = v;
+      y[r * 2 * K + K + k] = v;
+    } else {
+      const float v = reinterpret_cast<const float*>(x)[i];
+      const bf16 hi = __float2bfloat16_rn(v);
+      const bf16 lo = __float2bfloat16_rn(v - __bfloat162float(hi));
+      bf16* o = y + r * 3 * K;
+      o[k] = hi;
+      o[K + k] = mode == 0 ? hi : lo;
+      o[2 * K + k] = mode == 0 ? lo : hi;
+    }
+  }
+}
+
 }  // namespace
+
+bool rnnt_weights_valid(const cfb_rnnt_weights& w, int x_dtype) {
+  const int E = w.enc_hidden, H = w.pred_hidden, J = w.joint_hidden;
+  return E >= 8 && E % 8 == 0 && H >= 4 && H % 4 == 0 && J >= 4 && J % 4 == 0 && w.num_classes_with_blank >= 2 &&
+         w.activation >= 0 && w.activation <= 2 && (x_dtype == CFB_F32 || x_dtype == CFB_BF16) && w.embed && w.w_ih && w.w_hh &&
+         w.b_ih && w.b_hh && w.w_pred && w.b_pred && w.w_enc && w.b_enc && w.w_out && w.b_out;
+}
+
+int rnnt_device_query(int* sms, int* max_smem) {
+  int dev = 0, coop = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) return CFB_ERR_CUDA;
+  cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev);
+  cudaDeviceGetAttribute(max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+  cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
+  return !coop || *sms < 1 ? CFB_ERR_UNSUPPORTED : CFB_OK;
+}
+
+// On the tensor cores with split operands: A' = [hi | hi | lo] (fp32 input) or [x | x] (bf16), W' = [hi | lo | hi].
+int rnnt_joint_enc(const cfb_rnnt_weights& w, const void* encoded, int x_dtype, int B, int T, uint8_t* ws, const RnntEncScratch& s,
+                   cudaStream_t st) {
+  const int E = w.enc_hidden, J = w.joint_hidden;
+  const bool xf32 = x_dtype == CFB_F32;
+  const long long M = static_cast<long long>(B) * T;
+  bf16* a_split = reinterpret_cast<bf16*>(ws + s.a_off);
+  bf16* w_split = reinterpret_cast<bf16*>(ws + s.w_off);
+  const long long n = M * E;
+  const int blocks = static_cast<int>((n + 255) / 256 < 148 * 16 ? (n + 255) / 256 : 148 * 16);
+  split_bf16_kernel<<<blocks, 256, 0, st>>>(encoded, a_split, M, E, xf32 ? 0 : 2);
+  split_bf16_kernel<<<(J * E + 255) / 256, 256, 0, st>>>(w.w_enc, w_split, J, E, 1);
+  GemmDesc g;
+  g.A = a_split;
+  g.lda = xf32 ? 3 * E : 2 * E;
+  g.W = w_split;
+  g.ldw = 3 * E;
+  g.M = static_cast<int>(M);
+  g.N = J;
+  g.K = xf32 ? 3 * E : 2 * E;
+  g.epi = EPI_LINEAR;
+  g.out_bf16 = false;
+  g.ep.bias = w.b_enc;
+  g.ep.out = reinterpret_cast<float*>(ws + s.encp_off);
+  g.ep.ldo = J;
+  std::string err;
+  return launch_gemm_tc(g, st, &err) != 0 ? CFB_ERR_CUDA : CFB_OK;
+}
+
 }  // namespace cfb
 
 using namespace cfb;
@@ -984,7 +969,7 @@ extern "C" {
 
 size_t cfb_rnnt_greedy_scratch_bytes(int enc_hidden, int pred_hidden, int joint_hidden, int B, int T) {
   if (enc_hidden < 1 || pred_hidden < 1 || joint_hidden < 1 || B < 1 || T < 1) return 0;
-  return rnnt_scratch_layout(enc_hidden, pred_hidden, joint_hidden, B, T).total;
+  return rnnt_scratch_layout(enc_hidden, pred_hidden, joint_hidden, B, T).enc.end;
 }
 
 int cfb_op_rnnt_greedy(const cfb_rnnt_weights* w, const void* encoded, int x_dtype, const int32_t* encoded_len, int B, int T,
@@ -992,24 +977,15 @@ int cfb_op_rnnt_greedy(const cfb_rnnt_weights* w, const void* encoded, int x_dty
                        float* h_out, float* c_out, int32_t* flags, void* scratch, size_t scratch_bytes, cfb_stream stream) {
   if (!w || !encoded || !encoded_len || !tokens || !timesteps || !n_tokens || !scores || !h_out || !c_out || !flags || !scratch)
     return CFB_ERR_INVALID_ARG;
+  if (B < 1 || T < 1 || max_tokens < 1 || !rnnt_weights_valid(*w, x_dtype)) return CFB_ERR_INVALID_ARG;
   const int E = w->enc_hidden, H = w->pred_hidden, J = w->joint_hidden, V1 = w->num_classes_with_blank;
-  if (B < 1 || T < 1 || max_tokens < 1 || E < 8 || (E % 8) || H < 4 || (H % 4) || J < 4 || (J % 4) || V1 < 2)
-    return CFB_ERR_INVALID_ARG;
-  if (w->activation < 0 || w->activation > 2 || (x_dtype != CFB_F32 && x_dtype != CFB_BF16)) return CFB_ERR_INVALID_ARG;
-  if (!w->embed || !w->w_ih || !w->w_hh || !w->b_ih || !w->b_hh || !w->w_pred || !w->b_pred || !w->w_enc || !w->b_enc || !w->w_out ||
-      !w->b_out)
-    return CFB_ERR_INVALID_ARG;
   const RnntScratch lay = rnnt_scratch_layout(E, H, J, B, T);
-  if (scratch_bytes < lay.total || (reinterpret_cast<uintptr_t>(scratch) & 255)) return CFB_ERR_WORKSPACE;
+  if (scratch_bytes < lay.enc.end || (reinterpret_cast<uintptr_t>(scratch) & 255)) return CFB_ERR_WORKSPACE;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   uint8_t* ws = reinterpret_cast<uint8_t*>(scratch);
 
-  int dev = 0, sms = 0, max_smem = 0, coop = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return CFB_ERR_CUDA;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-  cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
-  if (!coop || sms < 1) return CFB_ERR_UNSUPPORTED;
+  int sms = 0, max_smem = 0;
+  if (int rc = rnnt_device_query(&sms, &max_smem)) return rc;
   RnntParams p = {};
   cudaFuncAttributes fa;
   if (cudaFuncGetAttributes(&fa, rnnt_greedy_kernel) != cudaSuccess) return CFB_ERR_CUDA;
@@ -1035,35 +1011,9 @@ int cfb_op_rnnt_greedy(const cfb_rnnt_weights* w, const void* encoded, int x_dty
     return CFB_OK;
   };
   if (int rc = plan()) return rc;
+  if (int rc = rnnt_joint_enc(*w, encoded, x_dtype, B, T, ws, lay.enc, st)) return rc;
 
-  // joint.enc over every frame: encp = encoded W_enc^T + b_enc on the tensor cores with split operands
-  const bool xf32 = x_dtype == CFB_F32;
-  const long long M = static_cast<long long>(B) * T;
-  bf16* a_split = reinterpret_cast<bf16*>(ws + lay.a_off);
-  bf16* w_split = reinterpret_cast<bf16*>(ws + lay.w_off);
-  float* encp = reinterpret_cast<float*>(ws + lay.encp_off);
-  {
-    const long long n = M * E;
-    const int blocks = static_cast<int>((n + 255) / 256 < 148 * 16 ? (n + 255) / 256 : 148 * 16);
-    split_bf16_kernel<<<blocks, 256, 0, st>>>(encoded, a_split, M, E, xf32 ? 0 : 2);
-    split_bf16_kernel<<<(J * E + 255) / 256, 256, 0, st>>>(w->w_enc, w_split, J, E, 1);
-    GemmDesc g;
-    g.A = a_split;
-    g.lda = xf32 ? 3 * E : 2 * E;
-    g.W = w_split;
-    g.ldw = 3 * E;
-    g.M = static_cast<int>(M);
-    g.N = J;
-    g.K = xf32 ? 3 * E : 2 * E;
-    g.epi = EPI_LINEAR;
-    g.out_bf16 = false;
-    g.ep.bias = w->b_enc;
-    g.ep.out = encp;
-    g.ep.ldo = J;
-    std::string err;
-    if (launch_gemm_tc(g, st, &err) != 0) return CFB_ERR_CUDA;
-  }
-
+  const float* encp = reinterpret_cast<const float*>(ws + lay.enc.encp_off);
   for (int b0 = 0; b0 < B; b0 += kMaxB) {
     const int Bc = B - b0 < kMaxB ? B - b0 : kMaxB;
     if (cudaMemsetAsync(ws + lay.sync_off, 0, lay.sync_bytes + lay.hbuf_bytes, st) != cudaSuccess) return CFB_ERR_CUDA;
@@ -1085,20 +1035,8 @@ int cfb_op_rnnt_greedy(const cfb_rnnt_weights* w, const void* encoded, int x_dty
     p.c_out = c_out + static_cast<size_t>(b0) * H;
     p.flags = flags;
     if (clustered) {
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(grid);
-      cfg.blockDim = dim3(kThreads);
-      cfg.dynamicSmemBytes = smem;
-      cfg.stream = st;
       cudaLaunchAttribute attr[2];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = kC;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      attr[1].id = cudaLaunchAttributeCooperative;
-      attr[1].val.cooperative = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 2;
+      const cudaLaunchConfig_t cfg = c4_launch_config(grid, smem, st, true, attr);
       if (cudaLaunchKernelEx(&cfg, rnnt_greedy_c4_kernel, p) != cudaSuccess) {
         cudaGetLastError();      // refused (e.g. the clusters are not co-resident right now): nothing was enqueued
         g_c4_unusable = true;

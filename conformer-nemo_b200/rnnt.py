@@ -137,23 +137,15 @@ class RNNTJoint(nn.Module):
                                   "joint tensor and the fused loss / WER are training code and stay with the reference")
 
 
-class GreedyBatchedRNNTInfer:
-    """rnnt_greedy_decoding.py:358-616 (the ``blank_as_pad`` branch)."""
+class _DeviceRNNTInfer:
+    """What the greedy and the beam decoder share: fp32 copies of the decoder / joint weights and their refresh, the
+    checks and layout of the encoder output and lengths, and the device scratch buffer of the decode."""
 
-    def __init__(self, decoder_model: RNNTDecoder, joint_model: RNNTJoint, blank_index: int,
-                 max_symbols_per_step: Optional[int] = None, preserve_alignments: bool = False):
-        if preserve_alignments:
-            raise NotImplementedError("GreedyBatchedRNNTInfer (B200): preserve_alignments is a debugging aid of the reference")
-        if blank_index != decoder_model.blank_idx or blank_index != joint_model.num_classes_with_blank - 1:
-            raise ValueError("blank_index must be len(vocabulary) for the decoder and the joint (blank_as_pad)")
-        if decoder_model.pred_hidden != joint_model.pred_hidden:
-            raise ValueError("decoder pred_hidden and joint pred_hidden differ")
+    _name = None  # the class the error messages name
+
+    def __init__(self, decoder_model: RNNTDecoder, joint_model: RNNTJoint):
         self.decoder = decoder_model
         self.joint = joint_model
-        self._blank_index = blank_index
-        self._SOS = blank_index
-        self.max_symbols = max_symbols_per_step
-        self.preserve_alignments = False
         self._packed = None
         self._scratch = None
 
@@ -186,7 +178,7 @@ class GreedyBatchedRNNTInfer:
                  b_ih=f(lstm.bias_ih_l0), b_hh=f(lstm.bias_hh_l0), w_pred=f(jn.pred.weight), b_pred=f(jn.pred.bias),
                  w_enc=f(jn.enc.weight), b_enc=f(jn.enc.bias), w_out=f(out.weight), b_out=f(out.bias))
         if float(t["embed"][self._blank_index].abs().max()) != 0.0:
-            raise NotImplementedError("GreedyBatchedRNNTInfer (B200): the blank row of prediction.embed must be the zero padding row")
+            raise NotImplementedError(f"{self._name} (B200): the blank row of prediction.embed must be the zero padding row")
         w = _lib.CfbRnntWeights()
         w.enc_hidden, w.pred_hidden, w.joint_hidden = jn.encoder_hidden, dec.pred_hidden, jn.joint_hidden
         w.num_classes_with_blank, w.activation = jn.num_classes_with_blank, _ACTIVATIONS[jn.activation]
@@ -194,34 +186,64 @@ class GreedyBatchedRNNTInfer:
             setattr(w, k, ctypes.cast(ctypes.c_void_p(v.data_ptr()), ctypes.POINTER(ctypes.c_float)))
         self._packed = (w, t, device, self._fingerprint())
 
-    @torch.no_grad()
-    def decode_arrays(self, encoder_output: torch.Tensor, encoded_lengths: torch.Tensor, max_tokens: Optional[int] = None):
-        """Device-side result: dict of tokens / timesteps (B, max_tokens) int32, n_tokens (B) int32, scores (B) fp32,
-        h / c (B, H) fp32.  Enqueue-only (no synchronisation)."""
+    def _inputs(self, encoder_output: torch.Tensor, encoded_lengths: torch.Tensor):
+        """Checks the (B, D, T) encoder output, refreshes the weight copies if needed and returns the weights, the
+        contiguous (B, T, D) fp32 / bf16 encoder output and the int32 lengths on its device."""
         jn = self.joint
         if encoder_output.dim() != 3 or encoder_output.size(1) != jn.encoder_hidden:
             raise TypeError(f"encoder_output must be (B, {jn.encoder_hidden}, T), got {tuple(encoder_output.shape)}")
         if not encoder_output.is_cuda:
-            raise RuntimeError("GreedyBatchedRNNTInfer (B200) has no CPU path: encoder_output must be a CUDA tensor")
+            raise RuntimeError(f"{self._name} (B200) has no CPU path: encoder_output must be a CUDA tensor")
         device = encoder_output.device
         if self._packed is None or self._packed[2] != device or self._packed[3] != self._fingerprint():
             self._prepare(device)
-        w = self._packed[0]
-        b, d, t = encoder_output.shape
         x = encoder_output.transpose(1, 2)  # the encoder returns the transposed view of a contiguous (B, T, D) buffer
         if x.dtype not in (torch.float32, torch.bfloat16):
             x = x.float()
         x = x.contiguous()
         lens = encoded_lengths.to(device=device, dtype=torch.int32).contiguous()
+        return self._packed[0], x, lens
+
+    def _scratch_ptr(self, nbytes: int, device) -> ctypes.c_void_p:
+        """A 256-byte aligned device buffer of `nbytes`, kept between calls."""
+        if self._scratch is None or self._scratch.numel() < nbytes + 256 or self._scratch.device != device:
+            self._scratch = torch.empty(nbytes + 256, dtype=torch.uint8, device=device)
+        return ctypes.c_void_p((self._scratch.data_ptr() + 255) // 256 * 256)
+
+
+class GreedyBatchedRNNTInfer(_DeviceRNNTInfer):
+    """rnnt_greedy_decoding.py:358-616 (the ``blank_as_pad`` branch)."""
+
+    _name = "GreedyBatchedRNNTInfer"
+
+    def __init__(self, decoder_model: RNNTDecoder, joint_model: RNNTJoint, blank_index: int,
+                 max_symbols_per_step: Optional[int] = None, preserve_alignments: bool = False):
+        if preserve_alignments:
+            raise NotImplementedError("GreedyBatchedRNNTInfer (B200): preserve_alignments is a debugging aid of the reference")
+        if blank_index != decoder_model.blank_idx or blank_index != joint_model.num_classes_with_blank - 1:
+            raise ValueError("blank_index must be len(vocabulary) for the decoder and the joint (blank_as_pad)")
+        if decoder_model.pred_hidden != joint_model.pred_hidden:
+            raise ValueError("decoder pred_hidden and joint pred_hidden differ")
+        super().__init__(decoder_model, joint_model)
+        self._blank_index = blank_index
+        self._SOS = blank_index
+        self.max_symbols = max_symbols_per_step
+        self.preserve_alignments = False
+
+    @torch.no_grad()
+    def decode_arrays(self, encoder_output: torch.Tensor, encoded_lengths: torch.Tensor, max_tokens: Optional[int] = None):
+        """Device-side result: dict of tokens / timesteps (B, max_tokens) int32, n_tokens (B) int32, scores (B) fp32,
+        h / c (B, H) fp32.  Enqueue-only (no synchronisation)."""
+        w, x, lens = self._inputs(encoder_output, encoded_lengths)
+        device = x.device
+        b, t, d = x.shape
         max_symbols = 0 if self.max_symbols is None else int(self.max_symbols)
         if max_tokens is None:
             max_tokens = t * max_symbols if 0 < max_symbols <= 8 else 4 * t + 64
         max_tokens = max(int(max_tokens), 1)
         lib = _lib.load_library()
-        need = lib.cfb_rnnt_greedy_scratch_bytes(d, w.pred_hidden, w.joint_hidden, b, t) + 256
-        if self._scratch is None or self._scratch.numel() < need or self._scratch.device != device:
-            self._scratch = torch.empty(need, dtype=torch.uint8, device=device)
-        sptr = (self._scratch.data_ptr() + 255) // 256 * 256
+        need = lib.cfb_rnnt_greedy_scratch_bytes(d, w.pred_hidden, w.joint_hidden, b, t)
+        sptr = self._scratch_ptr(need, device)
         out = dict(tokens=torch.empty(b, max_tokens, dtype=torch.int32, device=device),
                    timesteps=torch.empty(b, max_tokens, dtype=torch.int32, device=device),
                    n_tokens=torch.empty(b, dtype=torch.int32, device=device),
@@ -234,12 +256,9 @@ class GreedyBatchedRNNTInfer:
             rc = lib.cfb_op_rnnt_greedy(ctypes.byref(w), vp(x), _lib.CFB_F32 if x.dtype == torch.float32 else _lib.CFB_BF16,
                                         vp(lens), b, t, max_symbols, max_tokens, vp(out["tokens"]), vp(out["timesteps"]),
                                         vp(out["n_tokens"]), vp(out["scores"]), vp(out["h"]), vp(out["c"]), vp(out["flags"]),
-                                        ctypes.c_void_p(sptr), need - 256,
-                                        ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream))
+                                        sptr, need, ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream))
         _lib.check(rc, None, "cfb_op_rnnt_greedy")
         out["_keepalive"] = (x, lens)
-        off = sptr - self._scratch.data_ptr()
-        out["phase_cycles"] = self._scratch[off + 64:off + 192].view(torch.int64)  # CTA 0's clocks per phase (debugging)
         return out
 
     @torch.no_grad()
@@ -282,7 +301,7 @@ class NBestHypotheses:
     n_best_hypotheses: Optional[List[Hypothesis]]
 
 
-class BeamRNNTInfer:
+class BeamRNNTInfer(_DeviceRNNTInfer):
     """``decoding.strategy = beam`` (parts/submodules/rnnt_beam_decoding.py, ``BeamRNNTInfer``): ``search_type='default'``
     (default_beam_search) and, for ``beam_size == 1``, the class's own sample-level greedy_search.  The search for every
     utterance of the batch runs in one persistent kernel (``cfb_op_rnnt_beam``, csrc/rnnt_beam.cu) with one device-to-host
@@ -293,6 +312,8 @@ class BeamRNNTInfer:
     ``dec_state`` the LSTM state ``(h, c)`` as (1, 1, H) CPU tensors (None for greedy_search before its first label),
     ``length`` the utterance's encoded length.  TSD / ALSD / MAES, language models, alignments and partial hypotheses raise
     NotImplementedError."""
+
+    _name = "BeamRNNTInfer"
 
     def __init__(self, decoder_model: RNNTDecoder, joint_model: RNNTJoint, beam_size: int, search_type: str = "default",
                  score_norm: bool = True, return_best_hypothesis: bool = True, tsd_max_sym_exp_per_step: Optional[int] = 50,
@@ -318,8 +339,7 @@ class BeamRNNTInfer:
             raise ValueError("decoder pred_hidden and joint pred_hidden differ")
         if decoder_model.blank_idx != joint_model.num_classes_with_blank - 1:
             raise ValueError("the decoder's blank index must be the joint's last class (blank_as_pad)")
-        self.decoder = decoder_model
-        self.joint = joint_model
+        super().__init__(decoder_model, joint_model)
         self.blank = decoder_model.blank_idx
         self.vocab_size = decoder_model.vocab_size
         self.search_type = search_type
@@ -330,17 +350,6 @@ class BeamRNNTInfer:
         self.softmax_temperature = float(softmax_temperature)
         self.preserve_alignments = False
         self._blank_index = self.blank
-        self._packed = None
-        self._scratch = None
-
-    # the fp32 weight copies and their refresh are those of the greedy decode
-    _sources = GreedyBatchedRNNTInfer._sources
-    _fingerprint = GreedyBatchedRNNTInfer._fingerprint
-    _prepare = GreedyBatchedRNNTInfer._prepare
-    invalidate = GreedyBatchedRNNTInfer.invalidate
-
-    def __call__(self, *args, **kwargs):
-        return self.forward(*args, **kwargs)
 
     def widths(self) -> Tuple[int, int]:
         """(beam, beam_k) of default_beam_search: hypotheses that end a frame, non-blank candidates per expansion."""
@@ -358,31 +367,17 @@ class BeamRNNTInfer:
     def decode_arrays(self, encoder_output: torch.Tensor, encoded_lengths: torch.Tensor, caps: Optional[Dict[str, int]] = None):
         """Device-side result (enqueue-only): n_hyps (B), lengths (B, X), tokens / timesteps (B, X, L) int32, scores (B, X)
         fp64, h / c (B, X, H) fp32, stats (B, 4) int32, flags (1); X = max_expansions, L = max_len of ``caps``."""
-        jn = self.joint
-        if encoder_output.dim() != 3 or encoder_output.size(1) != jn.encoder_hidden:
-            raise TypeError(f"encoder_output must be (B, {jn.encoder_hidden}, T), got {tuple(encoder_output.shape)}")
-        if not encoder_output.is_cuda:
-            raise RuntimeError("BeamRNNTInfer (B200) has no CPU path: encoder_output must be a CUDA tensor")
-        device = encoder_output.device
-        if self._packed is None or self._packed[2] != device or self._packed[3] != self._fingerprint():
-            self._prepare(device)
-        w = self._packed[0]
-        b, d, t = encoder_output.shape
+        w, x, lens = self._inputs(encoder_output, encoded_lengths)
+        device = x.device
+        b, t, d = x.shape
         caps = dict(self.default_caps(t), **(caps or {}))
         c = _lib.CfbRnntBeamCaps()
         for k, v in caps.items():
             setattr(c, k, int(v))
-        x = encoder_output.transpose(1, 2)
-        if x.dtype not in (torch.float32, torch.bfloat16):
-            x = x.float()
-        x = x.contiguous()
-        lens = encoded_lengths.to(device=device, dtype=torch.int32).contiguous()
         lib = _lib.load_library()
         need = lib.cfb_rnnt_beam_scratch_bytes(d, w.pred_hidden, w.joint_hidden, w.num_classes_with_blank, b, t,
-                                               ctypes.byref(c)) + 256
-        if self._scratch is None or self._scratch.numel() < need or self._scratch.device != device:
-            self._scratch = torch.empty(need, dtype=torch.uint8, device=device)
-        sptr = (self._scratch.data_ptr() + 255) // 256 * 256
+                                               ctypes.byref(c))
+        sptr = self._scratch_ptr(need, device)
         X, L, H = c.max_expansions, c.max_len, w.pred_hidden
         i32 = dict(dtype=torch.int32, device=device)
         out = dict(n_hyps=torch.empty(b, **i32), lengths=torch.zeros(b, X, **i32), tokens=torch.empty(b, X, L, **i32),
@@ -396,13 +391,11 @@ class BeamRNNTInfer:
                                       vp(lens), b, t, self.beam_size, int(bool(self.score_norm)), self.softmax_temperature,
                                       ctypes.byref(c), vp(out["n_hyps"]), vp(out["lengths"]), vp(out["tokens"]),
                                       vp(out["timesteps"]), vp(out["scores"]), vp(out["h"]), vp(out["c"]), vp(out["stats"]),
-                                      vp(out["flags"]), ctypes.c_void_p(sptr), need - 256,
+                                      vp(out["flags"]), sptr, need,
                                       ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream))
         _lib.check(rc, None, "cfb_op_rnnt_beam")
         out["_keepalive"] = (x, lens)
         out["caps"] = caps
-        off = sptr - self._scratch.data_ptr()
-        out["phase_cycles"] = self._scratch[off + 64:off + 192].view(torch.int64)  # CTA 0's clocks per phase (debugging)
         return out
 
     @torch.no_grad()

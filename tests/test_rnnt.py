@@ -364,9 +364,9 @@ print("CLUSTER_VARIANT_OK")
 
 @pytest.mark.gpu
 def test_gpu_both_kernel_variants_match_oracle():
-    """CFB_RNNT_CLUSTER=1 selects the kernel that splits the weights over K inside clusters of 4 CTAs and adds the partial
-    sums through distributed shared memory (rnnt_greedy_c4_kernel); the default is the row-partitioned one
-    (rnnt_greedy_kernel).  Same hypotheses as the oracle from both.  Runs in a child process: tools that intercept launches
+    """The default kernel, wherever the sizes and the device allow it, splits the weights over K inside clusters of 4 CTAs
+    and adds the partial sums through distributed shared memory (rnnt_greedy_c4_kernel); CFB_RNNT_CLUSTER=0 forces the
+    row-partitioned one (rnnt_greedy_kernel).  Same hypotheses as the oracle from both.  Runs in a child process: tools that intercept launches
     (Nsight Compute) abort a process on a cooperative cluster launch, which must not take the test session with it."""
     import subprocess
     import sys

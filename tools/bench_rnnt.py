@@ -6,8 +6,8 @@ bias is calibrated (with the kernel itself) to a speech-like symbol rate (--rate
     python tools/bench_rnnt.py [--batch 32] [--frames 500] [--steps 20] [--cpu-sample 2]
 
 Prints one JSON line: audio-s/s of the decode alone (encoder output resident in HBM), the end-to-end figure through
-GreedyBatchedRNNTInfer.forward (hypotheses on the host), iterations (= lock-step joint evaluations), symbols, and the
-CPU oracle timed on a bounded sample of the same batch.
+GreedyBatchedRNNTInfer.forward (hypotheses on the host), symbols, and the CPU oracle timed on a bounded sample of the same
+batch.
 """
 import argparse
 import json
@@ -65,8 +65,6 @@ def main():
     out = greedy.decode_arrays(xg, lg)
     torch.cuda.synchronize()
     n_tok = out["n_tokens"].cpu()
-    phases = dict(zip(["joint", "barrier_joint", "control", "lstm", "barrier_lstm", "pred", "barrier_pred", "loop", "joint_stage", "joint_compute", "iterations", "lstm_stage", "pred_stage"],
-                      out["phase_cycles"].cpu().tolist()))
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     for _ in range(args.warmup):
         greedy.decode_arrays(xg, lg)
@@ -82,14 +80,12 @@ def main():
         greedy(encoder_output=xg, encoded_lengths=lg)
     e2e_ms = (time.perf_counter() - t0) / args.steps * 1e3
     audio_s = B * T * 0.04  # 40 ms per encoder frame (10 ms hop x 4 subsampling)
-    iters = int(phases.pop("iterations"))  # lock-step iterations (each consumes up to two frames or one symbol per utterance)
     line = dict(metric="transducer greedy decode audio-sec/sec", value=audio_s / (ms * 1e-3), unit="audio-sec/sec",
                 ms_per_batch=ms, e2e=dict(value=audio_s / (e2e_ms * 1e-3), ms_per_batch=e2e_ms,
                                           mode="GreedyBatchedRNNTInfer.forward: decode + hypotheses on the host"),
                 config=dict(workload=f"Conformer-Transducer Large decoder/joint (512/640/640/1025), {B} x {T} frames, max_symbols 30",
                             encoder_output_dtype=args.dtype, blank_bias=bias, symbols_per_frame=symbols_per_frame),
-                symbols=int(n_tok.sum()), iterations=iters, us_per_iteration=ms * 1e3 / max(iters, 1), gpu_launches=5,
-                phase_cycles_cta0=phases)
+                symbols=int(n_tok.sum()), gpu_launches=5)
     if args.cpu_sample > 0:
         k = min(args.cpu_sample, B)
         torch.set_num_threads(os.cpu_count() or 1)

@@ -6,7 +6,7 @@ blank bias calibrated with the greedy kernel to a speech-like symbol rate as in 
 
 For every beam size: ms per batch and audio-s/s of cfb_op_rnnt_beam (encoder output resident in HBM, capacities already
 grown to what the batch needs, so one launch sequence per decode), expansions per frame (hypotheses popped = lock-step
-work items), the end-to-end BeamRNNTInfer.forward time, and CTA 0's phase clocks.  The greedy kernel on the same input
+work items) and the end-to-end BeamRNNTInfer.forward time.  The greedy kernel on the same input
 and the CPU oracle (oracle/rnnt_beam_oracle.py, the restatement of the reference's BeamRNNTInfer) on a bounded sample
 of frames are timed beside it.  Prints one JSON document; --out also writes it to a file.
 """
@@ -23,8 +23,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 import conformer_nemo_b200 as cn  # noqa: E402
-
-PHASES = ["lstm", "pred", "joint", "control", "barrier", "unused5", "iterations", "loop"]
 
 
 def main():
@@ -102,21 +100,18 @@ def main():
         out = beam.decode_arrays(xg, lg, caps)
         assert int(out["flags"].cpu()) == 0
         stats = out["stats"].cpu()
-        phases = dict(zip(PHASES, out["phase_cycles"].cpu().tolist()[:len(PHASES)]))
         ms = timed(lambda: beam.decode_arrays(xg, lg, caps))
         t0 = time.perf_counter()
         for _ in range(args.steps):
             beam.decode_arrays(xg, lg, caps)["flags"].cpu()
         e2e_ms = (time.perf_counter() - t0) / args.steps * 1e3
-        iters = int(phases.pop("iterations"))
-        phases.pop("unused5")
         expansions = int(stats[:, 0].sum())
         doc["beams"][str(beam_size)] = dict(
             ms_per_batch=ms, value=audio_s / (ms * 1e-3), unit="audio-sec/sec", decode_arrays_with_sync_ms=e2e_ms,
             expansions_per_frame=expansions / (B * T), max_expansions_at_one_frame=int(stats[:, 3].max()),
             prefix_tree_nodes_max=int(stats[:, 1].max()), state_slots_max=int(stats[:, 2].max()),
             best_hypothesis_labels_per_frame=sum(len(h.y_sequence) - (beam_size > 1) for h in hyps) / (B * T),
-            lock_step_iterations=iters, us_per_iteration=ms * 1e3 / max(iters, 1), caps=caps, phase_cycles_cta0=phases)
+            caps=caps)
         print(json.dumps({str(beam_size): doc["beams"][str(beam_size)]}), flush=True)
     if args.cpu_frames > 0:
         tf = min(args.cpu_frames, T)

@@ -11,3 +11,4 @@ from .preprocessor import AudioToMelSpectrogramPreprocessor  # noqa: F401
 from .rnnt import RNNTDecoder, RNNTJoint, GreedyBatchedRNNTInfer, GreedyRNNTInfer, Hypothesis  # noqa: F401
 from .rnnt import BeamRNNTInfer, NBestHypotheses  # noqa: F401
 from .collation import (BucketingIterator, CollationService, ManifestEntry, read_manifest, speech_collate)  # noqa: F401
+from .buffered import FrameBatchASR, buffered_ctc_transcribe  # noqa: F401

@@ -24,7 +24,8 @@ SYMBOLS = [
     "cfb_create", "cfb_destroy", "cfb_last_error", "cfb_set_weight", "cfb_finalize_weights", "cfb_output_frames",
     "cfb_workspace_bytes", "cfb_forward", "cfb_packed_workspace_bytes", "cfb_forward_packed", "cfb_debug_buffer", "cfb_set_profiling", "cfb_profile_report",
     "cfb_last_launch_count", "cfb_op_gemm", "cfb_op_ctc_head", "cfb_ctc_head_scratch_bytes", "cfb_op_ctc_collapse",
-    "cfb_op_layernorm", "cfb_op_layernorm_dual", "cfb_op_depthwise", "cfb_op_dw_pw2", "cfb_op_logmel", "cfb_op_rel_attention", "cfb_op_lengths",
+    "cfb_op_layernorm", "cfb_op_layernorm_dual", "cfb_op_depthwise", "cfb_op_dw_pw2", "cfb_op_logmel", "cfb_op_logmel_raw",
+    "cfb_op_feature_buffers", "cfb_op_rel_attention", "cfb_op_lengths",
     "cfb_rnnt_greedy_scratch_bytes", "cfb_op_rnnt_greedy", "cfb_rnnt_beam_scratch_bytes", "cfb_op_rnnt_beam",
 ]
 
@@ -96,6 +97,9 @@ def load_library() -> ctypes.CDLL:
         lib.cfb_op_depthwise.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]
         lib.cfb_op_logmel.argtypes = [vp, vp, i32, i32, vp, i32, i32, i32, vp, vp, i32, ctypes.c_float, ctypes.c_float,
                                       ctypes.c_float, vp, i32, vp, vp, vp]
+        lib.cfb_op_logmel_raw.argtypes = [vp, vp, i32, i32, vp, i32, i32, i32, vp, vp, i32, ctypes.c_float, ctypes.c_float,
+                                          vp, i32, vp, vp]
+        lib.cfb_op_feature_buffers.argtypes = [vp, i32, i32, i32, vp, vp, i32, i32, i32, vp, vp]
         lib.cfb_op_dw_pw2.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, vp]
         lib.cfb_op_rel_attention.argtypes = [i32, vp, vp, i64, vp, vp, i32, i32, i32, i32, i32, vp]
         lib.cfb_op_lengths.argtypes = [vp, vp, i32, i32, i32, vp]

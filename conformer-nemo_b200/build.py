@@ -20,7 +20,7 @@ OBJ_DIR = os.path.join(HERE, "build")
 LIB_PATH = os.path.join(LIB_DIR, "libcfb.so")
 
 SOURCES = ["engine.cu", "tmap.cu", "gemm_tc.cu", "gemm_tc2.cu", "gemm_simt.cu", "elementwise.cu", "packed.cu", "conv_tail.cu", "attention_tc.cu", "attention_tcp.cu",
-           "attention_tc128.cu", "attention_simt.cu", "ctc_head.cu", "frontend.cu", "rnnt_greedy.cu",
+           "attention_tc128.cu", "attention_simt.cu", "ctc_head.cu", "frontend.cu", "buffered.cu", "rnnt_greedy.cu",
            "rnnt_beam.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
               "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr", "-Xptxas", "-v"]

@@ -194,8 +194,13 @@ struct LogMelDesc {
   int T_out = 0;                  // >= 1 + L / hop; frames from seq_len on are written as zeros
   void* seq_len = nullptr;        // (B) int64
   int* flag = nullptr;            // set to 1 when some utterance has exactly one frame (the reference raises)
+  bool normalize = true;          // false: normalize "None" -- no statistics, no flag (flag may be null)
 };
 int launch_logmel(const LogMelDesc& d, cudaStream_t st, std::string* err);
+
+// buffered long-audio inference (buffered.cu): the normalised overlapping windows of FeatureFrameBufferer
+int launch_feature_buffers(const float* feat, int n_files, int F, int T, const long long* seq_len, const int* first_window,
+                           int n_windows, int fl, int W, float* out, cudaStream_t st, std::string* err);
 
 // depth-wise conv (+ folded BatchNorm + Swish) fused into pointwise_conv2 and the residual update (conv_tail.cu):
 //   x[b,t,:] += W2 * swish(bias_dw + sum_k taps[k] * g[b, t + k - 15, :]) + bias2

@@ -1198,9 +1198,10 @@ int cfb_op_dw_pw2(const void* g, const float* taps32, const void* W, const float
   return rc == 0 ? CFB_OK : op_fail(rc, err);
 }
 
-int cfb_op_logmel(const float* audio, const int64_t* lengths, int B, int L, const float* window, int win_length, int n_fft,
-                  int hop, const float* fb, const int32_t* fb_span, int n_mels, float preemph, float log_guard, float std_eps, float* features,
-                  int T_out, int64_t* seq_len, int32_t* flag, cfb_stream stream) {
+namespace {
+int run_logmel(const float* audio, const int64_t* lengths, int B, int L, const float* window, int win_length, int n_fft,
+               int hop, const float* fb, const int32_t* fb_span, int n_mels, float preemph, float log_guard, bool normalize,
+               float std_eps, float* features, int T_out, int64_t* seq_len, int32_t* flag, cfb_stream stream) {
   LogMelDesc d;
   d.audio = audio;
   d.lengths = lengths;
@@ -1215,14 +1216,41 @@ int cfb_op_logmel(const float* audio, const int64_t* lengths, int B, int L, cons
   d.n_mels = n_mels;
   d.preemph = preemph;
   d.log_guard = log_guard;
+  d.normalize = normalize;
   d.std_eps = std_eps;
   d.features = features;
   d.T_out = T_out;
   d.seq_len = seq_len;
   d.flag = flag;
-  if (!audio || !lengths || !window || !fb || !fb_span || !features || !seq_len || !flag) return op_fail(-1, "logmel: null pointer");
+  if (!audio || !lengths || !window || !fb || !fb_span || !features || !seq_len || (normalize && !flag))
+    return op_fail(-1, "logmel: null pointer");
   std::string err;
   int rc = launch_logmel(d, reinterpret_cast<cudaStream_t>(stream), &err);
+  return rc == 0 ? CFB_OK : op_fail(rc, err);
+}
+}  // namespace
+
+int cfb_op_logmel(const float* audio, const int64_t* lengths, int B, int L, const float* window, int win_length, int n_fft,
+                  int hop, const float* fb, const int32_t* fb_span, int n_mels, float preemph, float log_guard, float std_eps, float* features,
+                  int T_out, int64_t* seq_len, int32_t* flag, cfb_stream stream) {
+  return run_logmel(audio, lengths, B, L, window, win_length, n_fft, hop, fb, fb_span, n_mels, preemph, log_guard, true, std_eps,
+                    features, T_out, seq_len, flag, stream);
+}
+
+int cfb_op_logmel_raw(const float* audio, const int64_t* lengths, int B, int L, const float* window, int win_length, int n_fft,
+                      int hop, const float* fb, const int32_t* fb_span, int n_mels, float preemph, float log_guard,
+                      float* features, int T_out, int64_t* seq_len, cfb_stream stream) {
+  return run_logmel(audio, lengths, B, L, window, win_length, n_fft, hop, fb, fb_span, n_mels, preemph, log_guard, false, 0.f,
+                    features, T_out, seq_len, nullptr, stream);
+}
+
+int cfb_op_feature_buffers(const float* features, int n_files, int F, int T, const int64_t* seq_len,
+                           const int32_t* first_window, int n_windows, int frame_len, int buffer_len, float* out,
+                           cfb_stream stream) {
+  if (!features || !seq_len || !first_window || !out) return op_fail(-1, "feature_buffers: null pointer");
+  std::string err;
+  int rc = launch_feature_buffers(features, n_files, F, T, reinterpret_cast<const long long*>(seq_len), first_window,
+                                  n_windows, frame_len, buffer_len, out, reinterpret_cast<cudaStream_t>(stream), &err);
   return rc == 0 ? CFB_OK : op_fail(rc, err);
 }
 

@@ -13,7 +13,8 @@
 //   logmel_normalize_kernel  one warp per (utterance, mel bin) row: mean, unbiased std + 1e-5 over the valid frames
 //                            (two passes over a row that the first kernel just left in L2), normalised in place,
 //                            zeros from seq_len on; also writes seq_len = floor(len / hop) + 1 computed in float32
-//                            like features.py:347-353.
+//                            like features.py:347-353.  With normalisation off (normalize: "None", the buffered
+//                            long-audio front end) the same kernel only writes seq_len and zeroes the tail.
 // Both are bandwidth-trivial next to the encoder (640 s of audio: 41 MB in, 20 MB out); no tensor cores on purpose.
 #include <math.h>
 #include <stdio.h>
@@ -143,7 +144,8 @@ __device__ __forceinline__ float warp_sum_f(float v) {
 
 __global__ void __launch_bounds__(256)
 logmel_normalize_kernel(float* __restrict__ feat, const long long* __restrict__ lengths, int n_rows, int n_mels, int T,
-                        int T_out, int hop, float std_eps, long long* __restrict__ seq_len_out, int* __restrict__ flag) {
+                        int T_out, int hop, bool normalize, float std_eps, long long* __restrict__ seq_len_out,
+                        int* __restrict__ flag) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   pdl_launch_dependents();
@@ -156,10 +158,14 @@ logmel_normalize_kernel(float* __restrict__ feat, const long long* __restrict__ 
                                                            static_cast<float>(hop)))) + 1;
   if (row % n_mels == 0 && lane == 0) {
     seq_len_out[b] = n_ll;
-    if (n_ll == 1) atomicExch(flag, 1);  // the reference raises: std of one frame is NaN (features.py:58-62)
+    if (normalize && n_ll == 1) atomicExch(flag, 1);  // the reference raises: std of one frame is NaN (features.py:58-62)
   }
   const int n = static_cast<int>(n_ll < 0 ? 0 : (n_ll > T ? T : n_ll));
   float* r = feat + static_cast<long long>(row) * T_out;
+  if (!normalize) {  // normalize_batch returns x unchanged; frames from seq_len on are still set to pad_value (0)
+    for (int t = n + lane; t < T_out; t += 32) r[t] = 0.f;
+    return;
+  }
   float s = 0.f;
   for (int t = lane; t < n; t += 32) s += r[t];
   const float mean = warp_sum_f(s) / static_cast<float>(n);
@@ -189,13 +195,15 @@ int launch_logmel(const LogMelDesc& d, cudaStream_t st, std::string* err) {
     if (err) *err = "logmel: T_out is smaller than 1 + L / hop";
     return -1;
   }
-  cudaError_t e = cudaMemsetAsync(d.flag, 0, sizeof(int), st);
-  if (e != cudaSuccess) return static_cast<int>(e);
+  if (d.normalize) {
+    cudaError_t e = cudaMemsetAsync(d.flag, 0, sizeof(int), st);
+    if (e != cudaSuccess) return static_cast<int>(e);
+  }
   launch_pdl(logmel_frames_kernel, dim3((T + kFramesPerCta - 1) / kFramesPerCta, d.B), dim3(32 * kWarps), 0, st, d.audio, d.L,
              d.window, d.win_length, d.hop, d.fb, d.fb_span, d.n_mels, d.preemph, d.log_guard, d.features, T, d.T_out);
   const int rows = d.B * d.n_mels;
   launch_pdl(logmel_normalize_kernel, dim3((rows + 7) / 8), dim3(256), 0, st, d.features,
-             reinterpret_cast<const long long*>(d.lengths), rows, d.n_mels, T, d.T_out, d.hop, d.std_eps,
+             reinterpret_cast<const long long*>(d.lengths), rows, d.n_mels, T, d.T_out, d.hop, d.normalize, d.std_eps,
              reinterpret_cast<long long*>(d.seq_len), d.flag);
   return static_cast<int>(cudaGetLastError());
 }

@@ -4,8 +4,9 @@
 Same constructor arguments, same buffers / ``state_dict`` keys (``featurizer.window`` (win_length),
 ``featurizer.fb`` (1, features, n_fft / 2 + 1)), same call
 ``preprocessor(input_signal=(B, L) float, length=(B,) int) -> (processed_signal (B, features, T), processed_length)``.
-The arithmetic runs in two CUDA kernels of libcfb.so (csrc/frontend.cu, C ABI ``cfb_op_logmel``); there is no CPU
-fallback.  Configurations no Conformer recipe uses are rejected at construction.
+The arithmetic runs in two CUDA kernels of libcfb.so (csrc/frontend.cu, C ABI ``cfb_op_logmel``; ``cfb_op_logmel_raw``
+for ``normalize=None`` / ``"None"``, the front end buffered inference builds); there is no CPU fallback.
+Configurations no Conformer recipe uses are rejected at construction.
 """
 from __future__ import annotations
 
@@ -88,7 +89,7 @@ class AudioToMelSpectrogramPreprocessor(nn.Module):
             unsupported.append(f"n_fft={self.n_fft} (the kernel is built for n_fft = 512)")
         if window not in self._WINDOWS:
             unsupported.append(f"window={window!r}")
-        if normalize != "per_feature":
+        if normalize not in ("per_feature", None, "None"):
             unsupported.append(f"normalize={normalize!r}")
         if not log or log_zero_guard_type != "add" or isinstance(log_zero_guard_value, str):
             unsupported.append("log / log_zero_guard settings other than log(x + number)")
@@ -100,6 +101,7 @@ class AudioToMelSpectrogramPreprocessor(nn.Module):
             unsupported.append(f"pad_to={pad_to!r}")
         if unsupported:
             raise NotImplementedError("AudioToMelSpectrogramPreprocessor (B200) does not support: " + "; ".join(unsupported))
+        self.normalize = None if normalize == "None" else normalize
         self.preemph = preemph
         self.log_zero_guard_value = float(log_zero_guard_value)
         self.dither = dither  # training-time noise only (features.py:367-368): inference ignores it
@@ -170,11 +172,15 @@ class AudioToMelSpectrogramPreprocessor(nn.Module):
         out = torch.empty(B, self.nfilt, T_out, dtype=torch.float32, device=dev)
         seq_len = torch.empty(B, dtype=torch.int64, device=dev)
         vp = ctypes.c_void_p
-        rc = lib.cfb_op_logmel(vp(x.data_ptr()), vp(lens.data_ptr()), B, L, vp(self._window.data_ptr()), self.win_length,
-                               self.n_fft, self.hop_length, vp(self._fb_km.data_ptr()), vp(self._fb_span.data_ptr()), self.nfilt,
-                               float(self.preemph if self.preemph is not None else 0.0), self.log_zero_guard_value, 1e-5,
-                               vp(out.data_ptr()), T_out, vp(seq_len.data_ptr()), vp(self._flag.data_ptr()),
-                               vp(torch.cuda.current_stream(dev).cuda_stream))
+        head = (vp(x.data_ptr()), vp(lens.data_ptr()), B, L, vp(self._window.data_ptr()), self.win_length, self.n_fft,
+                self.hop_length, vp(self._fb_km.data_ptr()), vp(self._fb_span.data_ptr()), self.nfilt,
+                float(self.preemph if self.preemph is not None else 0.0), self.log_zero_guard_value)
+        stream = vp(torch.cuda.current_stream(dev).cuda_stream)
+        if self.normalize is None:  # normalize_batch returns x unchanged: no statistics, nothing to check
+            _lib.check(lib.cfb_op_logmel_raw(*head, vp(out.data_ptr()), T_out, vp(seq_len.data_ptr()), stream), None,
+                       "cfb_op_logmel_raw")
+            return out, seq_len
+        rc = lib.cfb_op_logmel(*head, 1e-5, vp(out.data_ptr()), T_out, vp(seq_len.data_ptr()), vp(self._flag.data_ptr()), stream)
         _lib.check(rc, None, "cfb_op_logmel")
         if check_lengths and int(self._flag.item()):  # one device read-back; pass check_lengths=False to stay asynchronous
             raise ValueError("normalize_batch with `per_feature` normalize_type received a tensor of length 1. This will "

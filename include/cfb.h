@@ -200,6 +200,26 @@ CFB_API int cfb_op_logmel(const float* audio, const int64_t* lengths, int B, int
                   int n_fft, int hop, const float* fb, const int32_t* fb_span, int n_mels, float preemph, float log_guard, float std_eps,
                   float* features, int T_out, int64_t* seq_len, int32_t* flag, cfb_stream stream);
 
+/* The same front end with normalize = "None" (what buffered inference builds: features.py normalize_batch returns x
+ * unchanged): log-mel values as they are, frames t >= seq_len set to 0.  Same arguments as cfb_op_logmel without std_eps
+ * and flag (no statistics, so a one-frame utterance is not an error). */
+CFB_API int cfb_op_logmel_raw(const float* audio, const int64_t* lengths, int B, int L, const float* window, int win_length,
+                      int n_fft, int hop, const float* fb, const int32_t* fb_span, int n_mels, float preemph, float log_guard,
+                      float* features, int T_out, int64_t* seq_len, cfb_stream stream);
+
+/* Buffered long-audio inference (streaming_utils.py:455-684, AudioFeatureIterator + FeatureFrameBufferer): the normalised
+ * overlapping windows of many files in one launch, ready to be the encoder's audio_signal.
+ *   features      (n_files, F, T) fp32 raw log-mel features (cfb_op_logmel_raw);  seq_len (n_files) int64 valid frames n
+ *   first_window  (n_files) int32, ascending: file f owns windows first_window[f] ... first_window[f+1] - 1 (the last file
+ *                 up to n_windows - 1); a file has n / frame_len + 1 windows
+ *   out           (n_windows, F, buffer_len) fp32.  Column j of the file's window k is frame s = (k+1) frame_len -
+ *                 buffer_len + j: -16.635 (log-mel silence) for s < 0, features[:, s] for s < n, 0 after; then each
+ *                 (window, mel) row becomes (x - mean) / (std + 1e-5), mean and population std over its buffer_len columns.
+ * 1 <= frame_len <= buffer_len.  Enqueue-only on `stream`; all pointers are device pointers. */
+CFB_API int cfb_op_feature_buffers(const float* features, int n_files, int F, int T, const int64_t* seq_len,
+                           const int32_t* first_window, int n_windows, int frame_len, int buffer_len, float* out,
+                           cfb_stream stream);
+
 /* Relative-position multi-head attention core (multi_head_attention.py:195-210 + :104-113), everything between the
  * q/k/v projections and linear_out:
  *   qkv  (B*T, 4*Dp): [q+u | q+v | k | v], head h at columns h*dkp .. h*dkp+dk-1 of each part (Dp = H*dkp)

@@ -1134,11 +1134,36 @@ int op_fail(int rc, const std::string& err) {
   g_create_error = g_op_error;  // cfb_last_error(NULL) reports handle-less failures
   return CFB_ERR_CUDA;
 }
+int op_refuse(int code, const std::string& err) {
+  g_op_error = err;
+  g_create_error = g_op_error;
+  return code;
+}
+
+// The (epilogue, output type, shape) combinations the GEMM kernels can write; anything else would store another type's
+// rows into `out`, write past its rows or read past bias2, so it is refused before anything is enqueued.
+int gemm_args_error(int use_tc, int epi, int N, int64_t ldo, int out_dtype, int qkv_dp) {
+  if (epi < CFB_EPI_LINEAR || epi > CFB_EPI_GLU) return op_refuse(CFB_ERR_INVALID_ARG, "op_gemm: unknown epilogue");
+  if (out_dtype != CFB_F32 && out_dtype != CFB_BF16)
+    return op_refuse(CFB_ERR_UNSUPPORTED, "op_gemm: out_dtype must be CFB_F32 or CFB_BF16");
+  if (epi == CFB_EPI_RESID && out_dtype != CFB_F32)
+    return op_refuse(CFB_ERR_UNSUPPORTED, "op_gemm: the residual epilogue adds into an fp32 stream (out_dtype CFB_F32)");
+  if (use_tc && out_dtype == CFB_F32 && epi != CFB_EPI_LINEAR && epi != CFB_EPI_RESID)
+    return op_refuse(CFB_ERR_UNSUPPORTED, "op_gemm: on tensor cores only the linear and residual epilogues write fp32");
+  if (epi == CFB_EPI_QKV && (qkv_dp <= 0 || qkv_dp % 64 || static_cast<int64_t>(N) != 3 * static_cast<int64_t>(qkv_dp)))
+    return op_refuse(CFB_ERR_INVALID_ARG, "op_gemm: QKV needs qkv_dp > 0, qkv_dp % 64 == 0 and N == 3 * qkv_dp");
+  if (epi == CFB_EPI_GLU && N % 32)
+    return op_refuse(CFB_ERR_INVALID_ARG, "op_gemm: GLU needs N % 32 == 0 (groups of [16 a | 16 gate] columns)");
+  const int64_t cols = epi == CFB_EPI_QKV ? static_cast<int64_t>(N) + qkv_dp : epi == CFB_EPI_GLU ? N / 2 : N;
+  if (ldo < cols) return op_refuse(CFB_ERR_INVALID_ARG, "op_gemm: ldo is smaller than the output's column count");
+  return CFB_OK;
+}
 }  // namespace
 
 int cfb_op_gemm(int use_tc, int epilogue, const void* A, int64_t lda, const void* W, int64_t ldw, const float* bias,
                 const float* bias2, int M, int N, int K, void* out, int64_t ldo, int out_dtype, float alpha,
                 const int32_t* lens, int frames_per_seq, int qkv_dp, float* scratch, cfb_stream stream) {
+  if (int rc = gemm_args_error(use_tc, epilogue, N, ldo, out_dtype, qkv_dp)) return rc;
   GemmDesc g;
   g.A = A;
   g.lda = lda;

@@ -155,9 +155,17 @@ typedef enum cfb_epilogue {
 
 /* D = A (M x K, row-major, lda) * W^T (W: N x K row-major, ldw) with the selected epilogue.
  * use_tensor_cores != 0: A/W are bf16 and the tcgen05 kernel runs; == 0: A/W are fp32 and the CUDA-core
- * validation kernel runs (raw accumulators go through `scratch`, M*N floats).  out_dtype CFB_BF16 / CFB_F32.
- * bias2 only for QKV; lens/frames_per_seq only for GLU (row r belongs to sequence r / frames_per_seq);
- * for QKV and GLU, N counts accumulator columns (3*Dp resp. 2*d) and `out` has 4*Dp resp. d columns. */
+ * validation kernel runs (raw accumulators go through `scratch`, M*N floats).
+ * bias2 only for QKV.  lens/frames_per_seq (row r belongs to sequence r / frames_per_seq) zero the rows at frames
+ * t >= lens[seq] for LINEAR, SWISH, RELU and GLU; RESID and QKV ignore them.
+ * For QKV and GLU, N counts accumulator columns (3*Dp resp. 2*d) and `out` has 4*Dp resp. d columns.
+ * Accepted combinations (anything else returns before enqueueing anything):
+ *   out_dtype    CFB_F32 or CFB_BF16 (else CFB_ERR_UNSUPPORTED); RESID: CFB_F32 only, and with use_tensor_cores
+ *                the other epilogues except LINEAR: CFB_BF16 only (CFB_ERR_UNSUPPORTED);
+ *   QKV          qkv_dp > 0, qkv_dp % 64 == 0, N == 3 * qkv_dp (CFB_ERR_INVALID_ARG);
+ *   GLU          N % 32 == 0 (CFB_ERR_INVALID_ARG);
+ *   ldo          >= the output's column count: N, 4*Dp for QKV, N/2 for GLU (CFB_ERR_INVALID_ARG);
+ *   epilogue     a cfb_epilogue value (CFB_ERR_INVALID_ARG). */
 CFB_API int cfb_op_gemm(int use_tensor_cores, int epilogue, const void* A, int64_t lda, const void* W, int64_t ldw,
                 const float* bias, const float* bias2, int M, int N, int K, void* out, int64_t ldo, int out_dtype,
                 float alpha, const int32_t* lens, int frames_per_seq, int qkv_dp, float* scratch,

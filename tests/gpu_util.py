@@ -31,6 +31,31 @@ def op_gemm(use_tc, epi, A, W, bias=None, bias2=None, out=None, alpha=1.0, lens=
     return out
 
 
+def expected_instance(M, N, K, mode=None, sms=148):
+    """The tensor-core kernel launch_gemm_tc (gemm_tc.cu) picks for an (M, N, K) problem with 16-byte aligned operand
+    strides: ("tc", BN, STAGES) for gemm_tc_kernel<BN, STAGES, ...>, ("tc2",) for the CTA-pair gemm_tc2_kernel.
+    mode is CFB_GEMM_2CTA as a string ("0" never pairs, "1" pairs whenever gemm_tc2_supported, None: the default)."""
+    m_tiles = -(-M // 128)
+    small_m = N % 256 == 0 and 2 * m_tiles * (N // 256) <= sms
+    if not small_m:
+        flag = int(mode) if mode is not None else -1
+        tc2_supported = N % 256 == 0 and K % 8 == 0 and M > 128
+        if flag != 0 and tc2_supported and (flag == 1 or (K <= 1024 and N >= 1536)):
+            return ("tc2",)
+    if N % 256 == 0 and not small_m:
+        return ("tc", 256, 4 if -(-K // 64) >= 16 else 3)
+    return ("tc", 128, 5)
+
+
+def tiles_per_cta(M, N, inst, sms=148):
+    """Most output tiles one CTA (one CTA pair for "tc2") of the persistent grid works through."""
+    if inst[0] == "tc2":
+        tiles, workers = -(-M // 256) * (N // 256), sms // 2
+    else:
+        tiles, workers = -(-M // 128) * -(-N // inst[1]), sms
+    return -(-tiles // min(tiles, workers))
+
+
 def op_layernorm(x, gamma, beta, out, lens=None, frames_per_seq=1):
     lib = _lib.load_library()
     rows, d = x.shape

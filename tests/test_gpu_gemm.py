@@ -4,7 +4,7 @@ import pytest
 import torch
 
 from conformer_nemo_b200 import _lib
-from gpu_util import describe_mismatch, err_stats, op_gemm
+from gpu_util import describe_mismatch, err_stats, expected_instance, op_gemm, ptr, stream
 
 pytestmark = pytest.mark.gpu
 
@@ -146,11 +146,16 @@ def test_tc_matches_simt_on_bf16_inputs():
 
 
 @pytest.mark.parametrize("epi", ["LINEAR", "SWISH", "RESID", "QKV", "GLU"])
-@pytest.mark.parametrize("M,N,K", [(129, 256, 64), (300, 512, 176), (1000, 1536, 512), (16000, 2048, 512), (257, 768, 2048)])
+@pytest.mark.parametrize("M,N,K", [(4999, 2048, 512), (9900, 512, 176), (16000, 2048, 512), (19999, 1536, 512),
+                                   (19999, 2048, 512), (5000, 768, 2048), (20100, 1024, 2000), (20100, 768, 2000)])
 def test_cta_pair_kernel_is_bit_identical_to_the_single_cta_kernel(epi, M, N, K, monkeypatch):
-    """gemm_tc2.cu (cta_group::2, 256 x 256 tiles per CTA pair) against gemm_tc.cu on the same operands: same
-    k-block order and the same epilogue arithmetic -> identical bits, including M tails where the second CTA of the
-    last pair owns no valid row.  CFB_GEMM_2CTA forces either kernel (the default picks by shape)."""
+    """gemm_tc2.cu (cta_group::2, 256 x 256 tiles per CTA pair) against gemm_tc.cu's 256-wide kernel on the same
+    operands: same k-block order and the same epilogue arithmetic -> identical bits, including M tails where the last
+    pair's second CTA owns a few rows (4999, 9900, 5000, 20100), none (16000) or the first one only part of its rows
+    (19999).  CFB_GEMM_2CTA forces either kernel (the default picks by shape)."""
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    single, pair = expected_instance(M, N, K, "0", sms), expected_instance(M, N, K, "1", sms)
+    assert single[:2] == ("tc", 256) and pair == ("tc2",), (single, pair)
     A, W = _mk(M, N, K, seed=5)
     A, W = A.bfloat16(), W.bfloat16()
     bias = torch.randn(N, device="cuda") * 0.3
@@ -181,3 +186,51 @@ def test_cta_pair_kernel_is_bit_identical_to_the_single_cta_kernel(epi, M, N, K,
         outs.append(out)
     assert int(torch.isnan(outs[0].float()).sum()) == 0
     assert torch.equal(outs[0], outs[1]) and torch.equal(outs[1], outs[2]), err_stats(outs[1].float(), outs[0].float())
+
+
+CFB_ERR_INVALID_ARG, CFB_ERR_UNSUPPORTED = 1, 2
+
+
+# (use_tc, epilogue, N, out dtype, out columns, ldo, qkv_dp, status): combinations no GEMM kernel can write
+REFUSED = {
+    "tc-swish-f32": (1, _lib.EPI_SWISH, 256, torch.float32, 256, 256, 0, CFB_ERR_UNSUPPORTED),
+    "tc-relu-f32": (1, _lib.EPI_RELU, 256, torch.float32, 256, 256, 0, CFB_ERR_UNSUPPORTED),
+    "tc-qkv-f32": (1, _lib.EPI_QKV, 192, torch.float32, 256, 256, 64, CFB_ERR_UNSUPPORTED),
+    "tc-glu-f32": (1, _lib.EPI_GLU, 256, torch.float32, 128, 128, 0, CFB_ERR_UNSUPPORTED),
+    "tc-resid-bf16": (1, _lib.EPI_RESID, 256, torch.bfloat16, 256, 256, 0, CFB_ERR_UNSUPPORTED),
+    "simt-resid-bf16": (0, _lib.EPI_RESID, 256, torch.bfloat16, 256, 256, 0, CFB_ERR_UNSUPPORTED),
+    "tc-linear-f16": (1, _lib.EPI_LINEAR, 256, torch.float16, 256, 256, 0, CFB_ERR_UNSUPPORTED),
+    "tc-qkv-dp-96": (1, _lib.EPI_QKV, 288, torch.bfloat16, 384, 384, 96, CFB_ERR_INVALID_ARG),
+    "simt-qkv-dp-96": (0, _lib.EPI_QKV, 288, torch.float32, 384, 384, 96, CFB_ERR_INVALID_ARG),
+    "tc-qkv-dp-0": (1, _lib.EPI_QKV, 192, torch.bfloat16, 256, 256, 0, CFB_ERR_INVALID_ARG),
+    "tc-qkv-n-not-3dp": (1, _lib.EPI_QKV, 256, torch.bfloat16, 320, 320, 64, CFB_ERR_INVALID_ARG),
+    "tc-glu-n-200": (1, _lib.EPI_GLU, 200, torch.bfloat16, 104, 104, 0, CFB_ERR_INVALID_ARG),
+    "simt-glu-n-200": (0, _lib.EPI_GLU, 200, torch.float32, 104, 104, 0, CFB_ERR_INVALID_ARG),
+    "tc-linear-ldo": (1, _lib.EPI_LINEAR, 256, torch.bfloat16, 256, 248, 0, CFB_ERR_INVALID_ARG),
+    "tc-qkv-ldo": (1, _lib.EPI_QKV, 192, torch.bfloat16, 256, 192, 64, CFB_ERR_INVALID_ARG),
+    "simt-glu-ldo": (0, _lib.EPI_GLU, 256, torch.float32, 128, 120, 0, CFB_ERR_INVALID_ARG),
+    "tc-unknown-epilogue": (1, 6, 256, torch.bfloat16, 256, 256, 0, CFB_ERR_INVALID_ARG),
+}
+
+
+@pytest.mark.parametrize("case", list(REFUSED))
+def test_op_gemm_refuses_outputs_its_kernels_cannot_write(case):
+    """cfb_op_gemm returns an error before it enqueues anything: `out` (a sentinel) is left as it was."""
+    use_tc, epi, N, dt, cols, ldo, qkv_dp, status = REFUSED[case]
+    M, K = 64, 64
+    A, W = _mk(M, N, K, seed=7)
+    if use_tc:
+        A, W = A.bfloat16(), W.bfloat16()
+    bias = torch.zeros(N, device="cuda")
+    bias2 = torch.zeros(max(qkv_dp, 1), device="cuda")
+    out = torch.full((M, cols), 7.0, device="cuda", dtype=dt)
+    keep = out.clone()
+    scratch = torch.zeros(M * N, device="cuda")
+    lib = _lib.load_library()
+    dtype = {torch.float32: _lib.CFB_F32, torch.bfloat16: _lib.CFB_BF16, torch.float16: _lib.CFB_F16}[dt]
+    rc = lib.cfb_op_gemm(use_tc, epi, ptr(A), A.stride(0), ptr(W), W.stride(0), ptr(bias), ptr(bias2), M, N, K, ptr(out),
+                         ldo, dtype, 1.0, None, 1, qkv_dp, ptr(scratch), stream())
+    torch.cuda.synchronize()
+    assert rc == status, (rc, _lib.last_error(None))
+    assert "op_gemm" in _lib.last_error(None)
+    assert torch.equal(out, keep)

@@ -12,3 +12,4 @@ from .rnnt import RNNTDecoder, RNNTJoint, GreedyBatchedRNNTInfer, GreedyRNNTInfe
 from .rnnt import BeamRNNTInfer, NBestHypotheses  # noqa: F401
 from .collation import (BucketingIterator, CollationService, ManifestEntry, read_manifest, speech_collate)  # noqa: F401
 from .buffered import FrameBatchASR, buffered_ctc_transcribe  # noqa: F401
+from .buffered import BatchedFrameASRRNNT, buffered_rnnt_transcribe  # noqa: F401

@@ -191,7 +191,7 @@ def check_pos(r):
 def check_ctx(r):
     parts = [r.qkv[:, :, i, :, :r.dk].permute(0, 2, 1, 3) for i in range(4)]  # (B, H, T', dk)
     l = r.L - 1
-    p = r.pos[:, l * r.Dp:(l + 1) * r.Dp].view(r.P, r.H, 64)[..., :r.dk].permute(1, 0, 2)
+    p = r.pos[:, l * r.Dp:(l + 1) * r.Dp].view(r.P, r.H, -1)[..., :r.dk].permute(1, 0, 2)
     lens = r.ylen.long()
     want = torch_reference(*parts, p, lens)  # (B, T', H, dk)
     got = r.ctx[..., :r.dk]
